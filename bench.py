@@ -4,6 +4,7 @@
 batch of 64, no collective -- SURVEY.md section 8e).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload infer_sr|train_dn]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line on rank 0 (contract in the task statement): `value` is device-resident
@@ -27,6 +28,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # a bench run leaves the tree as it found it (which may be read-only)
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -142,6 +144,21 @@ def oracle_state_dict(kind: str):
     return O.init_state_dict(kind, 1, 1, NF, NB, 1, seed=21)
 
 
+DUMP_IMAGES = 8  # images of the batch written by --dump-outputs: 8 x 832 x 832 fp32 = 22 MB per output array
+
+
+def dump_index(batch: int) -> np.ndarray:
+    """The fixed, seeded sample of batch images that --dump-outputs writes."""
+    return np.sort(np.random.default_rng(0).choice(batch, size=min(batch, DUMP_IMAGES), replace=False))
+
+
+def write_outputs(directory: str, arrays) -> None:
+    """--dump-outputs: every array as <directory>/<name>.npy in float32, so that two builds can be compared."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def cpu_forward_fn():
     """The CPU arm's forward: the REFERENCE's own GeneratorRRDB_SR + Normalize (oracle/_ref, vendored from
     /root/reference by `python -m oracle.make_ref`; kind "reference") when present, else the oracle port (kind
@@ -203,9 +220,11 @@ def run_reference(args, rank: int) -> None:
     with torch.no_grad():
         for i in range(args.warmup + args.steps):
             t0 = time.perf_counter()
-            fwd(x)
+            out = fwd(x)
             if i >= args.warmup:
                 times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"output": out.numpy()})
     total = sum(times)
     value = n * args.steps / total
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": "images/s", "n_gpus": args.gpus,
@@ -268,6 +287,10 @@ def bench_train(args, kind: str, dev, dist, rank: int, world: int, local_rank: i
         barrier()
     launches = ops.LAUNCHES
     ms = e0.elapsed_time(e1)
+    if headline and args.dump_outputs and rank == 0:
+        # the last timed step's loss and the fp32 parameters it left (state_dict order), before the e2e steps train on
+        write_outputs(args.dump_outputs, {"loss": last.detach().reshape(1).cpu().numpy(),
+                                          "weights": step.flat.cpu().numpy()})
 
     loss_host = torch.empty(1, dtype=torch.float32).pin_memory()
 
@@ -338,6 +361,11 @@ def main() -> None:
     ap.add_argument("--no-parity", action="store_true", help="skip the post-run check of one output image (F=32 nb=4: ~1 s)")
     ap.add_argument("--filters", type=int, default=NF, help="developer sweeps only (BASELINE's configs are 32 / 4)")
     ap.add_argument("--blocks", type=int, default=NB)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32): "
+                         "infer_sr: output (device-resident call) and output_e2e (host pipeline), 8 seeded images "
+                         "of the batch each; train_*: loss and weights (the fp32 parameters after that step); "
+                         "--impl reference: output")
     args = ap.parse_args()
     NF, NB = args.filters, args.blocks
     if args.warmup < 3 and args.impl == "ours":
@@ -418,8 +446,10 @@ def main() -> None:
         prof_events.append((e0, e1, flop, ops.LAST_CHAIN_LAUNCHES))
 
     with torch.no_grad():
+        # the timed loop keeps each step's output until the next one exists (--dump-outputs reads the last): warming
+        # up the same way leaves both output blocks in the allocator's cache before timing starts
         for _ in range(args.warmup):
-            model(x_dev)
+            out = model(x_dev)
         import xmm_superres_denoise_b200.engine as engine_mod
 
         engine_mod.ops.conv3x3 = conv_profiled
@@ -430,11 +460,16 @@ def main() -> None:
         with ClockSampler(local_rank) as clocks:
             start.record()
             for _ in range(args.steps):
-                model(x_dev)
+                out = model(x_dev)
             stop.record()
             barrier()
         engine_mod.ops.conv3x3 = orig_conv
         engine_mod.ops.conv3x3_chain = orig_chain
+        dump = {}
+        if args.dump_outputs and rank == 0:
+            dump_idx = torch.from_numpy(dump_index(B))
+            dump["output"] = out[dump_idx].float().cpu().numpy()
+        del out
         launches = ops.LAUNCHES
         ms_total = start.elapsed_time(stop)
         k_ms = sum(e0.elapsed_time(e1) for e0, e1, _, _ in prof_events)
@@ -470,6 +505,9 @@ def main() -> None:
         t2.record()
         barrier()
         e2e_ms = max(s2.elapsed_time(t2), (time.perf_counter() - t_wall) * 1e3)  # device events vs host wall: the larger
+        if dump:
+            dump["output_e2e"] = out_hosts[(args.steps + 1) & 1][dump_idx].numpy()
+            write_outputs(args.dump_outputs, dump)
 
         # ------------------------------------------------------------ parity self-check (outside every timed region)
         # One image of the batch the bench just produced -- through the exact dispatch that was timed (batch-64 work

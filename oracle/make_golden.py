@@ -71,6 +71,31 @@ def net_case(ref, kind: str, nf: int, nb: int, seed: int, shape, counts: bool):
     return res
 
 
+INIT_SEED, INIT_NF, INIT_NB = 123, 32, 2
+INIT_SAMPLES = 64  # values kept per tensor: the full state_dict (3.4 MB per generator) is too large to store
+
+
+def init_fingerprint(cls, kind: str) -> dict:
+    """What ``torch.manual_seed(123); cls(1, 1, 32, 2[, num_upsample=1]).state_dict()`` holds: keys in order, element
+    counts, INIT_SAMPLES evenly spaced values of every tensor (exact fp32) and its float64 sum and sum of squares."""
+    torch.manual_seed(INIT_SEED)
+    model = cls(1, 1, INIT_NF, INIT_NB) if kind == "dn" else cls(1, 1, INIT_NF, INIT_NB, num_upsample=1)
+    flat = [v.detach().reshape(-1) for v in model.state_dict().values()]
+    picks = [np.linspace(0, v.numel() - 1, min(v.numel(), INIT_SAMPLES)).round().astype(np.int64) for v in flat]
+    return {"keys": np.array(list(model.state_dict().keys())),
+            "numel": np.array([v.numel() for v in flat]),
+            "sample": np.concatenate([v.numpy()[i] for v, i in zip(flat, picks)]),
+            "moments": np.array([[v.double().sum().item(), v.double().square().sum().item()] for v in flat])}
+
+
+def write_init_golden(gen_dn, gen_sr, source: str) -> None:
+    """tests/golden/init_seed123.npz: the default initialisation of both generators under one seed."""
+    res = {"source": np.array(source)}
+    for kind, cls in (("dn", gen_dn), ("sr", gen_sr)):
+        res.update({f"{kind}.{k}": v for k, v in init_fingerprint(cls, kind).items()})
+    np.savez_compressed(os.path.join(OUT, "init_seed123.npz"), **res)
+
+
 def main() -> None:
     os.makedirs(OUT, exist_ok=True)
     torch.manual_seed(0)
@@ -130,6 +155,9 @@ def main() -> None:
     img = det_input((2, 1, 5, 7), 77)
     np.savez_compressed(os.path.join(OUT, "imageupsample.npz"), x=img.numpy(),
                         up2=ref.ImageUpsample(2)(img).numpy(), up3_single=ref.ImageUpsample(3)(img[0]).numpy())
+
+    # (E) default initialisation under a fixed seed
+    write_init_golden(ref.GeneratorRRDB_DN, ref.GeneratorRRDB_SR, "reference classes")
     print("golden fixtures written to", OUT)
 
 

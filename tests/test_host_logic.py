@@ -1,9 +1,13 @@
 """CPU: host-side mirror of the reference interface (names, state_dict, error behaviour)."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
 from oracle import ref_loader
 from oracle import rrdb_oracle as O
+from oracle.make_golden import init_fingerprint
 from xmm_superres_denoise_b200.models import GeneratorRRDB_DN, GeneratorRRDB_SR
 from xmm_superres_denoise_b200.models.modules import RRDB, ResidualDenseBlock_5C, make_layer
 from xmm_superres_denoise_b200.transforms import ImageUpsample, Normalize
@@ -29,9 +33,20 @@ def test_default_num_upsample_and_attributes():
     assert len(make_layer(lambda: RRDB(32, 32), 3)) == 3
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
 @pytest.mark.parametrize("kind", ["dn", "sr"])
-def test_same_seed_gives_the_reference_initialisation(kind):
+def test_same_seed_gives_the_reference_initialisation(golden_dir, kind):
+    """The reference's initialisation is torch's default one, drawn in its module construction order.  The stored
+    fingerprint of it (tests/golden/init_seed123.npz: keys, sizes, exact sampled values, sums) was recorded from these
+    classes, which the comparison below holds bit-equal to the reference's own classes where its source is present."""
+    cls = GeneratorRRDB_DN if kind == "dn" else GeneratorRRDB_SR
+    got = init_fingerprint(cls, kind)
+    g = np.load(os.path.join(golden_dir, "init_seed123.npz"))
+    assert list(got["keys"]) == list(g[f"{kind}.keys"])
+    np.testing.assert_array_equal(got["numel"], g[f"{kind}.numel"])
+    np.testing.assert_array_equal(got["sample"], g[f"{kind}.sample"])
+    np.testing.assert_allclose(got["moments"], g[f"{kind}.moments"], rtol=1e-9, atol=1e-12)
+    if not ref_loader.available():
+        return
     ref = ref_loader.load_reference()
     torch.manual_seed(123)
     a = ref.GeneratorRRDB_DN(1, 1, 32, 2) if kind == "dn" else ref.GeneratorRRDB_SR(1, 1, 32, 2, num_upsample=1)

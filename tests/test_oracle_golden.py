@@ -88,7 +88,8 @@ def test_combine_mask_pad_geometry():
     assert float(out.sum()) == 6 * 100 * 403
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
+@pytest.mark.skipif(not ref_loader.available(),
+                    reason="needs the reference's source tree (XMM_REFERENCE_ROOT, or its copy in oracle/_ref)")
 @pytest.mark.parametrize("kind", ["dn", "sr"])
 def test_oracle_matches_live_reference(kind):
     ref = ref_loader.load_reference()
