@@ -42,6 +42,16 @@
 // quarter) iterate their own layer only -- pieces in order, rows top to bottom -- and meet the other roles through
 // mbarriers.  Rule for every barrier here: its waiter observes EVERY phase (a parity wait two phases ahead passes at
 // once) -- hence per-layer barriers and per-layer roles; tools/rdb_protocol_sim.py models the whole protocol.
+//
+// CTA pairs (template PAIR; conv4 + conv5).  There the resident weights (164 KB) leave five TMA stages and the issuer
+// waits for chunks to land.  Two CTAs of a cluster run as a tcgen05 cta_group::2 pair: the leader's issuers issue
+// M = 256 MMAs (rows 0..127 = the leader's row tile, 128..255 = the peer's) and each CTA holds a compacted HALF of every
+// (chunk, dx) group of the weight image (rank 0 rows 0..47, rank 1 rows 48..95, 3 KB per group), so 14 stages fit.
+// Each CTA keeps its own producer, stage ring, x4 ring, epilogue groups and TMEM lanes, and walks its own column of
+// the same pair-column (RdbSched<NL, true>): both CTAs take the same walk over the same stage count, so the stage and
+// ring-slot ids are the same in both and the leader's descriptors address both.  Both producers' loads complete on
+// the leader's `lfull`; the peer's epilogue warps arrive on the leader's `tdrain` / `mfull` (count 8); the leader's
+// commits (`empty`, `mempty`, `tfull`) are multicast to both CTAs.
 #pragma once
 #include <cstdio>
 
@@ -57,12 +67,19 @@ constexpr int kRdbThreads = 512;                  // producer warp, one issuer w
 constexpr int kRdbSlots = 5;                      // accumulator slots per layer
 constexpr int kRdbSlotCols = kRdbSlots * 32;
 constexpr int kRdbMaxRing = 8;
-constexpr int kRdbMaxStages = 8;
+constexpr int kRdbMaxStages = 16;
+// Length of the per-layer landed rings (lfull / lstage) = capacity of the stage ring.  Issuer l waits on slot
+// k = chunk mod kRdbLRing; the producer is at most `stages` chunks ahead of the last chunk consumed, so with
+// stages <= kRdbLRing no parity wait can pass a phase early.  A single CTA fits <= 8 stages next to its weights.
+template <bool PAIR>
+constexpr int kRdbLRing = PAIR ? kRdbMaxStages : 8;
 constexpr int kRdbTapBytes = 32 * 64;             // one (dx, dy) block of a chunk: 32 output channels x 32 inputs
+constexpr int kRdbGroupBytes = 3 * kRdbTapBytes;  // one (chunk, dx) group of the row-hop image: 96 rows of 64 B
+constexpr int kRdbProfSlots = 24;                 // XMM_RDB_PROFILE counters per CTA
 
 struct RdbLayerArgs {
   const void* wblob;   // row-hop order [chunk][dx][2 - dy][32][32] bf16 (SWIZZLE_64B applied) + 32 fp32 biases
-  uint32_t w_bytes;    // without the biases
+  uint32_t w_bytes;    // of the image in shared memory, without the biases (CTA pair: half of the blob's)
   uint32_t smem_off;   // where this layer's image starts in the weight region (1024-aligned)
   float lrelu_slope;   // 1 = none
   int store;           // the output is needed outside the kernel
@@ -74,7 +91,7 @@ struct RdbArgs {
   RdbLayerArgs layer[3];
   int cin_off;                 // channel of x0 in the input buffer (x_j at cin_off + 32 j)
   int batch, height, width, band_h, tiles_x;
-  long long total_rows;        // batch * tiles_x * band_h (rows of all columns)
+  long long total_rows;        // batch * tiles_x * band_h (rows of all columns; CTA pairs: of all pair-columns)
   int stages, ring0, ring1;    // TMA stages; row tiles of the first / second in-CTA map
   uint32_t w_total;            // bytes of the weight region
   // residuals of the LAST layer (conv5: out = s0 * v + s1 * r1 + s2 * r2, rrdb_blocks.py:54,70)
@@ -86,7 +103,7 @@ struct RdbArgs {
   int backoff_ns;   // nanosleep between polls of the producer / epilogue waits (0: none)
   int prefetch_rows;  // the producer asks L2 for the global maps of the row this many steps ahead (0: off)
   int split_producers;  // two fused layers: one TMA producer thread and stage-ring slice per layer
-  long long* prof;  // optional (XMM_RDB_PROF=1): 16 cycle counters per CTA, see launch_rdb
+  long long* prof;  // optional (XMM_RDB_PROF=1): kRdbProfSlots cycle counters per CTA, see launch_rdb
 };
 
 template <int NL>
@@ -108,30 +125,49 @@ struct RdbPiece {
 
 // The CTA's share of the work: the rows of all (image, tile) columns, in column order, cut into gridDim.x equal
 // contiguous ranges; a range touches a few columns = pieces.
-template <int NL>
+// PAIR: pair-column p is column 2p on cluster rank 0 and 2p + 1 on rank 1; the rows of the pair-columns are cut into
+// gridDim.x / 2 ranges, so both CTAs of a pair take the same pieces, rows and flush steps (the same walk) and differ
+// only in b, x0 and the owned pixels.  With an odd column count rank 1's last column is a phantom: it repeats the
+// last real column (in-bounds loads) and owns no pixel, so it stores nothing.
+template <int NL, bool PAIR = false>
 struct RdbSched {
   int band_h, tiles_x, width, c0, npieces;
+  int ncols, rank;  // PAIR: columns, cluster rank
   long long t0, t1;
   __device__ __forceinline__ void init(const RdbArgs& a) {
     band_h = a.band_h;
     tiles_x = a.tiles_x;
     width = a.width;
-    t0 = a.total_rows * blockIdx.x / gridDim.x;
-    t1 = a.total_rows * (blockIdx.x + 1) / gridDim.x;
+    if (PAIR) {
+      ncols = a.batch * a.tiles_x;
+      rank = int(ptx::cluster_ctarank());
+      const long long unit = blockIdx.x >> 1, nunits = gridDim.x >> 1;
+      t0 = a.total_rows * unit / nunits;
+      t1 = a.total_rows * (unit + 1) / nunits;
+    } else {
+      t0 = a.total_rows * blockIdx.x / gridDim.x;
+      t1 = a.total_rows * (blockIdx.x + 1) / gridDim.x;
+    }
     c0 = int(t0 / band_h);
     npieces = t1 > t0 ? int((t1 - 1) / band_h) - c0 + 1 : 0;
   }
   __device__ __forceinline__ RdbPiece get(int i) const {
     RdbPiece p;
-    const int col = c0 + i;
+    int col = c0 + i;
     const long long base = (long long)col * band_h;
     p.ra = t0 > base ? int(t0 - base) : 0;
     p.rb = t1 < base + band_h ? int(t1 - base) : band_h;
+    bool phantom = false;
+    if (PAIR) {
+      col = 2 * col + rank;
+      phantom = col >= ncols;
+      if (phantom) col = ncols - 1;
+    }
     p.b = col / tiles_x;
     const int t = col - p.b * tiles_x;
     p.own_lo = rdb_tile_origin<NL>(t);
     p.x0 = t == 0 ? 0 : p.own_lo - (NL - 1);
-    p.own_hi = t == tiles_x - 1 ? width : rdb_tile_origin<NL>(t + 1);
+    p.own_hi = phantom ? p.own_lo : t == tiles_x - 1 ? width : rdb_tile_origin<NL>(t + 1);
     return p;
   }
 };
@@ -139,8 +175,8 @@ struct RdbSched {
 // The step sequence.  f(l, piece, r, flush, n, seq): layer l takes its step on input row r of `piece` (flush: one of
 // the two MMA-less steps after the piece's last row); n = how many steps layer l took before; seq[m] = sequence
 // number, among all rows of in-CTA map m, of the piece's first row ra - (NL-1-m).
-template <int NL, class F>
-__device__ __forceinline__ void rdb_walk(const RdbSched<NL>& s, F&& f) {
+template <int NL, class S, class F>
+__device__ __forceinline__ void rdb_walk(const S& s, F&& f) {
   int piece[NL], r[NL], hi[NL], n[NL], seq[NL][NL];
   RdbPiece pc[NL];
   bool done[NL];
@@ -275,25 +311,27 @@ struct RdbCtx {
   uint8_t* w_s;        // weights + biases of every layer
   uint8_t* stage_s;    // TMA stages (one ring shared by all layers, handed out in walk order)
   uint8_t* map_s[2];   // row tiles of the in-CTA maps
-  uint64_t* lfull;     // [NL][8] chunk k (mod 8) of layer l has landed        (waiter: issuer l)
+  uint64_t* lfull;     // [3][R] chunk k (mod R = kRdbLRing) of layer l has landed (waiter: issuer l)
   uint64_t* empty;     // [stages] the MMAs that read the stage are done        (waiter: producer)
   uint64_t* tfull;     // [NL] the row a step completes is in TMEM              (waiter: epilogue group l)
   uint64_t* tdrain;    // [NL] ... has been drained and its slot re-initialised (waiter: issuer l)
   uint64_t* mfull;     // [2][8] row tile of map m written                       (waiters: issuers m+1 ..)
   uint64_t* mempty;    // [2][8] ... read by its last reader                     (waiter: epilogue group m)
   uint64_t* w_bar;
-  volatile int* lstage;  // [NL][8] which stage holds chunk k (mod 8) of layer l (written by the producer)
+  volatile int* lstage;  // [3][R] which stage holds chunk k (mod R) of layer l (written by the producer)
   uint32_t tmem_base;
 };
 
 // ---------------------------------------------------------------------------------------------------- MMA issuer
 // One thread per layer: the bookkeeping of one layer's step (~60 instructions of a single thread) overlaps the MMAs
 // of the other layers.  The thread walks its OWN layer only: pieces in order, rows top to bottom.
-template <int G, int NL, int L>
-__device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c, const RdbSched<NL>& sched) {
+// PAIR: runs in the leader only and issues for both CTAs; its commits reach both.
+template <int G, int NL, int L, bool PAIR>
+__device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c, const RdbSched<NL, PAIR>& sched) {
   constexpr int NM = NL - 1;
   constexpr int e = NL - 1 - L;
   constexpr int ring[2] = {NL == 3 ? 5 : 2, 3};
+  constexpr uint32_t kR = kRdbLRing<PAIR>;
   rdb_wait(c.w_bar, 0, 7, L, 0);
   ptx::tc_fence_after();
   const uint64_t bdesc0 = ptx::umma_smem_desc(ptx::smem_u32(c.w_s), 16, 512, ptx::UMMA_SW64);
@@ -303,15 +341,27 @@ __device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c,
   const uint32_t b_l = uint32_t(bdesc0) + (args.layer[L].smem_off >> 4);
   const uint32_t a_map0[2] = {a_lo0 + uint32_t((c.map_s[0] - c.stage_s) >> 4), a_lo0 + uint32_t((c.map_s[1] - c.stage_s) >> 4)};
   constexpr uint32_t kTile16 = uint32_t(kRdbTileBytes) >> 4;
-  constexpr uint32_t kTap16 = uint32_t(kRdbTapBytes) >> 4;
-  constexpr uint32_t kIdesc = ptx::umma_idesc_bf16_f32(128, 96, 0, 0);
+  // a (chunk, dx) group of B: 96 rows (3 dy x 32 couts) in one CTA, the CTA's 48 of them in a pair
+  constexpr uint32_t kGroup16 = uint32_t(PAIR ? kRdbGroupBytes / 2 : kRdbGroupBytes) >> 4;
+  constexpr uint32_t kChunk16 = 3 * kGroup16;
+  constexpr uint32_t kIdesc = ptx::umma_idesc_bf16_f32(PAIR ? 256 : 128, 96, 0, 0);
   auto issue6 = [&](uint32_t d, uint32_t a, uint32_t b) {
 #pragma unroll
     for (int dx = 0; dx < 3; ++dx)
 #pragma unroll
-      for (int ks = 0; ks < 2; ++ks)
-        ptx::umma_ss_lh<true>(d, a + uint32_t((dx * 64 + ks * 32) >> 4), a_hi, b + uint32_t(dx * 3) * kTap16 + uint32_t((ks * 32) >> 4),
-                              b_hi, kIdesc);
+      for (int ks = 0; ks < 2; ++ks) {
+        const uint32_t a_lo = a + uint32_t((dx * 64 + ks * 32) >> 4), b_lo = b + uint32_t(dx) * kGroup16 + uint32_t((ks * 32) >> 4);
+        if constexpr (PAIR)
+          ptx::umma_ss_lh_pair<true>(d, a_lo, a_hi, b_lo, b_hi, kIdesc);
+        else
+          ptx::umma_ss_lh<true>(d, a_lo, a_hi, b_lo, b_hi, kIdesc);
+      }
+  };
+  auto commit = [](uint64_t* bar) {
+    if constexpr (PAIR)
+      ptx::umma_commit_pair(bar);
+    else
+      ptx::umma_commit(bar);
   };
   const bool prof = XMM_RDB_PROFILE && args.prof != nullptr && L == 0;
   long long pw[3] = {0, 0, 0};
@@ -331,13 +381,13 @@ __device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c,
         auto global_chunks = [&]() {
 #pragma unroll
           for (int g = 0; g < G; ++g) {
-            const int k = int(fills & 7u);
-            rdb_wait_p(&c.lfull[L * 8 + k], (fills >> 3) & 1u, 3, L, k, prof, pw[1]);
-            const int stage = c.lstage[L * 8 + k];
+            const int k = int(fills % kR);
+            rdb_wait_p(&c.lfull[L * kR + k], (fills / kR) & 1u, 3, L, k, prof, pw[1]);
+            const int stage = c.lstage[L * kR + k];
             ++fills;
             ptx::tc_fence_after();
-            issue6(d, a_lo0 + uint32_t(stage) * kTile16, b_l + uint32_t(g * 9) * kTap16);
-            ptx::umma_commit(&c.empty[stage]);
+            issue6(d, a_lo0 + uint32_t(stage) * kTile16, b_l + uint32_t(g) * kChunk16);
+            commit(&c.empty[stage]);
           }
         };
         auto map_chunks = [&]() {
@@ -348,9 +398,9 @@ __device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c,
               const int slot = sq % ring[m];
               rdb_wait_p(&c.mfull[m * 8 + slot], uint32_t(sq / ring[m]) & 1u, 4, L * 10 + m, sq, prof, pw[2]);
               ptx::tc_fence_after();
-              issue6(d, a_map0[m] + uint32_t(slot) * kTile16, b_l + uint32_t((G + m) * 9) * kTap16);
+              issue6(d, a_map0[m] + uint32_t(slot) * kTile16, b_l + uint32_t(G + m) * kChunk16);
               // the last layer that reads this row gives the tile back: layer L+1 reads rows [ra-e, rb+e-1]
-              if (L == NL - 1 || r < pc.ra - e || r > pc.rb + e - 1) ptx::umma_commit(&c.mempty[m * 8 + slot]);
+              if (L == NL - 1 || r < pc.ra - e || r > pc.rb + e - 1) commit(&c.mempty[m * 8 + slot]);
             }
         };
         // Two fused layers: the in-CTA map first -- x4 was written a round ago, while the four global chunks of this
@@ -364,13 +414,13 @@ __device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c,
           map_chunks();
         }
       }
-      ptx::umma_commit(&c.tfull[L]);  // row r-1 is complete
+      commit(&c.tfull[L]);  // row r-1 is complete
     }
 #pragma unroll
     for (int m = 0; m < NM; ++m) seq[m] += (pc.rb - pc.ra) + 2 * (NL - 1 - m);
   }
   if (XMM_RDB_PROFILE && prof) {
-    long long* o = args.prof + size_t(blockIdx.x) * 16;
+    long long* o = args.prof + size_t(blockIdx.x) * kRdbProfSlots;
     o[0] = clock64() - t_begin;
     o[1] = pw[0];
     o[2] = pw[1];
@@ -380,8 +430,18 @@ __device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c,
 
 // ---------------------------------------------------------------------------------------------------- epilogue
 // Four warps per layer (one per TMEM lane quarter) drain that layer's rows in order.
-template <int G, int NL, int L>
-__device__ __forceinline__ void rdb_epilogue(const RdbArgs& args, const RdbCtx& c, const RdbSched<NL>& sched, int q, int lane) {
+// PAIR: the peer's warps arrive on the LEADER's tdrain / mfull (relaxed: a release.cluster arrive would wait for this
+// warp's global stores as well and stall the epilogue).
+template <int G, int NL, int L, bool PAIR>
+__device__ __forceinline__ void rdb_epilogue(const RdbArgs& args, const RdbCtx& c, const RdbSched<NL, PAIR>& sched, int q,
+                                             int lane) {
+  const bool remote = PAIR && sched.rank != 0;
+  auto arrive = [&](uint64_t* bar) {
+    if (remote)
+      ptx::mbar_arrive_cluster(ptx::mapa(ptx::smem_u32(bar), 0));
+    else
+      ptx::mbar_arrive(bar);
+  };
   constexpr int e = NL - 1 - L;
   constexpr int ring[2] = {NL == 3 ? 5 : 2, 3};
   constexpr bool last = L == NL - 1;
@@ -464,7 +524,7 @@ __device__ __forceinline__ void rdb_epilogue(const RdbArgs& args, const RdbCtx& 
       tmem_st_wait();
       ptx::tc_fence_before();
       __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(&c.tdrain[L]);
+      if (lane == 0) arrive(&c.tdrain[L]);
       if (XMM_RDB_PROFILE) {
         const long long t = clock64();
         ph[0] += t - tph;
@@ -529,7 +589,7 @@ __device__ __forceinline__ void rdb_epilogue(const RdbArgs& args, const RdbCtx& 
         for (int k = 0; k < 4; ++k) *reinterpret_cast<uint4*>(dst + ((uint32_t(k) ^ pos_xor) << 4)) = inimg ? o[k] : zero;
         ptx::fence_proxy_async();
         __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(&c.mfull[L * 8 + slot]);
+        if (lane == 0) arrive(&c.mfull[L * 8 + slot]);
         if (XMM_RDB_PROFILE) {
           const long long t = clock64();
           ph[2] += t - tph;
@@ -545,18 +605,16 @@ __device__ __forceinline__ void rdb_epilogue(const RdbArgs& args, const RdbCtx& 
     seq += (pc.rb - pc.ra) + 2 * e;
   }
   if (XMM_RDB_PROFILE && prof && q == 0 && lane == 0 && L < 2) {
-    long long* o = args.prof + size_t(blockIdx.x) * 16 + 4 + 4 * L;
+    long long* o = args.prof + size_t(blockIdx.x) * kRdbProfSlots + 4 + 4 * L;
     o[0] = clock64() - t_begin;
     o[1] = pw[0];
     o[2] = pw[1];
     o[3] = (long long)n;
-    if (L == 0) {
-      long long* o2 = args.prof + size_t(blockIdx.x) * 16 + 12;
-      o2[0] = ph[0];
-      o2[1] = ph[1];
-      o2[2] = ph[2];
-      o2[3] = ph[3];
-    }
+    long long* o2 = args.prof + size_t(blockIdx.x) * kRdbProfSlots + 12 + 4 * L;  // the phases of one row
+    o2[0] = ph[0];
+    o2[1] = ph[1];
+    o2[2] = ph[2];
+    o2[3] = ph[3];
   }
 }
 
@@ -625,12 +683,16 @@ __device__ __forceinline__ void rdb_layer_producer(const CUtensorMap* tmap_in, c
 // Warp roles (512 threads): warp 0 = TMA producer (the only role that follows the interleaved walk: it decides the
 // order in which the layers' rows are loaded), warp 1 + l = MMA issuer of layer l, warps 4 + 4 l .. 7 + 4 l = epilogue
 // of layer l.  Issuers and epilogue groups only know their own layer; everything between roles is an mbarrier.
-template <int G, int NL>
+// PAIR: launched as clusters of 2 (see the top of this file).
+template <int G, int NL, bool PAIR = false>
 __global__ void __launch_bounds__(kRdbThreads, 1)
 conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs args) {
   static_assert(NL == 2 || NL == 3, "two or three fused layers");
   static_assert(NL * kRdbSlotCols <= 512, "accumulators exceed TMEM");
   constexpr int NM = NL - 1;  // in-CTA maps
+  constexpr int kR = kRdbLRing<PAIR>;
+  // lfull, empty, tfull, tdrain, mfull, mempty, w_bar; lstage; the TMEM address: the 1024 B the launcher reserves
+  static_assert((3 * kR + kR + 3 + 3 + 16 + 16 + 1) * 8 + 3 * kR * 4 + 4 <= 1024, "barrier block exceeds 1024 B");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   RdbCtx c;
@@ -640,37 +702,46 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
   c.map_s[1] = c.map_s[0] + size_t(args.ring0) * kRdbTileBytes;
   uint8_t* after = c.map_s[1] + size_t(NM > 1 ? args.ring1 : 0) * kRdbTileBytes;
   uint64_t* bars = reinterpret_cast<uint64_t*>(after);
-  c.lfull = bars;            // 24
-  c.empty = c.lfull + 24;    // 8
-  c.tfull = c.empty + 8;     // 3
-  c.tdrain = c.tfull + 3;    // 3
-  c.mfull = c.tdrain + 3;    // 16
-  c.mempty = c.mfull + 16;   // 16
-  c.w_bar = c.mempty + 16;   // 1
-  c.lstage = reinterpret_cast<volatile int*>(c.w_bar + 1);  // 24 ints
-  uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(const_cast<int*>(c.lstage) + 24);
+  c.lfull = bars;              // 3 R
+  c.empty = c.lfull + 3 * kR;  // R
+  c.tfull = c.empty + kR;      // 3
+  c.tdrain = c.tfull + 3;      // 3
+  c.mfull = c.tdrain + 3;      // 16
+  c.mempty = c.mfull + 16;     // 16
+  c.w_bar = c.mempty + 16;     // 1
+  c.lstage = reinterpret_cast<volatile int*>(c.w_bar + 1);  // 3 R ints
+  uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(const_cast<int*>(c.lstage) + 3 * kR);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
+  const uint32_t rank = PAIR ? ptx::cluster_ctarank() : 0u;
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tmap_in);
-    for (int s = 0; s < NL * 8; ++s) ptx::mbar_init(&c.lfull[s], 1);
+    for (int s = 0; s < NL * kR; ++s) ptx::mbar_init(&c.lfull[s], 1);
     for (int s = 0; s < args.stages; ++s) ptx::mbar_init(&c.empty[s], 1);
     for (int l = 0; l < NL; ++l) {
       ptx::mbar_init(&c.tfull[l], 1);
-      ptx::mbar_init(&c.tdrain[l], 4);  // the four warps of the layer's epilogue group
+      ptx::mbar_init(&c.tdrain[l], PAIR ? 8 : 4);  // the four warps of the layer's epilogue group (pair: in both CTAs)
     }
     for (int s = 0; s < 16; ++s) {
-      ptx::mbar_init(&c.mfull[s], 4);
+      ptx::mbar_init(&c.mfull[s], PAIR ? 8 : 4);
       ptx::mbar_init(&c.mempty[s], 1);  // the commit of the row's last reader
     }
     ptx::mbar_init(c.w_bar, 1);
     ptx::fence_mbar_init();
   }
-  if (warp == 1) ptx::tmem_alloc<512>(tmem_ptr_s);
+  if (warp == 1) {
+    if constexpr (PAIR)
+      ptx::tmem_alloc_pair<512>(tmem_ptr_s);
+    else
+      ptx::tmem_alloc<512>(tmem_ptr_s);
+  }
   ptx::tc_fence_before();
-  __syncthreads();
+  if constexpr (PAIR)
+    ptx::cluster_sync();  // the peer's barriers are initialised before anything arrives on them
+  else
+    __syncthreads();
   ptx::tc_fence_after();
   c.tmem_base = *tmem_ptr_s;
 
@@ -680,9 +751,19 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
     ptx::mbar_expect_tx(c.w_bar, wtot);
     for (int l = 0; l < NL; ++l) {
       const uint8_t* gsrc = static_cast<const uint8_t*>(args.layer[l].wblob);
-      const uint32_t n_l = args.layer[l].w_bytes + 128u;
-      for (uint32_t off = 0; off < n_l; off += 32768u)
-        ptx::bulk_load(c.w_s + args.layer[l].smem_off + off, gsrc + off, n_l - off < 32768u ? n_l - off : 32768u, c.w_bar);
+      uint8_t* dst = c.w_s + args.layer[l].smem_off;
+      const uint32_t wb = args.layer[l].w_bytes;
+      if constexpr (PAIR) {
+        // this CTA's half of every (chunk, dx) group: rows [48 rank, 48 rank + 48), six whole SWIZZLE_64B atoms
+        constexpr uint32_t kHalf = kRdbGroupBytes / 2;
+        for (uint32_t grp = 0; grp < wb / kHalf; ++grp)
+          ptx::bulk_load(dst + grp * kHalf, gsrc + grp * kRdbGroupBytes + rank * kHalf, kHalf, c.w_bar);
+        ptx::bulk_load(dst + wb, gsrc + 2 * wb, 128u, c.w_bar);
+      } else {
+        const uint32_t n_l = wb + 128u;
+        for (uint32_t off = 0; off < n_l; off += 32768u)
+          ptx::bulk_load(dst + off, gsrc + off, n_l - off < 32768u ? n_l - off : 32768u, c.w_bar);
+      }
     }
   }
   const int egroup = (warp - 4) >> 2;  // epilogue group = layer (warps 4..)
@@ -707,21 +788,29 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
     }
   }
   ptx::tc_fence_before();
-  __syncthreads();
+  if constexpr (PAIR)
+    ptx::cluster_sync();  // the leader's first MMAs read the peer's weights and accumulate into the peer's TMEM
+  else
+    __syncthreads();
   ptx::tc_fence_after();
 
-  RdbSched<NL> sched;
+  RdbSched<NL, PAIR> sched;
   sched.init(args);
 
-  if (NL == 2 && args.split_producers && (warp == 0 || warp == 3)) {
+  if (!PAIR && NL == 2 && args.split_producers && (warp == 0 || warp == 3)) {
     // ------------------------------------------------------------ TMA producers, one per layer (warps 0 and 3)
-    if (ptx::elect_one()) {
-      const int ns0 = (args.stages + 1) / 2;  // conv4 (whose rows come from HBM) gets the larger half
-      if (warp == 0) rdb_layer_producer<G, NL, 0>(&tmap_in, args, c, sched, 0, ns0);
-      if (warp == 3) rdb_layer_producer<G, NL, 1>(&tmap_in, args, c, sched, ns0, args.stages - ns0);
+    if constexpr (!PAIR) {
+      if (ptx::elect_one()) {
+        const int ns0 = (args.stages + 1) / 2;  // conv4 (whose rows come from HBM) gets the larger half
+        if (warp == 0) rdb_layer_producer<G, NL, 0>(&tmap_in, args, c, sched, 0, ns0);
+        if (warp == 3) rdb_layer_producer<G, NL, 1>(&tmap_in, args, c, sched, ns0, args.stages - ns0);
+      }
     }
   } else if (warp == 0) {
     // ------------------------------------------------------------ TMA producer
+    // PAIR: both CTAs' producers take the same walk over the same stage count, so they write the same stage ids into
+    // lstage -- the leader's issuers address the peer's stages with the leader's ids.  Both loads of a chunk complete
+    // on the leader's lfull, which the leader's producer arms for both.
     if (ptx::elect_one()) {
       int stage = 0;
       uint32_t phase = 0;
@@ -742,12 +831,18 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
 #pragma unroll
         for (int g = 0; g < G; ++g) {
           rdb_wait_backoff(&c.empty[stage], phase ^ 1u, 1, l, stage, uint32_t(args.backoff_ns));
-          const int k = int(fills[l]++ & 7u);
-          c.lstage[l * 8 + k] = stage;  // (made visible to the issuer by the release of the arrive below)
-          uint64_t* fb = &c.lfull[l * 8 + k];
-          ptx::mbar_expect_tx(fb, kRdbTileData);
-          ptx::tma_load_5d(c.stage_s + size_t(stage) * kRdbTileBytes, &tmap_in, fb, args.cin_off + 32 * g, pc.x0 - 1, row, band0,
-                           pc.b);
+          const int k = int(fills[l]++ % uint32_t(kR));
+          c.lstage[l * kR + k] = stage;  // (made visible to the issuer by the release of the arrive below)
+          uint64_t* fb = &c.lfull[l * kR + k];
+          if constexpr (PAIR) {
+            if (rank == 0) ptx::mbar_expect_tx(fb, 2 * kRdbTileData);
+            ptx::tma_load_5d_pair(c.stage_s + size_t(stage) * kRdbTileBytes, &tmap_in, ptx::mapa(ptx::smem_u32(fb), 0),
+                                  args.cin_off + 32 * g, pc.x0 - 1, row, band0, pc.b);
+          } else {
+            ptx::mbar_expect_tx(fb, kRdbTileData);
+            ptx::tma_load_5d(c.stage_s + size_t(stage) * kRdbTileBytes, &tmap_in, fb, args.cin_off + 32 * g, pc.x0 - 1, row,
+                             band0, pc.b);
+          }
           if (++stage == args.stages) {
             stage = 0;
             phase ^= 1u;
@@ -777,27 +872,34 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
       });
     }
   } else if (warp <= 3) {
-    if (warp - 1 < NL && ptx::elect_one()) {  // (warp 3 of a two-layer kernel: idle, or the second producer above)
-      if (warp == 1) rdb_issuer<G, NL, 0>(args, c, sched);
-      if (warp == 2) rdb_issuer<G, NL, 1>(args, c, sched);
+    // (warp 3 of a two-layer kernel: idle, or the second producer above; PAIR: the peer issues nothing)
+    if (warp - 1 < NL && rank == 0 && ptx::elect_one()) {
+      if (warp == 1) rdb_issuer<G, NL, 0, PAIR>(args, c, sched);
+      if (warp == 2) rdb_issuer<G, NL, 1, PAIR>(args, c, sched);
       if constexpr (NL == 3) {
-        if (warp == 3) rdb_issuer<G, NL, 2>(args, c, sched);
+        if (warp == 3) rdb_issuer<G, NL, 2, PAIR>(args, c, sched);
       }
     }
   } else if (egroup < NL) {
     const int q = warp & 3;  // TMEM lane quarter this warp may read
-    if (egroup == 0) rdb_epilogue<G, NL, 0>(args, c, sched, q, lane);
-    if (egroup == 1) rdb_epilogue<G, NL, 1>(args, c, sched, q, lane);
+    if (egroup == 0) rdb_epilogue<G, NL, 0, PAIR>(args, c, sched, q, lane);
+    if (egroup == 1) rdb_epilogue<G, NL, 1, PAIR>(args, c, sched, q, lane);
     if constexpr (NL == 3) {
-      if (egroup == 2) rdb_epilogue<G, NL, 2>(args, c, sched, q, lane);
+      if (egroup == 2) rdb_epilogue<G, NL, 2, PAIR>(args, c, sched, q, lane);
     }
   }
 
   ptx::tc_fence_before();
-  __syncthreads();
+  if constexpr (PAIR)
+    ptx::cluster_sync();  // neither CTA may exit while the other can still multicast to it or arrive on it
+  else
+    __syncthreads();
   if (warp == 1) {
     ptx::tc_fence_after();
-    ptx::tmem_dealloc<512>(c.tmem_base);
+    if constexpr (PAIR)
+      ptx::tmem_dealloc_pair<512>(c.tmem_base);
+    else
+      ptx::tmem_dealloc<512>(c.tmem_base);
   }
 }
 

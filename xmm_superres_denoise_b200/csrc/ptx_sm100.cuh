@@ -268,6 +268,33 @@ __device__ __forceinline__ void tma_load_4d_pair(void* smem_dst, const CUtensorM
       "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
       : "memory");
 }
+// 5-D tiled load (the banded view of tma_load_5d) into THIS CTA's shared memory, completing on a barrier of either
+// CTA of the pair.
+__device__ __forceinline__ void tma_load_5d_pair(void* smem_dst, const CUtensorMap* m, uint32_t bar_cluster_addr,
+                                                 int c0, int c1, int c2, int c3, int c4) {
+  asm volatile(
+      "cp.async.bulk.tensor.5d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes "
+      "[%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
+      ::"r"(smem_u32(smem_dst)),
+      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
+      : "memory");
+}
+// umma_ss_lh for the pair (M = 256: the leader's A rows, then the peer's; each CTA's B holds half of the N rows).
+template <bool ACC>
+__device__ __forceinline__ void umma_ss_lh_pair(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
+                                                uint32_t idesc) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      ".reg .b64 da, db;\n\t"
+      "setp.ne.b32 p, %6, 0;\n\t"
+      "mov.b64 da, {%1, %2};\n\t"
+      "mov.b64 db, {%3, %4};\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t"
+      "}\n" ::"r"(tmem_d),
+      "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "n"(ACC ? 1 : 0)
+      : "memory");
+}
 // One warp of EACH CTA of the pair.
 template <int kCols>
 __device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_result) {

@@ -751,14 +751,16 @@ const char* rdb_blocker(const xmm_conv3x3_params* L, int n, const DeviceInfo& de
   return nullptr;
 }
 
-template <int G, int NL>
+// PAIR: clusters of two CTAs that share every MMA (conv3x3_rdb.cuh): each holds half of the weights, so 14 instead of
+// 5 TMA stages fit next to conv4 + conv5's.
+template <int G, int NL, bool PAIR>
 int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo& dev, cudaStream_t stream) {
   RdbArgs a{};
   uint32_t off = 0;
   for (int l = 0; l < NL; ++l) {
     const xmm_conv3x3_params& p = L[l];
     a.layer[l].wblob = p.wblob_row;
-    a.layer[l].w_bytes = uint32_t(p.cin / 32) * 9u * uint32_t(kRdbTapBytes);
+    a.layer[l].w_bytes = uint32_t(p.cin / 32) * 9u * uint32_t(kRdbTapBytes) / (PAIR ? 2u : 1u);
     a.layer[l].smem_off = off;
     off += (a.layer[l].w_bytes + 128u + 1023u) & ~1023u;
     a.layer[l].lrelu_slope = p.lrelu_slope;
@@ -775,7 +777,8 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
   a.width = L[0].width;
   a.band_h = a.height / 2;
   a.tiles_x = rdb_tiles_x<NL>(a.width);
-  a.total_rows = (long long)a.batch * a.tiles_x * a.band_h;
+  const long long ncols = (long long)a.batch * a.tiles_x;
+  a.total_rows = (PAIR ? (ncols + 1) / 2 : ncols) * a.band_h;  // (pairs: rows of the pair-columns)
   a.s0 = pl.s0; a.s1 = pl.s1; a.s2 = pl.s2;
   a.r1 = static_cast<const __nv_bfloat16*>(pl.r1); a.r1_ctot = pl.r1_ctot; a.r1_coff = pl.r1_coff;
   a.r2 = static_cast<const __nv_bfloat16*>(pl.r2); a.r2_ctot = pl.r2_ctot; a.r2_coff = pl.r2_coff;
@@ -789,60 +792,111 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
   a.ring0 = NL == 3 ? 5 : 2;  // (two fused layers: x4 is read one row behind its producer -- two tiles, one more TMA stage)
   a.ring1 = NL == 3 ? 3 : 0;
   a.stages = tiles - a.ring0 - a.ring1;
-  if (a.stages > kRdbMaxStages) a.stages = kRdbMaxStages;
+  if (a.stages > kRdbLRing<PAIR>) a.stages = kRdbLRing<PAIR>;
   static const int stages_env = env_int("XMM_RDB_STAGES", 0);
   if (stages_env > 0 && stages_env < a.stages) a.stages = stages_env;
   if (a.stages < 3) return fail(XMM_ERR_UNSUPPORTED_SHAPE, "conv3x3 (fused dense block): %d pipeline stages fit", a.stages);
   // measured (profiles/r02_rdb_v8_split_producers.log): 3.08 ms per block against 2.87 ms with one producer and one shared
-  // ring -- rings of 3 + 2 stages are less elastic than one of 5 -- so it is off
+  // ring -- rings of 3 + 2 stages are less elastic than one of 5 -- so it is off (and not built for pairs)
   static const int split_env = env_int("XMM_RDB_SPLIT_PRODUCERS", 0);
-  a.split_producers = (NL == 2 && split_env && a.stages >= 4) ? 1 : 0;
+  a.split_producers = (!PAIR && NL == 2 && split_env && a.stages >= 4) ? 1 : 0;
   CUtensorMap tmap;
   int rc = cached_band_tmap(&tmap, L[0].in, a.batch, a.height, a.width, L[0].in_ctot, a.band_h, 2, 32, kRdbBoxPx, 2);
   if (rc != XMM_OK) return rc;
-  rc = ensure_max_smem(reinterpret_cast<const void*>(conv3x3_rdb_kernel<G, NL>), dev);
+  const void* kernel = reinterpret_cast<const void*>(conv3x3_rdb_kernel<G, NL, PAIR>);
+  rc = ensure_max_smem(kernel, dev);
   if (rc != XMM_OK) return rc;
   const size_t smem = 1024 + size_t(a.w_total) + size_t(a.stages + a.ring0 + a.ring1) * kRdbTileBytes + kBarBytes;
   static const int max_ctas = env_int("XMM_RDB_MAX_CTAS", 0);
-  int grid = a.total_rows < dev.sm_count ? int(a.total_rows) : dev.sm_count;
-  if (max_ctas > 0 && grid > max_ctas) grid = max_ctas;
+  cudaLaunchConfig_t cfg{};
+  cudaLaunchAttribute attr[1];
+  cfg.blockDim = dim3(kRdbThreads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  long long grid;
+  if constexpr (PAIR) {
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    // persistent: every pair must be resident at once (a second wave would double the time), so the grid is what the
+    // device can co-schedule as clusters, not the SM count
+    static int max_clusters = 0;
+    if (max_clusters == 0) {
+      cfg.gridDim = dim3(unsigned(2 * dev.sm_count));
+      XMM_CUDA_OK(cudaOccupancyMaxActiveClusters(&max_clusters, conv3x3_rdb_kernel<G, NL, PAIR>, &cfg));
+      if (max_clusters < 1) return fail(XMM_ERR_UNSUPPORTED_SHAPE, "conv3x3 (fused dense block): no CTA pair fits an SM pair");
+    }
+    long long pairs = a.total_rows < max_clusters ? a.total_rows : max_clusters;
+    if (max_ctas > 0 && pairs > max_ctas / 2) pairs = max_ctas / 2 > 0 ? max_ctas / 2 : 1;
+    grid = 2 * pairs;
+  } else {
+    grid = a.total_rows < dev.sm_count ? a.total_rows : dev.sm_count;
+    if (max_ctas > 0 && grid > max_ctas) grid = max_ctas;
+  }
+  cfg.gridDim = dim3(unsigned(grid));
   // XMM_RDB_PROF=1 (developer): per-CTA cycle counters of the issuer and the two epilogue groups, printed per launch
   static const int prof_env = XMM_RDB_PROFILE ? env_int("XMM_RDB_PROF", 0) : 0;
   static long long* prof_dev = nullptr;
+  constexpr size_t kProfBytes = kRdbProfSlots * sizeof(long long) * 1024;
   if (prof_env) {
-    if (prof_dev == nullptr) XMM_CUDA_OK(cudaMalloc(&prof_dev, 16 * sizeof(long long) * 1024));
-    XMM_CUDA_OK(cudaMemsetAsync(prof_dev, 0, 16 * sizeof(long long) * 1024, stream));
+    if (prof_dev == nullptr) XMM_CUDA_OK(cudaMalloc(&prof_dev, kProfBytes));
+    XMM_CUDA_OK(cudaMemsetAsync(prof_dev, 0, kProfBytes, stream));
     a.prof = prof_dev;
   }
-  conv3x3_rdb_kernel<G, NL><<<grid, kRdbThreads, smem, stream>>>(tmap, a);
-  XMM_CUDA_OK(cudaGetLastError());
+  if constexpr (PAIR) {
+    XMM_CUDA_OK(cudaLaunchKernelEx(&cfg, conv3x3_rdb_kernel<G, NL, PAIR>, tmap, a));
+  } else {
+    conv3x3_rdb_kernel<G, NL, PAIR><<<cfg.gridDim, kRdbThreads, smem, stream>>>(tmap, a);
+    XMM_CUDA_OK(cudaGetLastError());
+  }
   if (prof_env) {
     XMM_CUDA_OK(cudaStreamSynchronize(stream));
-    std::vector<long long> h(size_t(grid) * 16);
+    std::vector<long long> h(size_t(grid) * kRdbProfSlots);
     XMM_CUDA_OK(cudaMemcpy(h.data(), prof_dev, h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-    static const char* names[16] = {"issuer total", "issuer wait drained", "issuer wait TMA", "issuer wait map row",
-                                    "epi0 total", "epi0 wait row complete", "epi0 wait map slot", "epi0 rows",
-                                    "epi1 total", "epi1 wait row complete", "epi1 wait map slot", "epi1 rows",
-                                    "epi0 drain (ld+st+arrive)", "epi0 math+pack", "epi0 map write+fence+arrive", "epi0 global store"};
-    fprintf(stderr, "conv3x3_rdb<%d,%d> grid %d stages %d:", G, NL, grid, a.stages);
-    for (int k = 0; k < 16; ++k) {
+    static const char* names[kRdbProfSlots] = {
+        "issuer total", "issuer wait drained", "issuer wait TMA", "issuer wait map row",
+        "epi0 total", "epi0 wait row complete", "epi0 wait map slot", "epi0 rows",
+        "epi1 total", "epi1 wait row complete", "epi1 wait map slot", "epi1 rows",
+        "epi0 drain (ld+st+arrive)", "epi0 math+pack", "epi0 map write+fence+arrive", "epi0 global store",
+        "epi1 drain (ld+st+arrive)", "epi1 math+residuals+pack", "epi1 map write (none)", "epi1 global store",
+        "", "", "", ""};
+    fprintf(stderr, "conv3x3_rdb<%d,%d%s> grid %lld stages %d:", G, NL, PAIR ? ",pair" : "", grid, a.stages);
+    for (int k = 0; k < 20; ++k) {
+      // (the issuer counters: of the CTAs that issue -- in pairs, the leaders)
       double sum = 0;
-      for (int c = 0; c < grid; ++c) sum += double(h[size_t(c) * 16 + k]);
-      fprintf(stderr, " %s %.0f;", names[k], sum / grid);
+      int n = 0;
+      for (long long c = 0; c < grid; ++c)
+        if (k >= 4 || !PAIR || c % 2 == 0) {
+          sum += double(h[size_t(c) * kRdbProfSlots + k]);
+          ++n;
+        }
+      fprintf(stderr, " %s %.0f;", names[k], sum / n);
     }
     fprintf(stderr, "\n");
   }
   return XMM_OK;
 }
 
+// Whether conv4..conv5 run as CTA pairs: XMM_RDB_PAIR = 0 / 1 (default 1, measured: DESIGN 4.3c), or per call the
+// XMM_CHAIN_RDB_PAIR / XMM_CHAIN_RDB_SINGLE flags.
+bool rdb_pair(int mode_flags) {
+  if (mode_flags & XMM_CHAIN_RDB_PAIR) return true;
+  if (mode_flags & XMM_CHAIN_RDB_SINGLE) return false;
+  static const int pair_env = env_int("XMM_RDB_PAIR", 1);
+  return pair_env != 0;
+}
+
 // conv1..conv3 in one launch, conv4..conv5 in a second one.  skip_dead: x4 is read by nobody after this block
 // (inference), so it is never written.
-int launch_rdb_block(const xmm_conv3x3_params* L, bool skip_dead, const DeviceInfo& dev, cudaStream_t stream) {
+int launch_rdb_block(const xmm_conv3x3_params* L, bool skip_dead, bool pair, const DeviceInfo& dev, cudaStream_t stream) {
   const bool store_a[3] = {true, true, true};
-  int rc = launch_rdb<1, 3>(L, store_a, dev, stream);
+  int rc = launch_rdb<1, 3, false>(L, store_a, dev, stream);
   if (rc != XMM_OK) return rc;
   const bool store_b[2] = {!skip_dead, true};
-  return launch_rdb<4, 2>(L + 3, store_b, dev, stream);
+  return pair ? launch_rdb<4, 2, true>(L + 3, store_b, dev, stream) : launch_rdb<4, 2, false>(L + 3, store_b, dev, stream);
 }
 
 extern "C" int xmm_set_sm_reserve(int sms) {
@@ -861,8 +915,11 @@ extern "C" int xmm_conv3x3_chain_bf16(const xmm_conv3x3_params* layers, int nlay
   g_last_chain_launches = 0;
   const int mode = mode_flags & 0xff;
   const bool skip_dead = (mode_flags & XMM_CHAIN_SKIP_DEAD_STORES) != 0;
-  XMM_REQUIRE(mode >= 0 && mode <= 3 && (mode_flags & ~(0xff | XMM_CHAIN_SKIP_DEAD_STORES)) == 0,
-              "conv3x3_chain: mode must be 0 (auto), 1 (pipelined), 2 (layer by layer) or 3 (fused dense block)");
+  constexpr int kFlags = XMM_CHAIN_SKIP_DEAD_STORES | XMM_CHAIN_RDB_PAIR | XMM_CHAIN_RDB_SINGLE;
+  XMM_REQUIRE(mode >= 0 && mode <= 3 && (mode_flags & ~(0xff | kFlags)) == 0 &&
+                  (mode_flags & (XMM_CHAIN_RDB_PAIR | XMM_CHAIN_RDB_SINGLE)) != (XMM_CHAIN_RDB_PAIR | XMM_CHAIN_RDB_SINGLE),
+              "conv3x3_chain: mode must be 0 (auto), 1 (pipelined), 2 (layer by layer) or 3 (fused dense block), with at most "
+              "one of the pair / single flags");
   DeviceInfo dev;
   int rc = require_sm100(&dev);
   if (rc != XMM_OK) return rc;
@@ -877,7 +934,7 @@ extern "C" int xmm_conv3x3_chain_bf16(const xmm_conv3x3_params* layers, int nlay
     const char* why_not = rdb_blocker(layers, nlayers, dev);
     if (why_not == nullptr) {
       g_last_chain_launches = 2;
-      return launch_rdb_block(layers, skip_dead, dev, s);
+      return launch_rdb_block(layers, skip_dead, rdb_pair(mode_flags), dev, s);
     }
     if (mode == 3) return fail(XMM_ERR_UNSUPPORTED_SHAPE, "conv3x3_chain: cannot fuse the dense block (%s)", why_not);
   }

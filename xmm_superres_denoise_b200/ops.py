@@ -108,6 +108,7 @@ _TORCH_FWD_KEYS = {"lrelu", "s0", "r1", "r1_coff", "s1", "r2", "r2_coff", "s2", 
 
 CHAIN_AUTO, CHAIN_PIPELINED, CHAIN_LAYER_BY_LAYER, CHAIN_FUSED = 0, 1, 2, 3
 CHAIN_SKIP_DEAD_STORES = 0x100  # flag: outputs of layers 1..n-1 are not read after the call (inference)
+CHAIN_RDB_PAIR, CHAIN_RDB_SINGLE = 0x200, 0x400  # flags: conv4..conv5 of the fused block as CTA pairs / single CTAs
 _chain_ws: dict = {}
 _chain_ws_retired: list = []  # outgrown workspaces stay allocated: a captured CUDA graph may still hold their address
 
@@ -118,7 +119,7 @@ def conv3x3_chain(layers, mode: int = CHAIN_AUTO) -> None:
     calling conv3x3 on them in order (up to fp32 summation order).  mode: CHAIN_AUTO (the fused dense-block kernels
     where the layers qualify, else layer by layer) / CHAIN_PIPELINED (one launch, layers pipelined over SM groups) /
     CHAIN_LAYER_BY_LAYER / CHAIN_FUSED (error if the layers are not a dense block), optionally
-    ``| CHAIN_SKIP_DEAD_STORES``."""
+    ``| CHAIN_SKIP_DEAD_STORES`` and ``| CHAIN_RDB_PAIR`` or ``| CHAIN_RDB_SINGLE``."""
     n = len(layers)
     arr = (Conv3x3Params * n)()
     for p, (a, kw) in zip(arr, layers):
