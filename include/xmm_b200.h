@@ -141,9 +141,9 @@ int xmm_conv3x3_bf16(const xmm_conv3x3_params* p, void* stream);
  * XMM_CHAIN_SKIP_DEAD_STORES: the caller will not read the outputs of layers 1..n-1 after this call (inference);
  *         outputs that no later launch of the chain reads need not be written (the fused form never writes x4).   */
 #define XMM_CHAIN_SKIP_DEAD_STORES 0x100
-/* XMM_CHAIN_RDB_PAIR / XMM_CHAIN_RDB_SINGLE (mode 0 / 3, at most one): run conv4..conv5 of the fused dense block as
- *         CTA pairs (two SMs share every MMA, each holding half of the weights) / as single CTAs, for this call,
- *         whatever XMM_RDB_PAIR selects.  Both forms compute the same bits.                                     */
+/* XMM_CHAIN_RDB_PAIR / XMM_CHAIN_RDB_SINGLE (mode 0 / 3, at most one): run both kernels of the fused dense block
+ *         (conv1..conv3, conv4..conv5) as CTA pairs (two SMs share every MMA, each holding half of the weights) / as
+ *         single CTAs, for this call, whatever XMM_RDB_PAIR selects.  Both forms compute the same bits.            */
 #define XMM_CHAIN_RDB_PAIR 0x200
 #define XMM_CHAIN_RDB_SINGLE 0x400
 size_t xmm_conv3x3_chain_workspace_bytes(int nlayers, int batch, int height);

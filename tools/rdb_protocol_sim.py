@@ -3,7 +3,8 @@ issuer, tensor pipe, two epilogue groups -- over the walk restated in tests/test
 and out-of-protocol barrier use before any GPU time is spent.  Pair mode (simulate_pair): the CTA-pair form of
 conv4 + conv5 -- two producers feeding the leader's landed barriers, count-8 drained / map-row barriers, multicast
 commits, 14 stages, landed rings of 16 -- where every arrival also checks that it lands in the phase it is meant
-for (a parity wait cannot tell a phase from the one two ahead).  python tools/rdb_protocol_sim.py"""
+for (a parity wait cannot tell a phase from the one two ahead).  The pair form of conv1..conv3 (simulate_pair, nl = 3)
+reads x0 from a ring that each row enters once, and every wait checks its phase as well.  python tools/rdb_protocol_sim.py"""
 import os
 import sys
 from collections import deque
@@ -30,6 +31,12 @@ class Bar:
 
     def ready(self, parity):
         return (self.phase & 1) != parity
+
+    def wait(self, use):
+        """a parity wait for the completion of phase `use` (-1: the phase before the first, complete from the start);
+        a parity cannot tell phase u from u + 2, so the barrier must be in phase use or use + 1 whenever it is polled"""
+        assert use <= self.phase <= use + 1, f"{self.name}: waiting for phase {use} in phase {self.phase}"
+        return self.ready(use & 1)
 
 
 def layer_steps(pieces, nl, l):
@@ -191,26 +198,39 @@ def simulate(nl, g, pieces, stages, verbose=False):
     return True, ticks
 
 
-def simulate_pair(g, pieces2, stages, lring=16):
-    """Two fused layers (conv4 + conv5) as a CTA pair; pieces2 = (rank 0's pieces, rank 1's pieces)."""
-    nl = 2
+def simulate_pair(g, pieces2, stages, lring=16, nl=2):
+    """The CTA-pair forms; pieces2 = (rank 0's pieces, rank 1's pieces).  nl = 2: conv4 + conv5 (G = 4) -- the
+    walk-order stage ring, per-layer landed rings of `lring`.  nl = 3: conv1..conv3 (G = 1) -- the x0 ring of `stages`
+    row tiles, each x0 row loaded once and released by its last reader.  Every wait checks that the barrier is in the
+    phase it waits for or the one after it (a parity wait passes early on the phase before it and never passes two
+    phases after it); every arrival checks that it lands in the phase it is meant for."""
+    xring = nl == 3
+    assert not xring or g == 1
     ring = RINGS[nl]
     steps2 = [list(walk(p, nl)) for p in pieces2]
     # both CTAs take the same walk: pieces, rows, flush steps (only b / x0 / the owned pixels differ)
     assert [s[:6] for s in steps2[0]] == [s[:6] for s in steps2[1]]
     pieces = pieces2[0]
-    # leader: lfull (the leader's arrive.expect_tx + one load per CTA), tdrain / mfull (4 warps per CTA)
+    # leader: full barriers (the leader's arrive.expect_tx + one load per CTA), tdrain / mfull (4 warps per CTA)
     lfull = [[Bar(3, f"lfull{l}.{s}") for s in range(lring)] for l in range(nl)]
+    xfull = [Bar(3, f"xfull{s}") for s in range(stages)]
     tdrain = [Bar(8, f"tdrain{l}") for l in range(nl)]
-    mfull = [Bar(8, f"mfull0.{s}") for s in range(ring[0])]
+    mfull = [[Bar(8, f"mfull{m}.{s}") for s in range(ring[m])] for m in range(nl - 1)]
     # per CTA: targets of the multicast commits
     empty = [[Bar(1, f"empty{s}@{c}") for s in range(stages)] for c in range(2)]
     tfull = [[Bar(1, f"tfull{l}@{c}") for l in range(nl)] for c in range(2)]
-    mempty = [[Bar(1, f"mempty0.{s}@{c}") for s in range(ring[0])] for c in range(2)]
+    mempty = [[[Bar(1, f"mempty{m}.{s}@{c}") for s in range(ring[m])] for m in range(nl - 1)] for c in range(2)]
     lstage = [[[None] * lring for _ in range(nl)] for _ in range(2)]
+    xrow = [[None] * stages for _ in range(2)]   # (piece, row) each CTA's x0 ring slot holds
+    xbase = [0]                                  # x0 ring: sequence number of each piece's first row, ra - nl
+    for pc in pieces:
+        xbase.append(xbase[-1] + (pc["rb"] - pc["ra"]) + 2 * nl)
     pipes = [deque() for _ in range(nl)]
     tma = deque()
     assert stages <= lring
+
+    def latency(c, k):  # loads land out of order
+        return 3 + c + (5 * k) % 7
 
     def producer(c):
         stage, phase, fill = 0, 0, 0
@@ -219,18 +239,31 @@ def simulate_pair(g, pieces2, stages, lring=16):
             if flush:
                 continue
             for _ in range(g):
-                while not empty[c][stage].ready(phase ^ 1):
+                while not empty[c][stage].wait(fill // stages - 1):
                     yield ("empty", c, stage)
                 k = fills[l] % lring
                 lstage[c][l][k] = stage
                 if c == 0:
                     lfull[l][k].arrive(fills[l] // lring)  # arrive.expect_tx for both CTAs' bytes
-                tma.append([3 + c, lfull[l][k], fills[l] // lring])
+                tma.append([latency(c, fill), lfull[l][k], fills[l] // lring])
                 fills[l] += 1
                 fill += 1
                 stage += 1
                 if stage == stages:
                     stage, phase = 0, phase ^ 1
+
+    def x0_producer(c):
+        sq = 0
+        for p, pc in enumerate(pieces2[c]):
+            for r in range(pc["ra"] - nl, pc["rb"] + nl):
+                slot = sq % stages
+                while not empty[c][slot].wait(sq // stages - 1):
+                    yield ("empty", c, slot)
+                xrow[c][slot] = (p, r)
+                if c == 0:
+                    xfull[slot].arrive(sq // stages)  # arrive.expect_tx for both CTAs' bytes
+                tma.append([latency(c, sq), xfull[slot], sq // stages])
+                sq += 1
 
     def multicast(bars, phase):
         return ("commit", [(b, phase) for b in bars])
@@ -241,25 +274,47 @@ def simulate_pair(g, pieces2, stages, lring=16):
         for (p, r, flush, n, seq) in layer_steps(pieces, nl, l):
             pc = pieces[p]
             if n > 0:
-                while not tdrain[l].ready((n - 1) & 1):
+                while not tdrain[l].wait(n - 1):
                     yield ("tdrain", l, n)
             if not flush:
-                if l == 1:  # the in-CTA map first (NL == 2)
-                    sq = seq[0] + (r - (pc["ra"] - (nl - 1)))
-                    slot = sq % ring[0]
-                    while not mfull[slot].ready((sq // ring[0]) & 1):
-                        yield ("mfull", 0, sq)
-                    pipes[l].append(("mma",))
-                    pipes[l].append(multicast([mempty[0][slot], mempty[1][slot]], sq // ring[0]))
-                for _ in range(g):
-                    k = fills % lring
-                    while not lfull[l][k].ready((fills // lring) & 1):
-                        yield ("lfull", l, fills)
-                    st = lstage[0][l][k]
-                    assert lstage[1][l][k] == st, "the CTAs of a pair loaded a chunk into different stages"
-                    fills += 1
-                    pipes[l].append(("mma",))
-                    pipes[l].append(("commit_stage", st))
+                # K order: two fused layers take the in-CTA map first, three take x0 first
+                for kind in (("map", "global") if nl == 2 else ("global", "map")):
+                    if kind == "map":
+                        for m in range(l):
+                            sq = seq[m] + (r - (pc["ra"] - (nl - 1 - m)))
+                            slot = sq % ring[m]
+                            while not mfull[m][slot].wait(sq // ring[m]):
+                                yield ("mfull", m, sq)
+                            pipes[l].append(("mma",))
+                            if l == nl - 1 or r < pc["ra"] - e or r > pc["rb"] + e - 1:
+                                pipes[l].append(multicast([mempty[0][m][slot], mempty[1][m][slot]], sq // ring[m]))
+                    elif xring:
+                        if r == pc["ra"] - e - 1:
+                            # a piece's first step follows flush steps: before the row can be given back, the layers
+                            # before this one must have read it -- their map rows r are written (their steps on r + 1)
+                            for m in range(l):
+                                sq = seq[m] + (r - (pc["ra"] - (nl - 1 - m)))
+                                while not mfull[m][sq % ring[m]].wait(sq // ring[m]):
+                                    yield ("mfull", m, sq)
+                        sq = xbase[p] + (r - (pc["ra"] - nl))
+                        slot = sq % stages
+                        while not xfull[slot].wait(sq // stages):
+                            yield ("xfull", l, sq)
+                        assert xrow[0][slot] == xrow[1][slot] == (p, r), (l, p, r, xrow[0][slot], xrow[1][slot])
+                        pipes[l].append(("mma",))
+                        # the last layer that reads the row gives the slot back
+                        if l == nl - 1 or r < pc["ra"] - e or r > pc["rb"] + e - 1:
+                            pipes[l].append(multicast([empty[0][slot], empty[1][slot]], sq // stages))
+                    else:
+                        for _ in range(g):
+                            k = fills % lring
+                            while not lfull[l][k].wait(fills // lring):
+                                yield ("lfull", l, fills)
+                            st = lstage[0][l][k]
+                            assert lstage[1][l][k] == st, "the CTAs of a pair loaded a chunk into different stages"
+                            fills += 1
+                            pipes[l].append(("mma",))
+                            pipes[l].append(("commit_stage", st))
             pipes[l].append(multicast([tfull[0][l], tfull[1][l]], n))
 
     stage_commits = [0] * stages
@@ -270,7 +325,7 @@ def simulate_pair(g, pieces2, stages, lring=16):
             pc = pieces2[c][p]
             j = r - 1
             real = pc["ra"] - e <= j < pc["rb"] + e
-            while not tfull[c][l].ready(n & 1):
+            while not tfull[c][l].wait(n):
                 yield ("tfull", c, l, n)
             for _ in range(4):
                 tdrain[l].arrive(n)
@@ -278,12 +333,12 @@ def simulate_pair(g, pieces2, stages, lring=16):
                 continue
             sq = seq[l] + (j - (pc["ra"] - e))
             slot = sq % ring[l]
-            while not mempty[c][slot].ready(((sq // ring[l]) & 1) ^ 1):
-                yield ("mempty", c, sq)
+            while not mempty[c][l][slot].wait(sq // ring[l] - 1):
+                yield ("mempty", c, l, sq)
             for _ in range(4):
-                mfull[slot].arrive(sq // ring[l])
+                mfull[l][slot].arrive(sq // ring[l])
 
-    agents = {"producer0": producer(0), "producer1": producer(1)}
+    agents = {f"producer{c}": (x0_producer(c) if xring else producer(c)) for c in range(2)}
     for l in range(nl):
         agents[f"issuer{l}"] = issuer(l)
         for c in range(2):
@@ -352,6 +407,19 @@ def main():
             print(f"pair NL=2 G=4 batch={batch} band_h={band_h} W={width} pairs={pairs} pair={u}: "
                   f"{'ok, ticks ' + str(info) if ok else 'DEADLOCK ' + str(info)}")
             ok_all &= ok
+    # CTA pairs: conv1..conv3 with the x0 ring (11 rows; 4, the launcher's minimum); band_h 4 and 5: pieces shorter
+    # than the ring, whose edge rows the later layers skip
+    for batch, band_h, width, grid in [(1, 4, 416, 148), (3, 20, 416, 148), (64, 208, 416, 148), (1, 208, 416, 148),
+                                       (3, 5, 200, 148), (2, 9, 64, 13 * 2), (3, 4, 416, 4)]:
+        ntx = tiles_x(width, 3)
+        pairs = min(grid // 2, (batch * ntx + 1) // 2 * band_h)
+        for u in sorted(set([0, 1, pairs // 2, pairs - 1])):
+            pcs = [pair_pieces(2 * u + rank, 2 * pairs, batch, band_h, width, 3) for rank in (0, 1)]
+            for xr in (11, 4):
+                ok, info = simulate_pair(1, pcs, xr, nl=3)
+                print(f"pair NL=3 G=1 x0 ring {xr} batch={batch} band_h={band_h} W={width} pairs={pairs} pair={u}: "
+                      f"{'ok, ticks ' + str(info) if ok else 'DEADLOCK ' + str(info)}")
+                ok_all &= ok
     sys.exit(0 if ok_all else 1)
 
 

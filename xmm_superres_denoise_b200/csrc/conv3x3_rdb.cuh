@@ -43,15 +43,26 @@
 // mbarriers.  Rule for every barrier here: its waiter observes EVERY phase (a parity wait two phases ahead passes at
 // once) -- hence per-layer barriers and per-layer roles; tools/rdb_protocol_sim.py models the whole protocol.
 //
-// CTA pairs (template PAIR; conv4 + conv5).  There the resident weights (164 KB) leave five TMA stages and the issuer
-// waits for chunks to land.  Two CTAs of a cluster run as a tcgen05 cta_group::2 pair: the leader's issuers issue
-// M = 256 MMAs (rows 0..127 = the leader's row tile, 128..255 = the peer's) and each CTA holds a compacted HALF of every
-// (chunk, dx) group of the weight image (rank 0 rows 0..47, rank 1 rows 48..95, 3 KB per group), so 14 stages fit.
-// Each CTA keeps its own producer, stage ring, x4 ring, epilogue groups and TMEM lanes, and walks its own column of
-// the same pair-column (RdbSched<NL, true>): both CTAs take the same walk over the same stage count, so the stage and
-// ring-slot ids are the same in both and the leader's descriptors address both.  Both producers' loads complete on
-// the leader's `lfull`; the peer's epilogue warps arrive on the leader's `tdrain` / `mfull` (count 8); the leader's
-// commits (`empty`, `mempty`, `tfull`) are multicast to both CTAs.
+// CTA pairs (template PAIR; both kernels).  Single CTAs hold all the weights (164 KB for conv4 + conv5, 111 KB for
+// conv1..conv3), which leaves five TMA stages, and the issuers wait for chunks to land.  Two CTAs of a cluster run as
+// a tcgen05 cta_group::2 pair: the leader's issuers issue M = 256 MMAs (rows 0..127 = the leader's row tile,
+// 128..255 = the peer's) and each CTA holds a compacted HALF of every (chunk, dx) group of the weight image (rank 0
+// rows 0..47, rank 1 rows 48..95, 3 KB per group).  Each CTA keeps its own producer, stage ring, map rings, epilogue
+// groups and TMEM lanes, and walks its own column of the same pair-column (RdbSched<NL, true>): both CTAs take the
+// same walk over the same stage count, so the stage and ring-slot ids are the same in both and the leader's
+// descriptors address both.  Both producers' loads complete on the leader's full barriers; the peer's epilogue warps
+// arrive on the leader's `tdrain` / `mfull` (count 8); the leader's commits (`empty`, `mempty`, `tfull`) are
+// multicast to both CTAs.
+//   conv4 + conv5 (G = 4): 14 stages of the shared walk-order ring fit.
+//   conv1..conv3 (G = 1, the x0 ring, kRdbXRing): every input chunk is an x0 row, and the walk-order ring loads each
+// of them three times (once per layer).  The pair instead loads each x0 row of a piece ONCE, in row order, into a ring
+// of 11 row tiles that all three issuers read the way they read map rows: the slot comes from the row's sequence
+// number, `lfull[slot]` is the TMA transaction barrier and `empty[slot]` is released by the commit of the last layer
+// that reads the row (conv3 for [ra-1, rb], conv2 for ra-2 and rb+1, conv1 for ra-3 and rb+2).  For that release to
+// come after the earlier layers' reads, the first step of a piece of conv2 / conv3 waits for its map rows before it
+// reads x0.  The issuers that skip a piece's edge rows skip phases of their slots; tools/rdb_protocol_sim.py checks
+// that no wait can land in the wrong phase.  The K order of every layer (x0 first, then its maps) is that of the
+// single CTA, so the bits are the same.
 #pragma once
 #include <cstdio>
 
@@ -73,6 +84,10 @@ constexpr int kRdbMaxStages = 16;
 // stages <= kRdbLRing no parity wait can pass a phase early.  A single CTA fits <= 8 stages next to its weights.
 template <bool PAIR>
 constexpr int kRdbLRing = PAIR ? kRdbMaxStages : 8;
+// conv1..conv3 as a CTA pair: the stage ring is the x0 row ring (see the top of this file), `lfull` / `empty` are its
+// [stages] full / empty barriers and there is no `lstage`.
+template <int G, bool PAIR>
+constexpr bool kRdbXRing = PAIR && G == 1;
 constexpr int kRdbTapBytes = 32 * 64;             // one (dx, dy) block of a chunk: 32 output channels x 32 inputs
 constexpr int kRdbGroupBytes = 3 * kRdbTapBytes;  // one (chunk, dx) group of the row-hop image: 96 rows of 64 B
 constexpr int kRdbProfSlots = 24;                 // XMM_RDB_PROFILE counters per CTA
@@ -309,10 +324,12 @@ __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.
 // Shared-memory carve-up, identical in every thread.
 struct RdbCtx {
   uint8_t* w_s;        // weights + biases of every layer
-  uint8_t* stage_s;    // TMA stages (one ring shared by all layers, handed out in walk order)
+  uint8_t* stage_s;    // TMA stages (one ring shared by all layers, handed out in walk order; x0 ring: in row order)
   uint8_t* map_s[2];   // row tiles of the in-CTA maps
   uint64_t* lfull;     // [3][R] chunk k (mod R = kRdbLRing) of layer l has landed (waiter: issuer l)
+                       // (x0 ring: [R] the row in slot s has landed                (waiters: all issuers))
   uint64_t* empty;     // [stages] the MMAs that read the stage are done        (waiter: producer)
+                       // (x0 ring: ... the row's last reader is done)
   uint64_t* tfull;     // [NL] the row a step completes is in TMEM              (waiter: epilogue group l)
   uint64_t* tdrain;    // [NL] ... has been drained and its slot re-initialised (waiter: issuer l)
   uint64_t* mfull;     // [2][8] row tile of map m written                       (waiters: issuers m+1 ..)
@@ -369,6 +386,7 @@ __device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c,
   uint32_t fills = 0;  // chunks consumed so far
   uint32_t n = 0;      // steps taken so far
   int seq[2] = {0, 0}; // sequence number, in map m, of the current piece's first row
+  int xseq = 0;        // x0 ring: sequence number of the current piece's first x0 row, ra - NL
   for (int pi = 0; pi < sched.npieces; ++pi) {
     const RdbPiece pc = sched.get(pi);
     const int r_last = pc.rb + e;  // last step with MMAs; two flush steps follow
@@ -379,15 +397,36 @@ __device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c,
       if (r <= r_last) {
         const uint32_t d = c.tmem_base + uint32_t(L * kRdbSlotCols + rdb_phi(r - 1) * 32);
         auto global_chunks = [&]() {
+          if constexpr (kRdbXRing<G, PAIR>) {
+            // x0 row r of this piece, loaded once for all layers; the last layer that reads it gives the slot back.
+            // Every later step of a piece follows a step that waited for the map rows r - 1 (the earlier layers' steps
+            // on r, which read x0 row r), but the first one follows flush steps: it waits for its map rows r (the
+            // earlier layers' steps on r + 1) before it can release row r.
+            if (L > 0 && r == pc.ra - e - 1) {
 #pragma unroll
-          for (int g = 0; g < G; ++g) {
-            const int k = int(fills % kR);
-            rdb_wait_p(&c.lfull[L * kR + k], (fills / kR) & 1u, 3, L, k, prof, pw[1]);
-            const int stage = c.lstage[L * kR + k];
-            ++fills;
+              for (int m = 0; m < NM; ++m)
+                if (m < L) {
+                  const int sq = seq[m] + (r - (pc.ra - (NL - 1 - m)));
+                  rdb_wait_p(&c.mfull[m * 8 + sq % ring[m]], uint32_t(sq / ring[m]) & 1u, 4, L * 10 + m, sq, prof, pw[2]);
+                }
+            }
+            const int sq = xseq + (r - (pc.ra - NL));
+            const int slot = sq % args.stages;
+            rdb_wait_p(&c.lfull[slot], uint32_t(sq / args.stages) & 1u, 3, L, sq, prof, pw[1]);
             ptx::tc_fence_after();
-            issue6(d, a_lo0 + uint32_t(stage) * kTile16, b_l + uint32_t(g) * kChunk16);
-            commit(&c.empty[stage]);
+            issue6(d, a_lo0 + uint32_t(slot) * kTile16, b_l);
+            if (L == NL - 1 || r < pc.ra - e || r > pc.rb + e - 1) commit(&c.empty[slot]);
+          } else {
+#pragma unroll
+            for (int g = 0; g < G; ++g) {
+              const int k = int(fills % kR);
+              rdb_wait_p(&c.lfull[L * kR + k], (fills / kR) & 1u, 3, L, k, prof, pw[1]);
+              const int stage = c.lstage[L * kR + k];
+              ++fills;
+              ptx::tc_fence_after();
+              issue6(d, a_lo0 + uint32_t(stage) * kTile16, b_l + uint32_t(g) * kChunk16);
+              commit(&c.empty[stage]);
+            }
           }
         };
         auto map_chunks = [&]() {
@@ -418,6 +457,7 @@ __device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c,
     }
 #pragma unroll
     for (int m = 0; m < NM; ++m) seq[m] += (pc.rb - pc.ra) + 2 * (NL - 1 - m);
+    xseq += (pc.rb - pc.ra) + 2 * NL;
   }
   if (XMM_RDB_PROFILE && prof) {
     long long* o = args.prof + size_t(blockIdx.x) * kRdbProfSlots;
@@ -678,6 +718,40 @@ __device__ __forceinline__ void rdb_layer_producer(const CUtensorMap* tmap_in, c
   }
 }
 
+// (conv1..conv3 as a CTA pair) The x0 ring: every x0 row of a piece once, in row order, over the first layer's rows
+// [ra - NL, rb + NL - 1]; no walk.  No L2 prefetch: the ring runs 11 rows ahead by itself, and a dense block took
+// 2.73 ms with a prefetch three rows ahead against 2.66 ms without (profiles/r05_rdb_probe_ring_prefetch.log).  Slot and phase follow the row's sequence number, as in the issuers.  Both CTAs'
+// loads complete on the leader's lfull[slot], which the leader arms for both; each CTA waits for its own empty[slot]
+// (the multicast commit of the row's last reader).
+template <int NL>
+__device__ __forceinline__ void rdb_x0_producer(const CUtensorMap* tmap_in, const RdbArgs& args, const RdbCtx& c,
+                                                const RdbSched<NL, true>& sched) {
+  int slot = 0;
+  uint32_t phase = 0;
+  for (int pi = 0; pi < sched.npieces; ++pi) {
+    const RdbPiece pc = sched.get(pi);
+    for (int r = pc.ra - NL; r <= pc.rb + NL - 1; ++r) {
+      int row = r, band0 = 0;
+      if (r < 0) {
+        row = r + args.band_h;
+        band0 = -1;
+      } else if (r >= args.band_h) {
+        row = r - args.band_h;
+        band0 = 1;
+      }
+      rdb_wait_backoff(&c.empty[slot], phase ^ 1u, 1, 0, slot, uint32_t(args.backoff_ns));
+      uint64_t* fb = &c.lfull[slot];
+      if (sched.rank == 0) ptx::mbar_expect_tx(fb, 2 * kRdbTileData);
+      ptx::tma_load_5d_pair(c.stage_s + size_t(slot) * kRdbTileBytes, tmap_in, ptx::mapa(ptx::smem_u32(fb), 0),
+                            args.cin_off, pc.x0 - 1, row, band0, pc.b);
+      if (++slot == args.stages) {
+        slot = 0;
+        phase ^= 1u;
+      }
+    }
+  }
+}
+
 // G: feature maps read from global memory (x0 .. x_{G-1}); NL: fused layers.  Layer l (0-based) is conv_{G+l}: its K
 // chunks are the G global maps then the l maps produced in this CTA.
 // Warp roles (512 threads): warp 0 = TMA producer (the only role that follows the interleaved walk: it decides the
@@ -691,8 +765,11 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
   static_assert(NL * kRdbSlotCols <= 512, "accumulators exceed TMEM");
   constexpr int NM = NL - 1;  // in-CTA maps
   constexpr int kR = kRdbLRing<PAIR>;
+  constexpr bool XR = kRdbXRing<G, PAIR>;
+  constexpr int kFull = XR ? kR : 3 * kR;   // lfull: per-layer landed rings, or the x0 ring's full barriers
+  constexpr int kStageIds = XR ? 0 : 3 * kR;  // lstage
   // lfull, empty, tfull, tdrain, mfull, mempty, w_bar; lstage; the TMEM address: the 1024 B the launcher reserves
-  static_assert((3 * kR + kR + 3 + 3 + 16 + 16 + 1) * 8 + 3 * kR * 4 + 4 <= 1024, "barrier block exceeds 1024 B");
+  static_assert((kFull + kR + 3 + 3 + 16 + 16 + 1) * 8 + kStageIds * 4 + 4 <= 1024, "barrier block exceeds 1024 B");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   RdbCtx c;
@@ -702,15 +779,15 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
   c.map_s[1] = c.map_s[0] + size_t(args.ring0) * kRdbTileBytes;
   uint8_t* after = c.map_s[1] + size_t(NM > 1 ? args.ring1 : 0) * kRdbTileBytes;
   uint64_t* bars = reinterpret_cast<uint64_t*>(after);
-  c.lfull = bars;              // 3 R
-  c.empty = c.lfull + 3 * kR;  // R
+  c.lfull = bars;              // 3 R (x0 ring: R)
+  c.empty = c.lfull + kFull;   // R
   c.tfull = c.empty + kR;      // 3
   c.tdrain = c.tfull + 3;      // 3
   c.mfull = c.tdrain + 3;      // 16
   c.mempty = c.mfull + 16;     // 16
   c.w_bar = c.mempty + 16;     // 1
-  c.lstage = reinterpret_cast<volatile int*>(c.w_bar + 1);  // 3 R ints
-  uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(const_cast<int*>(c.lstage) + 3 * kR);
+  c.lstage = reinterpret_cast<volatile int*>(c.w_bar + 1);  // 3 R ints (x0 ring: none)
+  uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(const_cast<int*>(c.lstage) + kStageIds);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -718,7 +795,7 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tmap_in);
-    for (int s = 0; s < NL * kR; ++s) ptx::mbar_init(&c.lfull[s], 1);
+    for (int s = 0; s < (XR ? kFull : NL * kR); ++s) ptx::mbar_init(&c.lfull[s], 1);
     for (int s = 0; s < args.stages; ++s) ptx::mbar_init(&c.empty[s], 1);
     for (int l = 0; l < NL; ++l) {
       ptx::mbar_init(&c.tfull[l], 1);
@@ -806,12 +883,17 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
         if (warp == 3) rdb_layer_producer<G, NL, 1>(&tmap_in, args, c, sched, ns0, args.stages - ns0);
       }
     }
+  } else if (XR && warp == 0) {
+    // ------------------------------------------------------------ TMA producer of the x0 ring (conv1..conv3 pair)
+    if constexpr (XR) {
+      if (ptx::elect_one()) rdb_x0_producer<NL>(&tmap_in, args, c, sched);
+    }
   } else if (warp == 0) {
     // ------------------------------------------------------------ TMA producer
     // PAIR: both CTAs' producers take the same walk over the same stage count, so they write the same stage ids into
     // lstage -- the leader's issuers address the peer's stages with the leader's ids.  Both loads of a chunk complete
     // on the leader's lfull, which the leader's producer arms for both.
-    if (ptx::elect_one()) {
+    if (!XR && ptx::elect_one()) {
       int stage = 0;
       uint32_t phase = 0;
       uint32_t fills[NL];  // chunks loaded for layer l so far

@@ -752,7 +752,7 @@ const char* rdb_blocker(const xmm_conv3x3_params* L, int n, const DeviceInfo& de
 }
 
 // PAIR: clusters of two CTAs that share every MMA (conv3x3_rdb.cuh): each holds half of the weights, so 14 instead of
-// 5 TMA stages fit next to conv4 + conv5's.
+// 5 TMA stages fit next to conv4 + conv5's, and an x0 ring of 11 rows next to conv1..conv3's.
 template <int G, int NL, bool PAIR>
 int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo& dev, cudaStream_t stream) {
   RdbArgs a{};
@@ -795,7 +795,10 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
   if (a.stages > kRdbLRing<PAIR>) a.stages = kRdbLRing<PAIR>;
   static const int stages_env = env_int("XMM_RDB_STAGES", 0);
   if (stages_env > 0 && stages_env < a.stages) a.stages = stages_env;
-  if (a.stages < 3) return fail(XMM_ERR_UNSUPPORTED_SHAPE, "conv3x3 (fused dense block): %d pipeline stages fit", a.stages);
+  // (the x0 ring holds the rows between the last layer's and the first layer's step: tools/rdb_protocol_sim.py)
+  const int min_stages = kRdbXRing<G, PAIR> ? 4 : 3;
+  if (a.stages < min_stages)
+    return fail(XMM_ERR_UNSUPPORTED_SHAPE, "conv3x3 (fused dense block): %d pipeline stages fit", a.stages);
   // measured (profiles/r02_rdb_v8_split_producers.log): 3.08 ms per block against 2.87 ms with one producer and one shared
   // ring -- rings of 3 + 2 stages are less elastic than one of 5 -- so it is off (and not built for pairs)
   static const int split_env = env_int("XMM_RDB_SPLIT_PRODUCERS", 0);
@@ -880,23 +883,23 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
   return XMM_OK;
 }
 
-// Whether conv4..conv5 run as CTA pairs: XMM_RDB_PAIR = 0 / 1 (default 1, measured: DESIGN 4.3c), or per call the
-// XMM_CHAIN_RDB_PAIR / XMM_CHAIN_RDB_SINGLE flags.
-bool rdb_pair(int mode_flags) {
-  if (mode_flags & XMM_CHAIN_RDB_PAIR) return true;
-  if (mode_flags & XMM_CHAIN_RDB_SINGLE) return false;
-  static const int pair_env = env_int("XMM_RDB_PAIR", 1);
-  return pair_env != 0;
+// Which fused kernels run as CTA pairs, a bit mask: bit 0 conv1..conv3, bit 1 conv4..conv5.  XMM_RDB_PAIR (default 3,
+// measured: DESIGN 4.3c), or per call the XMM_CHAIN_RDB_PAIR (both) / XMM_CHAIN_RDB_SINGLE (neither) flags.
+int rdb_pair(int mode_flags) {
+  if (mode_flags & XMM_CHAIN_RDB_PAIR) return 3;
+  if (mode_flags & XMM_CHAIN_RDB_SINGLE) return 0;
+  static const int pair_env = env_int("XMM_RDB_PAIR", 3);
+  return pair_env & 3;
 }
 
 // conv1..conv3 in one launch, conv4..conv5 in a second one.  skip_dead: x4 is read by nobody after this block
-// (inference), so it is never written.
-int launch_rdb_block(const xmm_conv3x3_params* L, bool skip_dead, bool pair, const DeviceInfo& dev, cudaStream_t stream) {
+// (inference), so it is never written.  pair: rdb_pair's mask.
+int launch_rdb_block(const xmm_conv3x3_params* L, bool skip_dead, int pair, const DeviceInfo& dev, cudaStream_t stream) {
   const bool store_a[3] = {true, true, true};
-  int rc = launch_rdb<1, 3, false>(L, store_a, dev, stream);
+  int rc = (pair & 1) ? launch_rdb<1, 3, true>(L, store_a, dev, stream) : launch_rdb<1, 3, false>(L, store_a, dev, stream);
   if (rc != XMM_OK) return rc;
   const bool store_b[2] = {!skip_dead, true};
-  return pair ? launch_rdb<4, 2, true>(L + 3, store_b, dev, stream) : launch_rdb<4, 2, false>(L + 3, store_b, dev, stream);
+  return (pair & 2) ? launch_rdb<4, 2, true>(L + 3, store_b, dev, stream) : launch_rdb<4, 2, false>(L + 3, store_b, dev, stream);
 }
 
 extern "C" int xmm_set_sm_reserve(int sms) {

@@ -108,7 +108,7 @@ _TORCH_FWD_KEYS = {"lrelu", "s0", "r1", "r1_coff", "s1", "r2", "r2_coff", "s2", 
 
 CHAIN_AUTO, CHAIN_PIPELINED, CHAIN_LAYER_BY_LAYER, CHAIN_FUSED = 0, 1, 2, 3
 CHAIN_SKIP_DEAD_STORES = 0x100  # flag: outputs of layers 1..n-1 are not read after the call (inference)
-CHAIN_RDB_PAIR, CHAIN_RDB_SINGLE = 0x200, 0x400  # flags: conv4..conv5 of the fused block as CTA pairs / single CTAs
+CHAIN_RDB_PAIR, CHAIN_RDB_SINGLE = 0x200, 0x400  # flags: both kernels of the fused block as CTA pairs / single CTAs
 _chain_ws: dict = {}
 _chain_ws_retired: list = []  # outgrown workspaces stay allocated: a captured CUDA graph may still hold their address
 
