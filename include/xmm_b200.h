@@ -120,6 +120,12 @@ typedef struct {
                          (cout == kc in {32, 64}, no pixel shuffle, height = nbands * band_h with 8 <= nbands <= 16,
                          weights resident next to >= 3 pipeline stages), the launch takes the row-hop form
                          (conv3x3_row.cuh); tap_mode 9 forces it (error if it does not qualify), 1..8 never use it. */
+  float* colsum_ws;   /* optional, with colsum: the deterministic form of the column sums.  colsum is then NOT written;
+                         the launch stores unscaled partial sums to colsum_ws_slots slots of 32 floats
+                         (xmm_det_slots(XMM_DET_CONV3X3, ...) of them at least), which must be zero on entry, and
+                         xmm_det_finalize adds them.  Not taken by the fused dense-block form of xmm_conv3x3_chain_bf16
+                         (column sums never are).                                                                 */
+  size_t colsum_ws_slots;
 } xmm_conv3x3_params;
 
 int xmm_conv3x3_bf16(const xmm_conv3x3_params* p, void* stream);
@@ -296,6 +302,12 @@ typedef struct {
 } xmm_colsum_segment;
 int xmm_colsum_multi_bf16(const void* in, int ctot, size_t npix, const xmm_colsum_segment* segs, int nseg,
                           void* stream);
+/* Deterministic form of xmm_colsum_multi_bf16: the segments' out / accumulate are not used; each CTA stores the
+ * unscaled sums of all segments' channels, concatenated in segment order, to its own slot of ws (ws_slots slots of
+ * sum(n) floats, xmm_det_slots(XMM_DET_COLSUM, ...) at least, zero on entry).  xmm_det_finalize applies the
+ * segments' scale and destination.                                                                                */
+int xmm_colsum_multi_det_bf16(const void* in, int ctot, size_t npix, const xmm_colsum_segment* segs, int nseg,
+                              float* ws, size_t ws_slots, void* stream);
 
 /* Weight/bias gradients of the two CUDA-core convolutions:
  *   R[o][c][tap] += sum_p s[o][p] * (V[p+off(tap)][c] + V2[p+off(tap)][c]);  S[o] += sum_p s[o][p]
@@ -308,8 +320,39 @@ typedef struct {
   float* r;                           /* fp32 [ns][channels][9], accumulated into              */
   float* ssum;                        /* fp32 [ns] or NULL, accumulated into                   */
   int batch, ns, height, width, channels; /* channels 32 or 64                                 */
+  float* ws;                          /* optional: deterministic form.  r / ssum are then NOT written; each CTA
+                                         stores R (ns*channels*9 floats) then S (ns floats, if ssum != NULL) to its
+                                         own slot of ns*channels*9 + ns floats (ws_slots slots,
+                                         xmm_det_slots(XMM_DET_EDGE_WGRAD, ...) at least, zero on entry)        */
+  size_t ws_slots;
 } xmm_edge_wgrad_params;
 int xmm_edge_wgrad(const xmm_edge_wgrad_params* p, void* stream);
+
+/* Deterministic gradient reductions ------------------------------------------------------ */
+/* The three reductions above (fused conv3x3 column sums, colsum, edge_wgrad) add per-warp / per-CTA partial sums with
+ * float atomics, in an order that depends on CTA timing.  Their deterministic forms store the partial sums to slots of
+ * a caller-owned workspace instead; one xmm_det_finalize launch then reduces any number of slot ranges, each in a
+ * fixed order, so the result is the same bits on every run (same device, same SM count and reserve, same shapes).
+ * Slots per call of a site, for xmm_set_sm_reserve's current value (the row length is the caller's: 32 floats for
+ * XMM_DET_CONV3X3, the segments' channels for XMM_DET_COLSUM, ns*channels*9 + ns for XMM_DET_EDGE_WGRAD);
+ * `channels` is the total channel count of the call (conv3x3: 32; edge_wgrad: its `channels`).                        */
+#define XMM_DET_CONV3X3 0
+#define XMM_DET_COLSUM 1
+#define XMM_DET_EDGE_WGRAD 2
+size_t xmm_det_slots(int site, int batch, int height, int width, int channels);
+
+/* dst_base[dst + i] = (accumulate ? dst_base[dst + i] : 0) + scale * sum_{k = 0..count-1} slots[k*stride + i], k in
+ * increasing order, for i < n; every slot read is left zero.  Jobs of one call must not share destinations.       */
+typedef struct {
+  float* slots;       /* count slots, stride floats apart                                                        */
+  int count, stride;
+  size_t dst;         /* destination: element offset from the call's dst_base                                    */
+  int n;
+  float scale;
+  int accumulate;
+} xmm_det_job;
+/* jobs_dev: device array of njobs jobs; max_n: the largest n among them.                                          */
+int xmm_det_finalize(const xmm_det_job* jobs_dev, int njobs, int max_n, float* dst_base, void* stream);
 
 /* Loss terms ------------------------------------------------------------------------- */
 /* Per-scale record kept on the device by the (MS-)SSIM kernels (12 floats). */

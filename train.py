@@ -13,11 +13,14 @@ routine and no Lightning branch.  What it keeps of the reference's configuration
   ``clamp_max`` (train.py:66-67: the normalisation maxima; ``max`` is accepted as an alias), [trainer] epochs;
 * ``res/configs/models.toml`` (train.py:35-36) when present in the working directory: the table named by
   [model].name supplies in/out channels, filters, residual_blocks, learning_rate and betas;
+* [trainer] deterministic (Lightning's ``Trainer(deterministic=...)``; ``--deterministic`` sets it too):
+  ``torch.use_deterministic_algorithms(True)`` and a seeded torch generator, so two runs of the same configuration on
+  the same GPU give the same weights bit for bit (the gradient all-reduce of multi-GPU runs is outside that promise);
 * ``res/configs/loss_functions.toml`` (train.py:45-53) when present: the [loss] percentages and, with
   ``use_scaling = true``, the [scaling.<dataset scaling>] table as ``sc_dict`` of ``create_loss``.  Without the file the
   [loss] table of the run file is used, unscaled (the scaling constants live in that file only).
 
-    python train.py fit run.toml [--synthetic] [--steps N]
+    python train.py fit run.toml [--synthetic] [--steps N] [--deterministic]
     python -m torch.distributed.run --nproc-per-node 8 train.py fit run.toml --synthetic
 """
 from __future__ import annotations
@@ -40,8 +43,10 @@ DEFAULTS = {
     "loss": {"l1": 0.5, "poisson": 0.5, "psnr": 0.0, "ssim": 0.0, "ms_ssim": 0.0, "use_scaling": True},
     "dataset": {"scaling": "sqrt", "lr": {"max": 0.0022336, "res": 416, "exps": [20]},
                 "hr": {"max": 0.0022336, "res": 416, "exp": 50}},
-    "trainer": {"epochs": 1},
+    "trainer": {"epochs": 1, "deterministic": False},
 }
+
+DETERMINISTIC_SEED = 0
 
 
 def _merge(base: dict, over: dict) -> dict:
@@ -84,6 +89,17 @@ def load_run_config(path):
     return cfg
 
 
+def configure_determinism(cfg: dict, flag: bool) -> bool:
+    """--deterministic or [trainer] deterministic = true: deterministic algorithms (the engine's reductions then run in
+    a fixed order, determinism.enabled) and a seeded torch generator (the initial weights).  Returns the mode."""
+    det = bool(flag) or bool(cfg["trainer"].get("deterministic", False))
+    if det:
+        os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")  # what torch asks of cuBLAS under the flag
+        torch.use_deterministic_algorithms(True)
+        torch.manual_seed(DETERMINISTIC_SEED)
+    return det
+
+
 def synthetic_batch(kind: str, batch: int, seed: int, cfg: dict, device):
     """Seeded Poisson count images of the reference shape (SURVEY.md 8d), normalised on the GPU."""
     from xmm_superres_denoise_b200 import ops
@@ -107,8 +123,11 @@ def main() -> None:
     ap.add_argument("config", nargs="?", default=None, help="run TOML (reference layout); defaults are the DeNoise setup")
     ap.add_argument("--synthetic", action="store_true")
     ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--deterministic", action="store_true",
+                    help="bit-reproducible training on one GPU ([trainer] deterministic = true does the same)")
     a = ap.parse_args()
     cfg = load_run_config(a.config)
+    configure_determinism(cfg, a.deterministic)
 
     import torch.distributed as dist
 

@@ -38,7 +38,7 @@ class Conv3x3Params(Structure):
                 ("r2", c_void_p), ("r2_ctot", c_int), ("r2_coff", c_int), ("s2", c_float),
                 ("out", c_void_p), ("out_ctot", c_int), ("out_coff", c_int),
                 ("pixel_shuffle", c_int), ("tap_mode", c_int), ("colsum", c_void_p), ("colsum_scale", c_float),
-                ("shuffle_stride", c_int), ("wblob_row", c_void_p)]
+                ("shuffle_stride", c_int), ("wblob_row", c_void_p), ("colsum_ws", c_void_p), ("colsum_ws_slots", c_size_t)]
 
 
 class NormalizeParams(Structure):
@@ -85,7 +85,8 @@ class WgradParams(Structure):
 class EdgeWgradParams(Structure):
     _fields_ = [("s", c_void_p), ("gate", c_void_p), ("v", c_void_p), ("v_ctot", c_int), ("v_coff", c_int),
                 ("v2", c_void_p), ("v2_ctot", c_int), ("v2_coff", c_int), ("r", c_void_p), ("ssum", c_void_p),
-                ("batch", c_int), ("ns", c_int), ("height", c_int), ("width", c_int), ("channels", c_int)]
+                ("batch", c_int), ("ns", c_int), ("height", c_int), ("width", c_int), ("channels", c_int),
+                ("ws", c_void_p), ("ws_slots", c_size_t)]
 
 
 class ScaleStats(Structure):
@@ -123,10 +124,18 @@ class ColsumSegment(Structure):
     _fields_ = [("c0", c_int), ("n", c_int), ("out", c_void_p), ("scale", c_float), ("accumulate", c_int)]
 
 
+class DetJob(Structure):
+    _fields_ = [("slots", c_void_p), ("count", c_int), ("stride", c_int), ("dst", c_size_t), ("n", c_int),
+                ("scale", c_float), ("accumulate", c_int)]
+
+
+DET_CONV3X3, DET_COLSUM, DET_EDGE_WGRAD = 0, 1, 2
+
+
 EXTRA_STRUCTS = {"xmm_colsum_segment": ColsumSegment, "xmm_prepare_counts_params": PrepareCountsParams, "xmm_scale_stats": ScaleStats, "xmm_ssim_stats_params": SsimStatsParams,
                  "xmm_ssim_grad_params": SsimGradParams, "xmm_msssim_finalize_params": MsssimFinalizeParams,
                  "xmm_wgrad_role": WgradRole, "xmm_wgrad_dst": WgradDst, "xmm_wgrad_params": WgradParams,
-                 "xmm_edge_wgrad_params": EdgeWgradParams}
+                 "xmm_edge_wgrad_params": EdgeWgradParams, "xmm_det_job": DetJob}
 
 # name -> (restype, argtypes); the non-GPU test-suite checks every name in include/xmm_b200.h is here
 # and exported by the shared object.
@@ -152,7 +161,11 @@ SIGNATURES = {
     "xmm_conv3x3_wgrad": (c_int, [POINTER(WgradParams), c_void_p]),
     "xmm_colsum_bf16": (c_int, [c_void_p, c_int, c_int, c_int, c_size_t, c_void_p, c_float, c_int, c_void_p]),
     "xmm_colsum_multi_bf16": (c_int, [c_void_p, c_int, c_size_t, POINTER(ColsumSegment), c_int, c_void_p]),
+    "xmm_colsum_multi_det_bf16": (c_int, [c_void_p, c_int, c_size_t, POINTER(ColsumSegment), c_int, c_void_p, c_size_t,
+                                          c_void_p]),
     "xmm_edge_wgrad": (c_int, [POINTER(EdgeWgradParams), c_void_p]),
+    "xmm_det_slots": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
+    "xmm_det_finalize": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "xmm_loss_workspace_floats": (c_size_t, []),
     "xmm_loss_reduce": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p]),
     "xmm_loss_grad": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),

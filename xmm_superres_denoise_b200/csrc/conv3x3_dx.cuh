@@ -62,6 +62,7 @@ constexpr int kDxTileW = 16;
 constexpr int kDxPatchH = kDxTileH + 2;
 constexpr int kDxEpiWarps = 8;
 constexpr int kDxThreads = 64 + 32 * kDxEpiWarps;
+static_assert(kDxEpiWarps <= kCsumWarpSlots, "one deterministic column-sum slot per epilogue warp");
 
 // G2: the eight epilogue warps form TWO GROUPS of four (one warp per TMEM lane quarter, all Cout columns each) that
 // work on DIFFERENT strips; the MMA warp alternates tiles between the two strips.  An epilogue pass costs a warp
@@ -683,7 +684,8 @@ conv3x3_dx_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_cons
       }
     }
     if (ptx::elect_one()) ptx::bulk_wait<0>();  // this warp's stores complete before the CTA (and its smem) goes away
-    if (args.epi.colsum != nullptr) colsum_flush<Cfg::kWarpCols>(args.epi, w.csum, w.col_w, lane);
+    if constexpr (NT == 32)  // (column sums are for cout = 32: xmm_conv3x3_bf16 rejects them elsewhere)
+      if (args.epi.colsum != nullptr) colsum_flush<Cfg::kWarpCols>(args.epi, w.csum, w.col_w, lane);
     if (warp == 2 && lane == 0) { XMM_PROF_FLUSH(4); XMM_PROF_FLUSH(5); }
 #ifdef XMM_CONV_PROFILE
     if (warp == 2 && lane == 0)

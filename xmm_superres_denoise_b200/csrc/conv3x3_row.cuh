@@ -43,6 +43,7 @@ constexpr int kRowPx = 8;
 constexpr int kRowPitch = kRowPx + 2;
 constexpr int kRowEpiWarps = 8;
 constexpr int kRowThreads = 64 + 32 * kRowEpiWarps;
+static_assert(kRowEpiWarps <= kCsumWarpSlots, "one deterministic column-sum slot per epilogue warp");
 // EVEN, like the accumulator slots: output rows alternate between the two epilogue groups, so with an even ring every
 // stage is always waited for by the SAME group, which therefore sees each of the barrier's phases.  (With 3 stages a
 // group saw every other phase of a stage's "landed" barrier: a parity wait two phases ahead passes at once, the

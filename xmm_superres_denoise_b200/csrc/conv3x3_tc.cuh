@@ -82,6 +82,12 @@ struct ConvEpilogue {
   // channel n (the data gradient dY a layer produces is also the bias gradient's integrand).  Cout = 32 kernels.
   float* colsum;
   float colsum_scale;
+  // Deterministic form of the same sums (colsum_ws != nullptr): every epilogue warp stores its unscaled column sums to
+  // its own slot, colsum_ws[(blockIdx.x * kCsumWarpSlots + warp - 2) * 32 + n], instead of adding them to colsum; a
+  // later xmm_det_finalize adds the slots in slot order.  The result depends only on which tiles each warp summed, so
+  // every kernel that flushes here hands its tiles to CTAs by a static schedule (a function of blockIdx.x and
+  // gridDim.x: conv3x3_tc, conv3x3_dx's DxRuns, conv3x3_row's RowSched, conv3x3_chain's item0 / item_step).
+  float* colsum_ws;
   float* img_out;
   const float* img_res;
   float* img_pre;   // optional copy of the un-clamped value (backward clamp gate)
@@ -268,15 +274,29 @@ __device__ __forceinline__ void conv_epilogue_32(const ConvEpilogue& e, const fl
   conv_epilogue_cols<NT, 32>(e, bias_s, v, col0, b, y, x, H, W, csum);
 }
 
-// End of a warp's life: add its lanes' column sums and publish them (one atomic per column and warp).
+// Deterministic column sums: slots per CTA, one per epilogue warp.  The epilogue warps of every kernel that calls
+// colsum_flush are warps 2 .. 2 + kCsumWarpSlots - 1; a warp that owns only some columns leaves the rest of its slot
+// as it found it (zero: xmm_det_finalize clears the slots it reads).
+constexpr int kCsumWarpSlots = 8;
+
+// End of a warp's life: add its lanes' column sums and publish them (one atomic per column and warp, or one store to
+// the warp's slot in the deterministic form).
 template <int NC>
 __device__ __forceinline__ void colsum_flush(const ConvEpilogue& e, float (&csum)[NC], int col0, int lane) {
+  static_assert(NC <= 32, "fused column sums are for cout = 32");
+  float* slot = e.colsum_ws == nullptr ? nullptr
+                : e.colsum_ws + (size_t(blockIdx.x) * kCsumWarpSlots + ((threadIdx.x >> 5) - 2)) * 32 + col0;
 #pragma unroll
   for (int i = 0; i < NC; ++i) {
     float x = csum[i];
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) x += __shfl_xor_sync(0xffffffffu, x, d);
-    if (lane == 0) atomicAdd(e.colsum + col0 + i, e.colsum_scale * x);
+    if (lane == 0) {
+      if (slot != nullptr)
+        slot[i] = x;
+      else
+        atomicAdd(e.colsum + col0 + i, e.colsum_scale * x);
+    }
   }
 }
 

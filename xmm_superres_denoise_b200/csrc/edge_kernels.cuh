@@ -348,6 +348,10 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
 // staged in shared memory; V is then streamed ONCE, 16 bytes (8 channels) per thread and pixel, and every thread
 // keeps an 8-channel x 9-tap accumulator block in registers: R[c][tap] += s[q - off(tap)] * V[q][c].  Warp
 // shuffles, a shared-memory pass and one atomicAdd per (channel, tap) and CTA finish the sum.
+// Deterministic form (ws != nullptr): the per-warp s sums are added in warp order instead of through a shared-memory
+// atomic, and CTA (x, y) stores its sums to its own slot ws[(y * gridDim.x + x) * (ns * C * 9 + ns) + ...]
+// (R[o][c][tap] at o * C * 9 + c * 9 + tap, S[o] at ns * C * 9 + o) instead of adding them to r / ssum; the slots are
+// added in slot order by xmm_det_finalize.
 // HBM-bound: C*2 (+C*2) + 4 (+4) bytes per pixel.
 struct EdgeWgradArgs {
   const float* s;     // [B][ns][H][W]
@@ -358,6 +362,8 @@ struct EdgeWgradArgs {
   float* ssum;        // [ns] or nullptr
   int batch, ns, height, width;
   int rows;           // image rows per CTA
+  float* ws;          // deterministic form: per-CTA slots (r and ssum are then not written; ssum != nullptr still
+                      // selects whether S is computed)
 };
 
 constexpr int kEdgeWgradThreads = 256;
@@ -372,12 +378,15 @@ __global__ void __launch_bounds__(kEdgeWgradThreads) edge_wgrad_kernel(const Edg
   float* s_tile = sm;                                        // [rows + 2][W + 2]
   float* red = sm + size_t(a.rows + 2) * pitch;              // [8 warps][C * 9]
   __shared__ float ssum_s;
+  __shared__ float ssum_w[kEdgeWgradThreads / 32];
   const int b = blockIdx.y;
   const int y0 = blockIdx.x * a.rows;
   const int nrows = (y0 + a.rows <= H) ? a.rows : H - y0;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int slot = tid / LP, cg = tid % LP;
   const size_t hw = size_t(H) * W;
+  float* ws_slot = a.ws == nullptr ? nullptr
+                   : a.ws + (size_t(blockIdx.y) * gridDim.x + blockIdx.x) * (size_t(a.ns) * C * 9 + a.ns);
 
   for (int o = 0; o < a.ns; ++o) {
     if (tid == 0) ssum_s = 0.f;
@@ -403,7 +412,12 @@ __global__ void __launch_bounds__(kEdgeWgradThreads) edge_wgrad_kernel(const Edg
     if (a.ssum != nullptr) {
 #pragma unroll
       for (int d = 16; d > 0; d >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, d);
-      if (lane == 0) atomicAdd(&ssum_s, ss);
+      if (lane == 0) {
+        if (a.ws != nullptr)
+          ssum_w[warp] = ss;
+        else
+          atomicAdd(&ssum_s, ss);
+      }
     }
     __syncthreads();
     // ---- stream V
@@ -448,9 +462,21 @@ __global__ void __launch_bounds__(kEdgeWgradThreads) edge_wgrad_kernel(const Edg
       float x = 0.f;
 #pragma unroll
       for (int w = 0; w < kEdgeWgradThreads / 32; ++w) x += red[w * (C * 9) + i];
-      atomicAdd(a.r + size_t(o) * C * 9 + i, x);
+      if (ws_slot != nullptr)
+        ws_slot[size_t(o) * C * 9 + i] = x;
+      else
+        atomicAdd(a.r + size_t(o) * C * 9 + i, x);
     }
-    if (a.ssum != nullptr && tid == 0) atomicAdd(a.ssum + o, ssum_s);
+    if (a.ssum != nullptr && tid == 0) {
+      if (ws_slot != nullptr) {
+        float x = 0.f;
+#pragma unroll
+        for (int w = 0; w < kEdgeWgradThreads / 32; ++w) x += ssum_w[w];
+        ws_slot[size_t(a.ns) * C * 9 + o] = x;
+      } else {
+        atomicAdd(a.ssum + o, ssum_s);
+      }
+    }
   }
 }
 

@@ -27,6 +27,7 @@
 #pragma once
 #include <cuda_bf16.h>
 
+#include "../../include/xmm_b200.h"
 #include "conv3x3_tc.cuh"
 
 namespace xmm {
@@ -289,6 +290,7 @@ struct ColsumArgs {
   int ctot, nseg, ngroups;
   size_t npix;
   ColsumSeg seg[kColsumMaxSeg];
+  float* ws;  // deterministic form: CTA b stores its unscaled sums to ws[b * ngroups * 8 + channel] (no atomics, outs unused)
 };
 
 __global__ void __launch_bounds__(kColsumThreads) colsum_multi_kernel(const ColsumArgs a) {
@@ -332,11 +334,49 @@ __global__ void __launch_bounds__(kColsumThreads) colsum_multi_kernel(const Cols
     const int gg = t / 8, i = t % 8;
     float x = 0.f;
     for (int l = 0; l < ppb; ++l) x += red[(l * a.ngroups + gg) * 8 + i];
+    if (a.ws != nullptr) {
+      a.ws[size_t(blockIdx.x) * (a.ngroups * 8) + t] = x;
+      continue;
+    }
     int sj = 0;
 #pragma unroll
     for (int k = 1; k < kColsumMaxSeg; ++k)
       if (k < a.nseg && gg >= a.seg[k].group0) sj = k;
     atomicAdd(a.seg[sj].out + (gg - a.seg[sj].group0) * 8 + i, a.seg[sj].scale * x);
+  }
+}
+
+// Deterministic reductions (xmm_det_finalize): job blockIdx.y, element i of it:
+//   dst[i] = (accumulate ? dst[i] : 0) + scale * sum_{k = 0, 1, .., count-1} slots[k * stride + i]
+// with k in increasing order, so the bits depend only on the slot contents.  Each slot is cleared after it is read: a
+// producer that leaves some of its slots unwritten (a smaller grid, a warp without some of the columns) adds exact
+// zeros the next time, and needs no clearing launch of its own.  One thread per element; eight independent loads in
+// flight per thread (a conv3x3 job reads ~1200 slots).
+constexpr int kDetFinalizeThreads = 128;
+__global__ void __launch_bounds__(kDetFinalizeThreads) det_finalize_kernel(const xmm_det_job* __restrict__ jobs,
+                                                                          float* __restrict__ dst_base) {
+  const xmm_det_job& j = jobs[blockIdx.y];
+  for (int i = blockIdx.x * kDetFinalizeThreads + threadIdx.x; i < j.n; i += gridDim.x * kDetFinalizeThreads) {
+    float* p = j.slots + i;
+    const size_t st = size_t(j.stride);
+    float s = 0.f;
+    int k = 0;
+    for (; k + 8 <= j.count; k += 8) {
+      float v[8];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) v[u] = p[(k + u) * st];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) {
+        s += v[u];
+        p[(k + u) * st] = 0.f;
+      }
+    }
+    for (; k < j.count; ++k) {
+      s += p[k * st];
+      p[k * st] = 0.f;
+    }
+    float* d = dst_base + j.dst + i;
+    *d = (j.accumulate ? *d : 0.f) + j.scale * s;
   }
 }
 

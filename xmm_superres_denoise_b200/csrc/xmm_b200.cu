@@ -22,7 +22,7 @@
 using namespace xmm;
 
 extern "C" const char* xmm_last_error(void) { return last_error_ref().c_str(); }
-extern "C" int xmm_version(void) { return 100; }
+extern "C" int xmm_version(void) { return 101; }
 extern "C" int xmm_check_device(void) {
   DeviceInfo d;
   return require_sm100(&d);
@@ -111,6 +111,7 @@ void fill_epilogue(ConvEpilogue& e, const xmm_conv3x3_params& p) {
   e.shuffle_stride = p.shuffle_stride > 0 ? p.shuffle_stride : p.cout;
   e.img_out = nullptr; e.img_res = nullptr; e.img_pre = nullptr; e.img_cout = 0; e.img_clamp = 0;
   e.colsum = p.colsum; e.colsum_scale = p.colsum_scale;
+  e.colsum_ws = p.colsum ? p.colsum_ws : nullptr;
 }
 
 struct ImageOut {
@@ -477,7 +478,7 @@ int launch_conv_mode(const xmm_conv3x3_params& p, const DeviceInfo& dev, cudaStr
 }  // namespace
 
 namespace {
-int check_conv_params(const xmm_conv3x3_params& p) {
+int check_conv_params(const xmm_conv3x3_params& p, const DeviceInfo& dev) {
   XMM_REQUIRE(p.in && p.out && p.wblob, "conv3x3: null tensor pointer");
   XMM_REQUIRE(p.batch > 0 && p.height > 0 && p.width > 0, "conv3x3: bad shape %dx%dx%d", p.batch, p.height, p.width);
   XMM_REQUIRE(p.kc == 32 || p.kc == 64, "conv3x3: kc must be 32 or 64 (got %d)", p.kc);
@@ -497,6 +498,11 @@ int check_conv_params(const xmm_conv3x3_params& p) {
   XMM_REQUIRE(!p.r1 || (p.r1_ctot % 8 == 0 && p.r1_coff % 8 == 0), "conv3x3: r1 window alignment");
   XMM_REQUIRE(!p.r2 || (p.r2_ctot % 8 == 0 && p.r2_coff % 8 == 0), "conv3x3: r2 window alignment");
   XMM_REQUIRE(!p.colsum || (p.cout == 32 && p.pixel_shuffle == 0), "conv3x3: fused column sums need cout = 32");
+  // every form that takes column sums launches at most dev.sm_count CTAs (the pipelined chain: all of its layers)
+  XMM_REQUIRE(!p.colsum_ws || (p.colsum && p.colsum_ws_slots >= size_t(dev.sm_count) * kCsumWarpSlots &&
+                               (reinterpret_cast<uintptr_t>(p.colsum_ws) & 3) == 0),
+              "conv3x3: colsum_ws needs colsum and %zu slots (got %zu)", size_t(dev.sm_count) * kCsumWarpSlots,
+              p.colsum_ws_slots);
   XMM_REQUIRE(p.pixel_shuffle != 1 || (!p.mask && !p.r1 && !p.r2 && p.cout % 128 == 0),
               "conv3x3: pixel_shuffle needs cout %% 128 == 0 and no mask/residual");
   XMM_REQUIRE((reinterpret_cast<uintptr_t>(p.in) & 15) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0 &&
@@ -512,7 +518,7 @@ extern "C" int xmm_conv3x3_bf16(const xmm_conv3x3_params* pp, void* stream) {
   DeviceInfo dev;
   int rc = require_sm100(&dev);
   if (rc != XMM_OK) return rc;
-  rc = check_conv_params(p);
+  rc = check_conv_params(p, dev);
   if (rc != XMM_OK) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   // Row-hop form (conv3x3_row.cuh): the default for the NARROW layers it qualifies for (tap_mode 0 with a row-hop
@@ -927,7 +933,7 @@ extern "C" int xmm_conv3x3_chain_bf16(const xmm_conv3x3_params* layers, int nlay
   int rc = require_sm100(&dev);
   if (rc != XMM_OK) return rc;
   for (int l = 0; l < nlayers; ++l) {
-    rc = check_conv_params(layers[l]);
+    rc = check_conv_params(layers[l], dev);
     if (rc != XMM_OK) return rc;
   }
   cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -1267,8 +1273,17 @@ extern "C" int xmm_conv3x3_wgrad(const xmm_wgrad_params* pp, void* stream) {
   return XMM_OK;
 }
 
-extern "C" int xmm_colsum_multi_bf16(const void* in, int ctot, size_t npix, const xmm_colsum_segment* segs, int nseg,
-                                     void* stream) {
+namespace {
+// Grid of one colsum launch: >= 8 pixels per thread, at most 8 CTAs per SM.
+unsigned colsum_grid(size_t npix, int groups, const DeviceInfo& dev) {
+  const int ppb = kColsumThreads / groups;
+  const size_t want = (npix + size_t(ppb) * 8 - 1) / (size_t(ppb) * 8);
+  const size_t cap = size_t(dev.sm_count) * 8;
+  return unsigned(want < 1 ? 1 : (want > cap ? cap : want));
+}
+
+int colsum_launch(const void* in, int ctot, size_t npix, const xmm_colsum_segment* segs, int nseg, float* ws,
+                  size_t ws_slots, void* stream) {
   DeviceInfo dev;
   int rc = require_sm100(&dev);
   if (rc != XMM_OK) return rc;
@@ -1279,27 +1294,48 @@ extern "C" int xmm_colsum_multi_bf16(const void* in, int ctot, size_t npix, cons
   a.ctot = ctot;
   a.npix = npix;
   a.nseg = nseg;
+  a.ws = ws;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   int groups = 0;
   for (int i = 0; i < nseg; ++i) {
     const xmm_colsum_segment& g = segs[i];
-    XMM_REQUIRE(g.out != nullptr && g.n > 0 && g.n % 8 == 0 && g.c0 % 8 == 0 && g.c0 >= 0 && g.c0 + g.n <= ctot,
+    XMM_REQUIRE((ws != nullptr || g.out != nullptr) && g.n > 0 && g.n % 8 == 0 && g.c0 % 8 == 0 && g.c0 >= 0 &&
+                    g.c0 + g.n <= ctot,
                 "colsum: channel window [%d,%d) of %d", g.c0, g.c0 + g.n, ctot);
     a.seg[i].c0 = g.c0; a.seg[i].n = g.n; a.seg[i].out = g.out; a.seg[i].scale = g.scale;
     a.seg[i].group0 = groups;
     groups += g.n / 8;
-    if (!g.accumulate) XMM_CUDA_OK(cudaMemsetAsync(g.out, 0, size_t(g.n) * sizeof(float), s));
+    if (ws == nullptr && !g.accumulate) XMM_CUDA_OK(cudaMemsetAsync(g.out, 0, size_t(g.n) * sizeof(float), s));
   }
   XMM_REQUIRE(groups <= kColsumThreads, "colsum: %d channels in one call (max %d)", groups * 8, kColsumThreads * 8);
   a.ngroups = groups;
   if (npix == 0) return XMM_OK;
-  const int ppb = kColsumThreads / groups;
-  size_t want = (npix + size_t(ppb) * 8 - 1) / (size_t(ppb) * 8);  // >= 8 pixels per thread
-  const size_t cap = size_t(dev.sm_count) * 8;
-  const unsigned grid = unsigned(want < 1 ? 1 : (want > cap ? cap : want));
+  const unsigned grid = colsum_grid(npix, groups, dev);
+  XMM_REQUIRE(ws == nullptr || (ws_slots >= grid && (reinterpret_cast<uintptr_t>(ws) & 3) == 0),
+              "colsum: %u workspace slots needed (got %zu)", grid, ws_slots);
   colsum_multi_kernel<<<grid, kColsumThreads, 0, s>>>(a);
   XMM_CUDA_OK(cudaGetLastError());
   return XMM_OK;
+}
+
+// Rows of one image per edge_wgrad CTA: as many as fit 40 KB of staged s rows (+ halo), at most 8 (0: too wide).
+int edge_rows(int height, int width) {
+  int rows = int((40 * 1024) / (size_t(width + 2) * sizeof(float))) - 2;
+  if (rows > 8) rows = 8;
+  if (rows > height) rows = height;
+  return rows;
+}
+}  // namespace
+
+extern "C" int xmm_colsum_multi_bf16(const void* in, int ctot, size_t npix, const xmm_colsum_segment* segs, int nseg,
+                                     void* stream) {
+  return colsum_launch(in, ctot, npix, segs, nseg, nullptr, 0, stream);
+}
+
+extern "C" int xmm_colsum_multi_det_bf16(const void* in, int ctot, size_t npix, const xmm_colsum_segment* segs,
+                                         int nseg, float* ws, size_t ws_slots, void* stream) {
+  XMM_REQUIRE(ws != nullptr, "colsum (deterministic): null workspace");
+  return colsum_launch(in, ctot, npix, segs, nseg, ws, ws_slots, stream);
 }
 
 extern "C" int xmm_colsum_bf16(const void* in, int ctot, int c0, int n, size_t npix, float* out, float scale,
@@ -1308,31 +1344,58 @@ extern "C" int xmm_colsum_bf16(const void* in, int ctot, int c0, int n, size_t n
   return xmm_colsum_multi_bf16(in, ctot, npix, &g, 1, stream);
 }
 
+extern "C" size_t xmm_det_slots(int site, int batch, int height, int width, int channels) {
+  DeviceInfo dev;
+  if (require_sm100(&dev) != XMM_OK || batch < 1 || height < 1 || width < 1 || channels < 8) return 0;
+  switch (site) {
+    case XMM_DET_CONV3X3: return size_t(dev.sm_count) * kCsumWarpSlots;
+    case XMM_DET_COLSUM:
+      return channels / 8 > kColsumThreads ? 0 : colsum_grid(size_t(batch) * height * width, channels / 8, dev);
+    case XMM_DET_EDGE_WGRAD: {
+      const int rows = edge_rows(height, width);
+      return rows < 1 ? 0 : size_t((height + rows - 1) / rows) * size_t(batch);
+    }
+    default: return 0;
+  }
+}
+
+extern "C" int xmm_det_finalize(const xmm_det_job* jobs_dev, int njobs, int max_n, float* dst_base, void* stream) {
+  DeviceInfo dev;
+  int rc = require_sm100(&dev);
+  if (rc != XMM_OK) return rc;
+  XMM_REQUIRE(jobs_dev != nullptr && dst_base != nullptr && njobs >= 1 && njobs <= 65535 && max_n >= 1,
+              "det_finalize: %d jobs (1..65535), max_n %d", njobs, max_n);
+  const dim3 grid(unsigned((max_n + kDetFinalizeThreads - 1) / kDetFinalizeThreads), unsigned(njobs));
+  det_finalize_kernel<<<grid, kDetFinalizeThreads, 0, static_cast<cudaStream_t>(stream)>>>(jobs_dev, dst_base);
+  XMM_CUDA_OK(cudaGetLastError());
+  return XMM_OK;
+}
+
 extern "C" int xmm_edge_wgrad(const xmm_edge_wgrad_params* pp, void* stream) {
   XMM_REQUIRE(pp != nullptr, "edge_wgrad: null params");
   const xmm_edge_wgrad_params& p = *pp;
   DeviceInfo dev;
   int rc = require_sm100(&dev);
   if (rc != XMM_OK) return rc;
-  XMM_REQUIRE(p.s && p.v && p.r, "edge_wgrad: null tensor pointer");
+  XMM_REQUIRE(p.s && p.v && (p.r || p.ws), "edge_wgrad: null tensor pointer");
   XMM_REQUIRE(p.ns >= 1 && p.ns <= 4 && p.batch > 0 && p.height > 0 && p.width > 0, "edge_wgrad: bad shape");
   EdgeWgradArgs a{};
   a.s = p.s; a.gate = p.gate;
   a.v = static_cast<const __nv_bfloat16*>(p.v); a.v_ctot = p.v_ctot; a.v_coff = p.v_coff;
   a.v2 = static_cast<const __nv_bfloat16*>(p.v2); a.v2_ctot = p.v2_ctot; a.v2_coff = p.v2_coff;
   a.r = p.r; a.ssum = p.ssum; a.batch = p.batch; a.ns = p.ns; a.height = p.height; a.width = p.width;
+  a.ws = p.ws;
   XMM_REQUIRE(p.v_ctot % 8 == 0 && p.v_coff % 8 == 0 && (!p.v2 || (p.v2_ctot % 8 == 0 && p.v2_coff % 8 == 0)),
               "edge_wgrad: channel windows must be 8-channel aligned");
   XMM_REQUIRE(p.channels == 32 || p.channels == 64, "edge_wgrad: channels=%d (supported: 32, 64)", p.channels);
-  // rows per CTA: as many as fit 40 KB of staged s rows (+ halo), at most 8
   const size_t red_bytes = size_t(kEdgeWgradThreads / 32) * p.channels * 9 * sizeof(float);
-  int rows = int((40 * 1024) / (size_t(p.width + 2) * sizeof(float))) - 2;
-  if (rows > 8) rows = 8;
-  if (rows > p.height) rows = p.height;
+  const int rows = edge_rows(p.height, p.width);
   XMM_REQUIRE(rows >= 1, "edge_wgrad: image width %d too large for the shared-memory row staging", p.width);
   a.rows = rows;
   const size_t smem = size_t(rows + 2) * (p.width + 2) * sizeof(float) + red_bytes;
   const dim3 grid(unsigned((p.height + rows - 1) / rows), unsigned(p.batch));
+  XMM_REQUIRE(!p.ws || (p.ws_slots >= size_t(grid.x) * grid.y && (reinterpret_cast<uintptr_t>(p.ws) & 3) == 0),
+              "edge_wgrad: %zu workspace slots needed (got %zu)", size_t(grid.x) * grid.y, p.ws_slots);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (p.channels == 32) {
     static bool attr32 = false;

@@ -209,6 +209,8 @@ class _LayerPlans:
                 if key in k2 and k2.get(key[:-5]) is not None:
                     k2[key] = k2[key] + n0
             if k2.get("colsum") is not None:  # fused bias gradient: this part's window of the bias gradient
+                if k2.get("colsum_ws") is not None and len(plan) > 1:
+                    raise RuntimeError(f"{name}: the deterministic fused bias gradient needs an unsplit layer")
                 k2["colsum"] = k2["colsum"][n0:n0 + nt]
             if k2.get("pixel_shuffle", 0) == 2 and len(plan) > 1:
                 k2["shuffle_stride"] = rows  # the four (y&1, x&1) blocks are a full layer apart

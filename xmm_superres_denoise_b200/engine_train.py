@@ -22,7 +22,7 @@ from typing import Dict, List, Optional
 
 import torch
 
-from . import ops
+from . import determinism, ops
 from .engine import RRDBEngine, _Blob, _Segment
 
 
@@ -66,6 +66,7 @@ class TrainEngine(RRDBEngine):
         self.generation = 0
         self._params = list(gen.parameters())
         self._pindex = {id(p): n for n, p in enumerate(self._params)}
+        self._det: Optional[determinism.DetPlan] = None  # the running backward's plan in deterministic mode
 
     # ------------------------------------------------------------------ buffers
     def _train_buffers(self, b: int, h: int, w: int, device: torch.device) -> Dict[str, object]:
@@ -121,16 +122,41 @@ class TrainEngine(RRDBEngine):
         return out, bufs
 
     # ------------------------------------------------------------------ backward
-    def _grad_views(self, device: torch.device) -> List[torch.Tensor]:
-        """Fresh flat fp32 gradient buffer (autograd may adopt the returned tensors as .grad)."""
+    def _grad_views(self, device: torch.device, extra: int = 0) -> List[torch.Tensor]:
+        """Fresh flat fp32 gradient buffer (autograd may adopt the returned tensors as .grad).  extra: zeroed scratch
+        floats after the gradients (deterministic mode: destinations that are copied into a gradient afterwards)."""
         total = sum(p.numel() for p in self._params)
-        flat = torch.zeros(total, dtype=torch.float32, device=device)
+        flat = torch.zeros(total + extra, dtype=torch.float32, device=device)
         views, off = [], 0
         for p in self._params:
             views.append(flat[off:off + p.numel()].view(p.shape))
             off += p.numel()
-        self.last_flat_grad = flat
+        self.last_flat_grad = flat[:total] if extra else flat
+        self._flat_ext, self._ext_off = flat, total
         return views
+
+    def _scratch(self, n: int) -> torch.Tensor:
+        t = self._flat_ext[self._ext_off:self._ext_off + n]
+        self._ext_off += n
+        return t
+
+    def _det_scratch_floats(self) -> int:
+        return self.gen.in_channels * self.nf * 9 + (4 * self.nf * self.num_upsample if self.kind == "sr" else 0)
+
+    def _colsum(self, inp: torch.Tensor, segments) -> None:
+        """Bias gradients from one buffer: segments [(c0, n, dst, scale, accumulate)]."""
+        if self._det is not None:
+            self._det.colsum([inp], segments)
+        elif len(segments) == 1:
+            ops.colsum(inp, *segments[0])
+        else:
+            ops.colsum_multi(inp, segments)
+
+    def _edge_wgrad(self, *a, **kw) -> None:
+        if self._det is not None:
+            self._det.edge_wgrad(*a, **kw)
+        else:
+            ops.edge_wgrad(*a, **kw)
 
     def _gv(self, grads, p: torch.Tensor) -> torch.Tensor:
         return grads[self._pindex[id(p)]]
@@ -151,11 +177,16 @@ class TrainEngine(RRDBEngine):
         if conv.bias is not None:
             db = self._gv(grads, conv.bias)
             if perm:
-                tmp = torch.empty(n, dtype=torch.float32, device=dy.device)
-                ops.colsum(dy, 0, n, tmp)
-                db.copy_(tmp.view(4, n // 4).t().reshape(n))  # packed g*F+c -> channel 4c+g
+                if self._det is None:
+                    tmp = torch.empty(n, dtype=torch.float32, device=dy.device)
+                    ops.colsum(dy, 0, n, tmp)
+                    db.copy_(tmp.view(4, n // 4).t().reshape(n))  # packed g*F+c -> channel 4c+g
+                else:
+                    tmp = self._scratch(n)
+                    self._det.colsum([dy], [(0, n, tmp, 1.0, False)])
+                    self._det.after(lambda: db.copy_(tmp.view(4, n // 4).t().reshape(n)))
             else:
-                ops.colsum(dy, 0, n, db, accumulate=True)  # db is a view of the zero-initialised flat buffer
+                self._colsum(dy, [(0, n, db, 1.0, True)])  # db is a view of the zero-initialised flat buffer
 
     def _rdb_backward(self, i: int, r: int, bufs, grads, d_fea: torch.Tensor) -> None:
         f, kc, a = self.nf, self.kc, self.arena
@@ -193,6 +224,8 @@ class TrainEngine(RRDBEngine):
         zero-initialised flat gradient buffer)."""
         if conv.bias is None or not self.fuse_bias:
             return {}
+        if self._det is not None:
+            return self._det.conv_kwargs(*self._det_bhw, self._gv(grads, conv.bias), scale)
         return dict(colsum=self._gv(grads, conv.bias), colsum_scale=scale)
 
     def _rdb_wgrad(self, i: int, r: int, bufs, grads) -> None:
@@ -207,7 +240,7 @@ class TrainEngine(RRDBEngine):
             segs = [((k - 1) * f, f, self._gv(grads, c.bias), s5 if k == 5 else 1.0, True)
                     for k, c in enumerate(convs, 1) if c.bias is not None]
             if segs:
-                ops.colsum_multi(G, segs)
+                self._colsum(G, segs)
         if f == 64:
             self._rdb_wgrad_64(A, G, dws, s5)
             return
@@ -258,10 +291,31 @@ class TrainEngine(RRDBEngine):
         if generation != self.generation:
             raise RuntimeError("backward through a GeneratorRRDB forward whose saved activations were overwritten by a "
                                "later forward (run backward before the next training-mode forward)")
+        if not determinism.enabled():
+            self._det = None
+            return self._backward(bufs, x, gout, need_x_grad, rrdb_done_hook)
+        # deterministic mode: the plan (slot ranges, finalize job tables) lives with this shape's training buffers
+        plan = bufs.get("det")
+        if plan is None:
+            plan = bufs["det"] = determinism.DetPlan(x.device)
+        self._det = plan
+        try:
+            return self._backward(bufs, x, gout, need_x_grad, rrdb_done_hook)
+        except BaseException:
+            bufs.pop("det", None)  # slots written without their finalize: start the next deterministic call afresh
+            raise
+        finally:
+            self._det = None
+
+    def _backward(self, bufs, x: torch.Tensor, gout: torch.Tensor, need_x_grad: bool, rrdb_done_hook):
         g, f, kc, a = self.gen, self.nf, self.kc, self.arena
+        det = self._det
         gout = gout.contiguous().float()
         x = x.contiguous().float()
-        grads = self._grad_views(x.device)
+        grads = self._grad_views(x.device, self._det_scratch_floats() if det is not None else 0)
+        if det is not None:
+            det.begin(self._flat_ext)
+            self._det_bhw = tuple(bufs["trunk"].shape[:3])
         pre = bufs["pre"]
         # flipped / transposed conv_last filter: data gradient of an F->1 conv is a 1->F stencil (288 floats)
         wt_last = g.conv_last.weight.detach().flip(2, 3).permute(1, 0, 2, 3).contiguous()
@@ -270,11 +324,11 @@ class TrainEngine(RRDBEngine):
         if self.kind == "dn":
             feat_in = bufs["trunk"]
             ops.conv_first(gout, wt_last, None, bufs["d_trunk"], 0, gate=pre)
-            ops.edge_wgrad(gout, feat_in, 0, f, dw_last.view(g.out_channels, f, 9), ssum=db_last, gate=pre)
+            self._edge_wgrad(gout, feat_in, 0, f, dw_last.view(g.out_channels, f, 9), ssum=db_last, gate=pre)
         else:
             hr = bufs["hr"]
             ops.conv_first(gout, wt_last, None, bufs["d_hr"], 0, gate=pre, mask=hr, mask_coff=0, mask_slope=0.2)
-            ops.edge_wgrad(gout, hr, 0, f, dw_last.view(g.out_channels, f, 9), ssum=db_last, gate=pre)
+            self._edge_wgrad(gout, hr, 0, f, dw_last.view(g.out_channels, f, 9), ssum=db_last, gate=pre)
             ups = [bufs["trunk"]] + [bufs[f"up{s}"] for s in range(self.num_upsample)]
             self._single_conv_wgrad(g.HRconv, ups[-1], bufs["d_hr"], grads)
             dy = bufs["d_hr"]
@@ -299,19 +353,30 @@ class TrainEngine(RRDBEngine):
                 for r in (2, 1, 0):
                     self._rdb_backward(i, r, bufs, grads, d_fea)
                     self._rdb_wgrad(i, r, bufs, grads)
+                if det is not None:  # this RRDB's (and, first time round, the tail layers') reductions, in order
+                    det.flush()
                 if rrdb_done_hook is not None:  # every gradient of RRDB i (and of all later layers) is enqueued
                     rrdb_done_hook(i, self.last_flat_grad)
         else:
             self._run(self._conv("d.trunk", d_trunk, 0, f, d_fea, 0))
         # conv_first: dL/d(fea) = d_fea (through the RRDBs) + d_trunk (skip)
         cin = g.in_channels
-        r_first = torch.zeros(cin, f, 9, dtype=torch.float32, device=x.device)
-        ops.edge_wgrad(x, d_fea, 0, f, r_first, v2=d_trunk, v2_coff=0)
-        self._gv(grads, g.conv_first.weight).copy_(r_first.flip(2).permute(1, 0, 2).reshape(f, cin, 3, 3))
-        if g.conv_first.bias is not None:
-            dbf = self._gv(grads, g.conv_first.bias)
-            ops.colsum(d_fea, 0, f, dbf)
-            ops.colsum(d_trunk, 0, f, dbf, accumulate=True)
+        dwf = self._gv(grads, g.conv_first.weight)
+        if det is None:
+            r_first = torch.zeros(cin, f, 9, dtype=torch.float32, device=x.device)
+            ops.edge_wgrad(x, d_fea, 0, f, r_first, v2=d_trunk, v2_coff=0)
+            dwf.copy_(r_first.flip(2).permute(1, 0, 2).reshape(f, cin, 3, 3))
+            if g.conv_first.bias is not None:
+                dbf = self._gv(grads, g.conv_first.bias)
+                ops.colsum(d_fea, 0, f, dbf)
+                ops.colsum(d_trunk, 0, f, dbf, accumulate=True)
+        else:
+            r_first = self._scratch(cin * f * 9).view(cin, f, 9)
+            det.edge_wgrad(x, d_fea, 0, f, r_first, v2=d_trunk, v2_coff=0)
+            det.after(lambda: dwf.copy_(r_first.flip(2).permute(1, 0, 2).reshape(f, cin, 3, 3)))
+            if g.conv_first.bias is not None:  # both integrands in one job: d_fea's slots, then d_trunk's
+                det.colsum([d_fea, d_trunk], [(0, f, self._gv(grads, g.conv_first.bias), 1.0, False)])
+            det.flush()
         gx = None
         if need_x_grad:
             # dL/dx = conv_first^T(dL/dfea) (+ the DN residual path); an F->cin stencil = conv_last kernel

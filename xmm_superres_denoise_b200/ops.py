@@ -41,7 +41,8 @@ def _conv3x3_params(p: Conv3x3Params, inp: torch.Tensor, in_coff: int, cin: int,
                     r2: Optional[torch.Tensor] = None, r2_coff: int = 0, s2: float = 0.0,
                     mask: Optional[torch.Tensor] = None, mask_coff: int = 0, mask_slope: float = 1.0,
                     pixel_shuffle: int = 0, tap_mode: int = 0, colsum: Optional[torch.Tensor] = None,
-                    colsum_scale: float = 1.0, shuffle_stride: int = 0, wblob_row: Optional[int] = None) -> None:
+                    colsum_scale: float = 1.0, shuffle_stride: int = 0, wblob_row: Optional[int] = None,
+                    colsum_ws: Optional[torch.Tensor] = None) -> None:
     _nhwc(inp, "conv3x3 input")
     _nhwc(out, "conv3x3 output")
     b, h, w, ctot = inp.shape
@@ -76,6 +77,9 @@ def _conv3x3_params(p: Conv3x3Params, inp: torch.Tensor, in_coff: int, cin: int,
         if colsum.numel() != cout:
             raise RuntimeError("conv3x3 colsum: one float per output channel")
         p.colsum, p.colsum_scale = colsum.data_ptr(), colsum_scale
+        if colsum_ws is not None:
+            _lib.require_cuda_tensor(colsum_ws, torch.float32, "conv3x3 colsum_ws")
+            p.colsum_ws, p.colsum_ws_slots = colsum_ws.data_ptr(), colsum_ws.numel() // 32
 
 
 def conv3x3(inp: torch.Tensor, in_coff: int, cin: int, wblob_ptr: int, kc: int, cout: int,
@@ -83,7 +87,8 @@ def conv3x3(inp: torch.Tensor, in_coff: int, cin: int, wblob_ptr: int, kc: int, 
     """out[..., out_coff:out_coff+cout] = epilogue(conv3x3(inp[..., in_coff:in_coff+cin])).
 
     Keywords: lrelu, s0, r1/r1_coff/s1, r2/r2_coff/s2, mask/mask_coff/mask_slope, pixel_shuffle, tap_mode,
-    colsum/colsum_scale (fused bias gradient: colsum += scale * column sums of the written values),
+    colsum/colsum_scale (fused bias gradient: colsum += scale * column sums of the written values), colsum_ws (its
+    deterministic form: unscaled per-warp sums to slots of 32 floats, for det_finalize; colsum is then not written),
     wblob_row (the layer's row-hop weight image: lets the library pick conv3x3_row.cuh where the shape qualifies).
     See ``xmm_conv3x3_params`` in include/xmm_b200.h for the epilogue definition."""
     if _TORCH_OPS and not (kw.keys() - _TORCH_FWD_KEYS):
@@ -379,8 +384,9 @@ def colsum_multi(inp: torch.Tensor, segments) -> None:
 
 def edge_wgrad(s: torch.Tensor, v: torch.Tensor, v_coff: int, channels: int, r: torch.Tensor,
                ssum: Optional[torch.Tensor] = None, gate: Optional[torch.Tensor] = None,
-               v2: Optional[torch.Tensor] = None, v2_coff: int = 0) -> None:
-    """r[o][c][tap] += sum_p s[o][p] * (v + v2)[p + off(tap)][c];  ssum[o] += sum_p s[o][p]."""
+               v2: Optional[torch.Tensor] = None, v2_coff: int = 0, ws: Optional[torch.Tensor] = None) -> None:
+    """r[o][c][tap] += sum_p s[o][p] * (v + v2)[p + off(tap)][c];  ssum[o] += sum_p s[o][p].
+    ws: deterministic form -- per-CTA sums to slots of ns * channels * 9 + ns floats (r / ssum are not written)."""
     _lib.require_cuda_tensor(s, torch.float32, "edge_wgrad s")
     _nhwc(v, "edge_wgrad v")
     _lib.require_cuda_tensor(r, torch.float32, "edge_wgrad r")
@@ -392,5 +398,40 @@ def edge_wgrad(s: torch.Tensor, v: torch.Tensor, v_coff: int, channels: int, r: 
         p.v2, p.v2_ctot, p.v2_coff = v2.data_ptr(), v2.shape[3], v2_coff
     p.r, p.ssum = r.data_ptr(), _ptr(ssum)
     p.batch, p.ns, p.height, p.width, p.channels = s.shape[0], s.shape[1], s.shape[2], s.shape[3], channels
+    if ws is not None:
+        _lib.require_cuda_tensor(ws, torch.float32, "edge_wgrad ws")
+        p.ws, p.ws_slots = ws.data_ptr(), ws.numel() // (s.shape[1] * channels * 9 + s.shape[1])
     _lib.check(_lib.load().xmm_edge_wgrad(ctypes.byref(p), _lib.stream_ptr()))
+    _count()
+
+
+def colsum_multi_det(inp: torch.Tensor, segments, ws: torch.Tensor) -> None:
+    """Deterministic form of :func:`colsum_multi`: segments [(c0, n, scale)]; each CTA stores the unscaled sums of the
+    segments' channels (concatenated) to its own slot of ``ws`` (sum(n) floats per slot, zero on entry)."""
+    _nhwc(inp, "colsum input")
+    _lib.require_cuda_tensor(ws, torch.float32, "colsum ws")
+    arr = (_lib.ColsumSegment * len(segments))()
+    for a, (c0, n, scale) in zip(arr, segments):
+        a.c0, a.n, a.scale = c0, n, scale
+    npix = inp.shape[0] * inp.shape[1] * inp.shape[2]
+    row = sum(n for _, n, _ in segments)
+    _lib.check(_lib.load().xmm_colsum_multi_det_bf16(inp.data_ptr(), inp.shape[3], npix, arr, len(segments),
+                                                     ws.data_ptr(), ws.numel() // row, _lib.stream_ptr()))
+    _count()
+
+
+def det_slots(site: int, batch: int, height: int, width: int, channels: int) -> int:
+    """Slots one call of a deterministic reduction site writes at most (_lib.DET_*; xmm_det_slots)."""
+    n = int(_lib.load().xmm_det_slots(site, batch, height, width, channels))
+    if n == 0:
+        raise RuntimeError(f"xmm_det_slots: no slot layout for site {site} at {batch}x{height}x{width}x{channels} "
+                           f"({_lib.load().xmm_last_error().decode()})")
+    return n
+
+
+def det_finalize(jobs_dev: torch.Tensor, njobs: int, max_n: int, dst_base: torch.Tensor) -> None:
+    """One launch for a device table of :class:`_lib.DetJob`: dst_base[dst + i] (+)= scale * sum of the slots, in
+    slot order; the slots read are left zero."""
+    _lib.require_cuda_tensor(dst_base, torch.float32, "det_finalize dst_base")
+    _lib.check(_lib.load().xmm_det_finalize(jobs_dev.data_ptr(), njobs, max_n, dst_base.data_ptr(), _lib.stream_ptr()))
     _count()

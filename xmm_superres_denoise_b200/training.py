@@ -21,7 +21,7 @@ from typing import List, Optional, Tuple
 import torch
 from torch import nn
 
-from . import _lib, ops
+from . import _lib, determinism, ops
 
 
 def flatten_parameters(module: nn.Module) -> torch.Tensor:
@@ -202,7 +202,8 @@ class TrainStep:
         return st, flat_grad
 
     def __call__(self, lr_img: torch.Tensor, hr_img: torch.Tensor) -> torch.Tensor:
-        key = (tuple(lr_img.shape), tuple(hr_img.shape), lr_img.dtype, hr_img.dtype)
+        # (the deterministic mode changes the backward's launches: a graph is captured per mode)
+        key = (tuple(lr_img.shape), tuple(hr_img.shape), lr_img.dtype, hr_img.dtype, determinism.enabled())
         if self.use_graph and self._graph is not None and self._graph[0] == key:
             _, graph, s_lr, s_hr, st, flat_grad = self._graph
             s_lr.copy_(lr_img)
