@@ -147,6 +147,13 @@ int xmm_conv3x3_bf16(const xmm_conv3x3_params* p, void* stream);
  * XMM_CHAIN_SKIP_DEAD_STORES: the caller will not read the outputs of layers 1..n-1 after this call (inference);
  *         outputs that no later launch of the chain reads need not be written (the fused form never writes x4).   */
 #define XMM_CHAIN_SKIP_DEAD_STORES 0x100
+/* XMM_CHAIN_SKIP_LAST: compute and store the outputs of layers 1..n-1 only; the last layer's output is never written
+ *         (recomputing a dense block's x1..x4 from its input for a backward pass).  The launch form is chosen as
+ *         without the flag; the fused form then runs conv1..conv3 as usual and conv4 in a conv4-only form of the
+ *         second kernel, every other form runs layers 1..n-1 one by one.  The fused and layer-by-layer forms store
+ *         the bits the same call without the flag stores (mode 1: the same values up to fp32 summation order).
+ *         Not with XMM_CHAIN_SKIP_DEAD_STORES (XMM_ERR_INVALID_ARGUMENT); nlayers >= 2.                            */
+#define XMM_CHAIN_SKIP_LAST 0x800
 /* XMM_CHAIN_RDB_PAIR / XMM_CHAIN_RDB_SINGLE (mode 0 / 3, at most one): run both kernels of the fused dense block
  *         (conv1..conv3, conv4..conv5) as CTA pairs (two SMs share every MMA, each holding half of the weights) / as
  *         single CTAs, for this call, whatever XMM_RDB_PAIR selects.  Both forms compute the same bits.            */
@@ -292,6 +299,12 @@ int xmm_conv3x3_wgrad(const xmm_wgrad_params* p, void* stream);
 /* out[i] (+)= scale * sum over pixels of in[p][c0 + i]  (bias gradients), n multiple of 8.  */
 int xmm_colsum_bf16(const void* in, int ctot, int c0, int n, size_t npix, float* out, float scale,
                     int accumulate, void* stream);
+
+/* dst[p][dst_coff + i] = src[p][src_coff + i] for every pixel p < npix and i < channels: a channel window between two
+ * bf16 NHWC buffers of different channel pitch (a dense block's input into and out of its 5F-channel buffer).
+ * 16-byte accesses: channels, both pitches and both offsets multiples of 8, pointers 16-byte aligned.            */
+int xmm_copy_channels_bf16(const void* src, int src_ctot, int src_coff, void* dst, int dst_ctot, int dst_coff,
+                           int channels, size_t npix, void* stream);
 
 /* Several channel windows of one buffer in a single pass (a dense block's five bias gradients).           */
 typedef struct {

@@ -4,7 +4,10 @@ and out-of-protocol barrier use before any GPU time is spent.  Pair mode (simula
 conv4 + conv5 -- two producers feeding the leader's landed barriers, count-8 drained / map-row barriers, multicast
 commits, 14 stages, landed rings of 16 -- where every arrival also checks that it lands in the phase it is meant
 for (a parity wait cannot tell a phase from the one two ahead).  The pair form of conv1..conv3 (simulate_pair, nl = 3)
-reads x0 from a ring that each row enters once, and every wait checks its phase as well.  python tools/rdb_protocol_sim.py"""
+reads x0 from a ring that each row enters once, and every wait checks its phase as well.  first_only (simulate and
+simulate_pair, nl = 2): the conv4-only form (conv3x3_rdb_kernel<4, 2, PAIR, true>) -- the walk-order producer loads
+conv4's chunks only, conv5's issuer and epilogue group do nothing and conv4's epilogue writes no map rows; its waits
+check their phase too.  python tools/rdb_protocol_sim.py"""
 import os
 import sys
 from collections import deque
@@ -53,8 +56,13 @@ def layer_steps(pieces, nl, l):
             seq[m] += (pc["rb"] - pc["ra"]) + 2 * (nl - 1 - m)
 
 
-def simulate(nl, g, pieces, stages, verbose=False):
+def simulate(nl, g, pieces, stages, verbose=False, first_only=False):
+    assert not first_only or nl == 2
     ring = RINGS[nl]
+    nact = 1 if first_only else nl   # layers whose issuer / epilogue group run
+
+    def poll(bar, use):  # first_only: every wait also checks that it cannot pass a phase early
+        return bar.wait(use) if first_only else bar.ready(use & 1)
     lfull = [[Bar(1, f"lfull{l}.{s}") for s in range(8)] for l in range(nl)]
     lstage = [[None] * 8 for _ in range(nl)]
     empty = [Bar(1, f"empty{s}") for s in range(stages)]
@@ -74,12 +82,14 @@ def simulate(nl, g, pieces, stages, verbose=False):
     def producer():
         stage, phase = 0, 0
         fills = [0] * nl
+        fill = 0
         for (rnd, l, p, r, flush, n, seq) in steps:
-            if flush:
+            if flush or l >= nact:
                 continue
             for _ in range(g):
-                while not empty[stage].ready(phase ^ 1):
+                while not poll(empty[stage], fill // stages - 1):
                     yield ("empty", stage)
+                fill += 1
                 k = fills[l] % 8
                 fills[l] += 1
                 lstage[l][k] = stage
@@ -95,12 +105,12 @@ def simulate(nl, g, pieces, stages, verbose=False):
         for (p, r, flush, n, seq) in layer_steps(pieces, nl, l):
             pc = pieces[p]
             if n > 0:
-                while not tdrain[l].ready((n - 1) & 1):
+                while not poll(tdrain[l], n - 1):
                     yield ("tdrain", l, n)
             if not flush:
                 for _ in range(g):
                     k = fills % 8
-                    while not lfull[l][k].ready((fills // 8) & 1):
+                    while not poll(lfull[l][k], fills // 8):
                         yield ("lfull", l, fills)
                     st = lstage[l][k]
                     fills += 1
@@ -124,11 +134,11 @@ def simulate(nl, g, pieces, stages, verbose=False):
             pc = pieces[p]
             j = r - 1
             real = pc["ra"] - e <= j < pc["rb"] + e
-            while not tfull[l].ready(n & 1):
+            while not poll(tfull[l], n):
                 yield ("tfull", l, n)
             for _ in range(4):
                 tdrain[l].arrive()
-            if not real:
+            if not real or first_only:
                 continue
             if l < nl - 1:
                 sq = seq[l] + (j - (pc["ra"] - e))
@@ -157,12 +167,12 @@ def simulate(nl, g, pieces, stages, verbose=False):
                     idx, phase = 0, phase ^ 1
         return
 
-    if nl == 2:   # one producer and stage-ring slice per layer (conv3x3_rdb.cuh: rdb_layer_producer)
+    if nl == 2 and not first_only:   # one producer and stage-ring slice per layer (conv3x3_rdb.cuh: rdb_layer_producer)
         ns0 = (stages + 1) // 2
         agents = {"producer0": layer_producer(0, 0, ns0), "producer1": layer_producer(1, ns0, stages - ns0)}
     else:
         agents = {"producer": producer()}
-    for l in range(nl):
+    for l in range(nact):
         agents[f"issuer{l}"] = issuer(l)
         agents[f"epi{l}"] = epilogue(l)
     blocked = {}
@@ -198,7 +208,7 @@ def simulate(nl, g, pieces, stages, verbose=False):
     return True, ticks
 
 
-def simulate_pair(g, pieces2, stages, lring=16, nl=2):
+def simulate_pair(g, pieces2, stages, lring=16, nl=2, first_only=False):
     """The CTA-pair forms; pieces2 = (rank 0's pieces, rank 1's pieces).  nl = 2: conv4 + conv5 (G = 4) -- the
     walk-order stage ring, per-layer landed rings of `lring`.  nl = 3: conv1..conv3 (G = 1) -- the x0 ring of `stages`
     row tiles, each x0 row loaded once and released by its last reader.  Every wait checks that the barrier is in the
@@ -206,6 +216,8 @@ def simulate_pair(g, pieces2, stages, lring=16, nl=2):
     phases after it); every arrival checks that it lands in the phase it is meant for."""
     xring = nl == 3
     assert not xring or g == 1
+    assert not first_only or nl == 2
+    nact = 1 if first_only else nl   # layers whose issuer / epilogue groups run
     ring = RINGS[nl]
     steps2 = [list(walk(p, nl)) for p in pieces2]
     # both CTAs take the same walk: pieces, rows, flush steps (only b / x0 / the owned pixels differ)
@@ -236,7 +248,7 @@ def simulate_pair(g, pieces2, stages, lring=16, nl=2):
         stage, phase, fill = 0, 0, 0
         fills = [0] * nl
         for (rnd, l, p, r, flush, n, seq) in steps2[c]:
-            if flush:
+            if flush or l >= nact:
                 continue
             for _ in range(g):
                 while not empty[c][stage].wait(fill // stages - 1):
@@ -329,7 +341,7 @@ def simulate_pair(g, pieces2, stages, lring=16, nl=2):
                 yield ("tfull", c, l, n)
             for _ in range(4):
                 tdrain[l].arrive(n)
-            if not real or l == nl - 1:
+            if not real or l == nl - 1 or first_only:
                 continue
             sq = seq[l] + (j - (pc["ra"] - e))
             slot = sq % ring[l]
@@ -339,7 +351,7 @@ def simulate_pair(g, pieces2, stages, lring=16, nl=2):
                 mfull[l][slot].arrive(sq // ring[l])
 
     agents = {f"producer{c}": (x0_producer(c) if xring else producer(c)) for c in range(2)}
-    for l in range(nl):
+    for l in range(nact):
         agents[f"issuer{l}"] = issuer(l)
         for c in range(2):
             agents[f"epi{l}@{c}"] = epilogue(c, l)
@@ -420,6 +432,23 @@ def main():
                 print(f"pair NL=3 G=1 x0 ring {xr} batch={batch} band_h={band_h} W={width} pairs={pairs} pair={u}: "
                       f"{'ok, ticks ' + str(info) if ok else 'DEADLOCK ' + str(info)}")
                 ok_all &= ok
+    # the conv4-only form: single CTAs with the launcher's 8 stages, pairs with 16; batch 1 has a phantom column
+    for batch, band_h, width, grid in [(1, 208, 416, 148), (16, 208, 416, 148), (64, 208, 416, 148), (3, 4, 200, 148),
+                                       (2, 9, 64, 13 * 2)]:
+        ntx = tiles_x(width, 2)
+        g1 = min(grid, batch * ntx * band_h)
+        for cta in sorted(set([0, 1, g1 // 2, g1 - 1])):
+            ok, info = simulate(2, 4, cta_pieces(cta, g1, batch, band_h, width, 2), 8, first_only=True)
+            print(f"conv4-only NL=2 G=4 batch={batch} band_h={band_h} W={width} grid={g1} cta={cta}: "
+                  f"{'ok, ticks ' + str(info) if ok else 'DEADLOCK ' + str(info)}")
+            ok_all &= ok
+        pairs = min(grid // 2, (batch * ntx + 1) // 2 * band_h)
+        for u in sorted(set([0, 1, pairs // 2, pairs - 1])):
+            pcs = [pair_pieces(2 * u + rank, 2 * pairs, batch, band_h, width, 2) for rank in (0, 1)]
+            ok, info = simulate_pair(4, pcs, 16, first_only=True)
+            print(f"conv4-only pair NL=2 G=4 batch={batch} band_h={band_h} W={width} pairs={pairs} pair={u}: "
+                  f"{'ok, ticks ' + str(info) if ok else 'DEADLOCK ' + str(info)}")
+            ok_all &= ok
     sys.exit(0 if ok_all else 1)
 
 

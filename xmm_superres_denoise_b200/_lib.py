@@ -160,6 +160,7 @@ SIGNATURES = {
     "xmm_wgrad_workspace_bytes": (c_size_t, []),
     "xmm_conv3x3_wgrad": (c_int, [POINTER(WgradParams), c_void_p]),
     "xmm_colsum_bf16": (c_int, [c_void_p, c_int, c_int, c_int, c_size_t, c_void_p, c_float, c_int, c_void_p]),
+    "xmm_copy_channels_bf16": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_size_t, c_void_p]),
     "xmm_colsum_multi_bf16": (c_int, [c_void_p, c_int, c_size_t, POINTER(ColsumSegment), c_int, c_void_p]),
     "xmm_colsum_multi_det_bf16": (c_int, [c_void_p, c_int, c_size_t, POINTER(ColsumSegment), c_int, c_void_p, c_size_t,
                                           c_void_p]),

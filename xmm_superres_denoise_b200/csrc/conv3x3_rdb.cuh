@@ -472,7 +472,7 @@ __device__ __forceinline__ void rdb_issuer(const RdbArgs& args, const RdbCtx& c,
 // Four warps per layer (one per TMEM lane quarter) drain that layer's rows in order.
 // PAIR: the peer's warps arrive on the LEADER's tdrain / mfull (relaxed: a release.cluster arrive would wait for this
 // warp's global stores as well and stall the epilogue).
-template <int G, int NL, int L, bool PAIR>
+template <int G, int NL, int L, bool PAIR, bool FIRST_ONLY = false>
 __device__ __forceinline__ void rdb_epilogue(const RdbArgs& args, const RdbCtx& c, const RdbSched<NL, PAIR>& sched, int q,
                                              int lane) {
   const bool remote = PAIR && sched.rank != 0;
@@ -616,7 +616,7 @@ __device__ __forceinline__ void rdb_epilogue(const RdbArgs& args, const RdbCtx& 
         st_global_256(gp, o[0], o[1]);
         st_global_256(gp + 16, o[2], o[3]);
       }
-      if (!last) {
+      if (!last && !FIRST_ONLY) {
         // the next layers' A operand: row j of map L, swizzled as a TMA load would have written it; zeros outside
         // the image (padding) and on the junk lanes
         const int sq = seq + (j - (pc.ra - e));
@@ -758,10 +758,15 @@ __device__ __forceinline__ void rdb_x0_producer(const CUtensorMap* tmap_in, cons
 // order in which the layers' rows are loaded), warp 1 + l = MMA issuer of layer l, warps 4 + 4 l .. 7 + 4 l = epilogue
 // of layer l.  Issuers and epilogue groups only know their own layer; everything between roles is an mbarrier.
 // PAIR: launched as clusters of 2 (see the top of this file).
-template <int G, int NL, bool PAIR = false>
+// FIRST_ONLY (conv4 + conv5 only): the conv4-only form that recomputes x4 for a backward pass.  It keeps the two-layer
+// work split, walk and conv4 accumulator rule, so x4 is bit-equal to what the full kernel stores; conv5's issuer and
+// epilogue group do nothing, the producer loads conv4's chunks only and conv4's epilogue writes no map rows.
+template <int G, int NL, bool PAIR = false, bool FIRST_ONLY = false>
 __global__ void __launch_bounds__(kRdbThreads, 1)
 conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs args) {
   static_assert(NL == 2 || NL == 3, "two or three fused layers");
+  static_assert(!FIRST_ONLY || NL == 2, "the conv4-only form is a form of conv4 + conv5");
+  constexpr int NA = FIRST_ONLY ? 1 : NL;  // layers that run
   static_assert(NL * kRdbSlotCols <= 512, "accumulators exceed TMEM");
   constexpr int NM = NL - 1;  // in-CTA maps
   constexpr int kR = kRdbLRing<PAIR>;
@@ -824,9 +829,9 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
 
   if (warp == 0 && ptx::elect_one()) {  // weights + biases of every layer (the accumulators are initialised from them)
     uint32_t wtot = 0;
-    for (int l = 0; l < NL; ++l) wtot += args.layer[l].w_bytes + 128u;
+    for (int l = 0; l < NA; ++l) wtot += args.layer[l].w_bytes + 128u;
     ptx::mbar_expect_tx(c.w_bar, wtot);
-    for (int l = 0; l < NL; ++l) {
+    for (int l = 0; l < NA; ++l) {
       const uint8_t* gsrc = static_cast<const uint8_t*>(args.layer[l].wblob);
       uint8_t* dst = c.w_s + args.layer[l].smem_off;
       const uint32_t wb = args.layer[l].w_bytes;
@@ -852,7 +857,7 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
     ptx::fence_proxy_async();
     // Every MMA accumulates.  A row's accumulator (window slots 0..2) starts as the layer's BIAS, its carry slot
     // (3, 4) as zero: the epilogue re-initialises a slot right after draining it and never adds the bias itself.
-    if (egroup < NL) {
+    if (egroup < NA) {
       rdb_wait(c.w_bar, 0, 9, 0, 0);
       const uint32_t lane_base = c.tmem_base + (uint32_t((warp & 3) * 32) << 16) + uint32_t(egroup * kRdbSlotCols);
       const float* bias_s = reinterpret_cast<const float*>(c.w_s + args.layer[egroup].smem_off + args.layer[egroup].w_bytes);
@@ -874,7 +879,7 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
   RdbSched<NL, PAIR> sched;
   sched.init(args);
 
-  if (!PAIR && NL == 2 && args.split_producers && (warp == 0 || warp == 3)) {
+  if (!PAIR && NL == 2 && !FIRST_ONLY && args.split_producers && (warp == 0 || warp == 3)) {
     // ------------------------------------------------------------ TMA producers, one per layer (warps 0 and 3)
     if constexpr (!PAIR) {
       if (ptx::elect_one()) {
@@ -900,7 +905,7 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
 #pragma unroll
       for (int l = 0; l < NL; ++l) fills[l] = 0;
       rdb_walk<NL>(sched, [&](int l, const RdbPiece& pc, int r, bool flush, int, const int*) {
-        if (flush) return;
+        if (flush || (FIRST_ONLY && l > 0)) return;
         // input row r of both bands; above / below a band: the neighbouring band's rows (outside the image: zeros)
         int row = r, band0 = 0;
         if (r < 0) {
@@ -955,16 +960,16 @@ conv3x3_rdb_kernel(const __grid_constant__ CUtensorMap tmap_in, const RdbArgs ar
     }
   } else if (warp <= 3) {
     // (warp 3 of a two-layer kernel: idle, or the second producer above; PAIR: the peer issues nothing)
-    if (warp - 1 < NL && rank == 0 && ptx::elect_one()) {
+    if (warp - 1 < NA && rank == 0 && ptx::elect_one()) {
       if (warp == 1) rdb_issuer<G, NL, 0, PAIR>(args, c, sched);
       if (warp == 2) rdb_issuer<G, NL, 1, PAIR>(args, c, sched);
       if constexpr (NL == 3) {
         if (warp == 3) rdb_issuer<G, NL, 2, PAIR>(args, c, sched);
       }
     }
-  } else if (egroup < NL) {
+  } else if (egroup < NA) {
     const int q = warp & 3;  // TMEM lane quarter this warp may read
-    if (egroup == 0) rdb_epilogue<G, NL, 0, PAIR>(args, c, sched, q, lane);
+    if (egroup == 0) rdb_epilogue<G, NL, 0, PAIR, FIRST_ONLY>(args, c, sched, q, lane);
     if (egroup == 1) rdb_epilogue<G, NL, 1, PAIR>(args, c, sched, q, lane);
     if constexpr (NL == 3) {
       if (egroup == 2) rdb_epilogue<G, NL, 2, PAIR>(args, c, sched, q, lane);

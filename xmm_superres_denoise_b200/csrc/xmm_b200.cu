@@ -759,11 +759,13 @@ const char* rdb_blocker(const xmm_conv3x3_params* L, int n, const DeviceInfo& de
 
 // PAIR: clusters of two CTAs that share every MMA (conv3x3_rdb.cuh): each holds half of the weights, so 14 instead of
 // 5 TMA stages fit next to conv4 + conv5's, and an x0 ring of 11 rows next to conv1..conv3's.
-template <int G, int NL, bool PAIR>
+// FIRST_ONLY: the conv4-only form (L[0] only; conv5's weights are not loaded, and there is no map ring).
+template <int G, int NL, bool PAIR, bool FIRST_ONLY = false>
 int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo& dev, cudaStream_t stream) {
+  constexpr int NA = FIRST_ONLY ? 1 : NL;
   RdbArgs a{};
   uint32_t off = 0;
-  for (int l = 0; l < NL; ++l) {
+  for (int l = 0; l < NA; ++l) {
     const xmm_conv3x3_params& p = L[l];
     a.layer[l].wblob = p.wblob_row;
     a.layer[l].w_bytes = uint32_t(p.cin / 32) * 9u * uint32_t(kRdbTapBytes) / (PAIR ? 2u : 1u);
@@ -776,7 +778,7 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
     a.layer[l].out_coff = p.out_coff;
   }
   a.w_total = off;
-  const xmm_conv3x3_params& pl = L[NL - 1];
+  const xmm_conv3x3_params& pl = L[NA - 1];
   a.cin_off = L[0].in_coff;
   a.batch = L[0].batch;
   a.height = L[0].height;
@@ -795,7 +797,7 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
   constexpr int kBarBytes = 1024;
   const long long room = (long long)dev.max_smem_optin - 1024 - kBarBytes - (long long)a.w_total;
   int tiles = int(room / kRdbTileBytes);
-  a.ring0 = NL == 3 ? 5 : 2;  // (two fused layers: x4 is read one row behind its producer -- two tiles, one more TMA stage)
+  a.ring0 = FIRST_ONLY ? 0 : NL == 3 ? 5 : 2;  // (two fused layers: x4 is read one row behind its producer -- two tiles, one more TMA stage)
   a.ring1 = NL == 3 ? 3 : 0;
   a.stages = tiles - a.ring0 - a.ring1;
   if (a.stages > kRdbLRing<PAIR>) a.stages = kRdbLRing<PAIR>;
@@ -808,11 +810,11 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
   // measured (profiles/r02_rdb_v8_split_producers.log): 3.08 ms per block against 2.87 ms with one producer and one shared
   // ring -- rings of 3 + 2 stages are less elastic than one of 5 -- so it is off (and not built for pairs)
   static const int split_env = env_int("XMM_RDB_SPLIT_PRODUCERS", 0);
-  a.split_producers = (!PAIR && NL == 2 && split_env && a.stages >= 4) ? 1 : 0;
+  a.split_producers = (!PAIR && NL == 2 && !FIRST_ONLY && split_env && a.stages >= 4) ? 1 : 0;
   CUtensorMap tmap;
   int rc = cached_band_tmap(&tmap, L[0].in, a.batch, a.height, a.width, L[0].in_ctot, a.band_h, 2, 32, kRdbBoxPx, 2);
   if (rc != XMM_OK) return rc;
-  const void* kernel = reinterpret_cast<const void*>(conv3x3_rdb_kernel<G, NL, PAIR>);
+  const void* kernel = reinterpret_cast<const void*>(conv3x3_rdb_kernel<G, NL, PAIR, FIRST_ONLY>);
   rc = ensure_max_smem(kernel, dev);
   if (rc != XMM_OK) return rc;
   const size_t smem = 1024 + size_t(a.w_total) + size_t(a.stages + a.ring0 + a.ring1) * kRdbTileBytes + kBarBytes;
@@ -835,7 +837,7 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
     static int max_clusters = 0;
     if (max_clusters == 0) {
       cfg.gridDim = dim3(unsigned(2 * dev.sm_count));
-      XMM_CUDA_OK(cudaOccupancyMaxActiveClusters(&max_clusters, conv3x3_rdb_kernel<G, NL, PAIR>, &cfg));
+      XMM_CUDA_OK(cudaOccupancyMaxActiveClusters(&max_clusters, conv3x3_rdb_kernel<G, NL, PAIR, FIRST_ONLY>, &cfg));
       if (max_clusters < 1) return fail(XMM_ERR_UNSUPPORTED_SHAPE, "conv3x3 (fused dense block): no CTA pair fits an SM pair");
     }
     long long pairs = a.total_rows < max_clusters ? a.total_rows : max_clusters;
@@ -856,9 +858,9 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
     a.prof = prof_dev;
   }
   if constexpr (PAIR) {
-    XMM_CUDA_OK(cudaLaunchKernelEx(&cfg, conv3x3_rdb_kernel<G, NL, PAIR>, tmap, a));
+    XMM_CUDA_OK(cudaLaunchKernelEx(&cfg, conv3x3_rdb_kernel<G, NL, PAIR, FIRST_ONLY>, tmap, a));
   } else {
-    conv3x3_rdb_kernel<G, NL, PAIR><<<cfg.gridDim, kRdbThreads, smem, stream>>>(tmap, a);
+    conv3x3_rdb_kernel<G, NL, PAIR, FIRST_ONLY><<<cfg.gridDim, kRdbThreads, smem, stream>>>(tmap, a);
     XMM_CUDA_OK(cudaGetLastError());
   }
   if (prof_env) {
@@ -872,7 +874,8 @@ int launch_rdb(const xmm_conv3x3_params* L, const bool* store, const DeviceInfo&
         "epi0 drain (ld+st+arrive)", "epi0 math+pack", "epi0 map write+fence+arrive", "epi0 global store",
         "epi1 drain (ld+st+arrive)", "epi1 math+residuals+pack", "epi1 map write (none)", "epi1 global store",
         "", "", "", ""};
-    fprintf(stderr, "conv3x3_rdb<%d,%d%s> grid %lld stages %d:", G, NL, PAIR ? ",pair" : "", grid, a.stages);
+    fprintf(stderr, "conv3x3_rdb<%d,%d%s%s> grid %lld stages %d:", G, NL, PAIR ? ",pair" : "", FIRST_ONLY ? ",first" : "",
+            grid, a.stages);
     for (int k = 0; k < 20; ++k) {
       // (the issuer counters: of the CTAs that issue -- in pairs, the leaders)
       double sum = 0;
@@ -899,11 +902,18 @@ int rdb_pair(int mode_flags) {
 }
 
 // conv1..conv3 in one launch, conv4..conv5 in a second one.  skip_dead: x4 is read by nobody after this block
-// (inference), so it is never written.  pair: rdb_pair's mask.
-int launch_rdb_block(const xmm_conv3x3_params* L, bool skip_dead, int pair, const DeviceInfo& dev, cudaStream_t stream) {
+// (inference), so it is never written.  skip_last: x1..x4 only (recompute for a backward pass), conv4 in the conv4-only
+// form of the second kernel.  pair: rdb_pair's mask.
+int launch_rdb_block(const xmm_conv3x3_params* L, bool skip_dead, bool skip_last, int pair, const DeviceInfo& dev,
+                     cudaStream_t stream) {
   const bool store_a[3] = {true, true, true};
   int rc = (pair & 1) ? launch_rdb<1, 3, true>(L, store_a, dev, stream) : launch_rdb<1, 3, false>(L, store_a, dev, stream);
   if (rc != XMM_OK) return rc;
+  if (skip_last) {
+    const bool store_c[1] = {true};
+    return (pair & 2) ? launch_rdb<4, 2, true, true>(L + 3, store_c, dev, stream)
+                      : launch_rdb<4, 2, false, true>(L + 3, store_c, dev, stream);
+  }
   const bool store_b[2] = {!skip_dead, true};
   return (pair & 2) ? launch_rdb<4, 2, true>(L + 3, store_b, dev, stream) : launch_rdb<4, 2, false>(L + 3, store_b, dev, stream);
 }
@@ -924,11 +934,14 @@ extern "C" int xmm_conv3x3_chain_bf16(const xmm_conv3x3_params* layers, int nlay
   g_last_chain_launches = 0;
   const int mode = mode_flags & 0xff;
   const bool skip_dead = (mode_flags & XMM_CHAIN_SKIP_DEAD_STORES) != 0;
-  constexpr int kFlags = XMM_CHAIN_SKIP_DEAD_STORES | XMM_CHAIN_RDB_PAIR | XMM_CHAIN_RDB_SINGLE;
+  const bool skip_last = (mode_flags & XMM_CHAIN_SKIP_LAST) != 0;
+  constexpr int kFlags = XMM_CHAIN_SKIP_DEAD_STORES | XMM_CHAIN_RDB_PAIR | XMM_CHAIN_RDB_SINGLE | XMM_CHAIN_SKIP_LAST;
   XMM_REQUIRE(mode >= 0 && mode <= 3 && (mode_flags & ~(0xff | kFlags)) == 0 &&
                   (mode_flags & (XMM_CHAIN_RDB_PAIR | XMM_CHAIN_RDB_SINGLE)) != (XMM_CHAIN_RDB_PAIR | XMM_CHAIN_RDB_SINGLE),
               "conv3x3_chain: mode must be 0 (auto), 1 (pipelined), 2 (layer by layer) or 3 (fused dense block), with at most "
               "one of the pair / single flags");
+  XMM_REQUIRE(!(skip_dead && skip_last), "conv3x3_chain: XMM_CHAIN_SKIP_LAST and XMM_CHAIN_SKIP_DEAD_STORES exclude each other");
+  XMM_REQUIRE(!skip_last || nlayers >= 2, "conv3x3_chain: XMM_CHAIN_SKIP_LAST needs at least two layers");
   DeviceInfo dev;
   int rc = require_sm100(&dev);
   if (rc != XMM_OK) return rc;
@@ -943,25 +956,26 @@ extern "C" int xmm_conv3x3_chain_bf16(const xmm_conv3x3_params* layers, int nlay
     const char* why_not = rdb_blocker(layers, nlayers, dev);
     if (why_not == nullptr) {
       g_last_chain_launches = 2;
-      return launch_rdb_block(layers, skip_dead, rdb_pair(mode_flags), dev, s);
+      return launch_rdb_block(layers, skip_dead, skip_last, rdb_pair(mode_flags), dev, s);
     }
     if (mode == 3) return fail(XMM_ERR_UNSUPPORTED_SHAPE, "conv3x3_chain: cannot fuse the dense block (%s)", why_not);
   }
   const char* why = chain_blocker(layers, nlayers);
   bool pipelined = mode == 1 && why == nullptr;
   if (mode == 1 && why != nullptr) return fail(XMM_ERR_UNSUPPORTED_SHAPE, "conv3x3_chain: cannot pipeline (%s)", why);
-  if (pipelined) {
+  const int nrun = skip_last ? nlayers - 1 : nlayers;
+  if (pipelined && !skip_last) {
     const size_t need = xmm_conv3x3_chain_workspace_bytes(nlayers, layers[0].batch, layers[0].height);
     XMM_REQUIRE(workspace != nullptr && workspace_bytes >= need && (reinterpret_cast<uintptr_t>(workspace) & 3) == 0,
                 "conv3x3_chain: workspace of %zu bytes needed (got %zu)", need, workspace_bytes);
     g_last_chain_launches = 1;
     return launch_chain(layers, nlayers, dev, static_cast<int*>(workspace), s);
   }
-  for (int l = 0; l < nlayers; ++l) {
+  for (int l = 0; l < nrun; ++l) {
     rc = xmm_conv3x3_bf16(&layers[l], stream);
     if (rc != XMM_OK) return rc;
   }
-  g_last_chain_launches = nlayers;
+  g_last_chain_launches = nrun;
   return XMM_OK;
 }
 
@@ -1342,6 +1356,48 @@ extern "C" int xmm_colsum_bf16(const void* in, int ctot, int c0, int n, size_t n
                                int accumulate, void* stream) {
   xmm_colsum_segment g{c0, n, out, scale, accumulate};
   return xmm_colsum_multi_bf16(in, ctot, npix, &g, 1, stream);
+}
+
+// ----------------------------------------------------------------------------- channel-window copy
+namespace {
+// One 16-byte vector (8 channels of one pixel) per thread and turn; consecutive threads take consecutive vectors of a
+// pixel, then the next pixel, so each warp reads and writes whole runs of the two windows.
+__global__ void __launch_bounds__(256) copy_channels_kernel(const uint4* __restrict__ src, int src_ctot8, int src_coff8,
+                                                            uint4* __restrict__ dst, int dst_ctot8, int dst_coff8,
+                                                            int nvec, size_t total) {
+  const size_t stride = size_t(gridDim.x) * blockDim.x;
+  for (size_t v = size_t(blockIdx.x) * blockDim.x + threadIdx.x; v < total; v += stride) {
+    const size_t pix = v / unsigned(nvec);
+    const int k = int(v - pix * unsigned(nvec));
+    dst[pix * dst_ctot8 + dst_coff8 + k] = __ldg(src + pix * src_ctot8 + src_coff8 + k);
+  }
+}
+}  // namespace
+
+extern "C" int xmm_copy_channels_bf16(const void* src, int src_ctot, int src_coff, void* dst, int dst_ctot, int dst_coff,
+                                      int channels, size_t npix, void* stream) {
+  DeviceInfo dev;
+  int rc = require_sm100(&dev);
+  if (rc != XMM_OK) return rc;
+  XMM_REQUIRE(src && dst, "copy_channels: null tensor pointer");
+  XMM_REQUIRE((reinterpret_cast<uintptr_t>(src) & 15) == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0,
+              "copy_channels: pointers must be 16-byte aligned");
+  XMM_REQUIRE(channels > 0 && channels % 8 == 0 && src_ctot % 8 == 0 && dst_ctot % 8 == 0 && src_coff % 8 == 0 &&
+                  dst_coff % 8 == 0,
+              "copy_channels: channel counts and offsets must be multiples of 8");
+  XMM_REQUIRE(src_coff >= 0 && src_coff + channels <= src_ctot && dst_coff >= 0 && dst_coff + channels <= dst_ctot,
+              "copy_channels: window [%d,%d) of %d -> [%d,%d) of %d", src_coff, src_coff + channels, src_ctot, dst_coff,
+              dst_coff + channels, dst_ctot);
+  if (npix == 0) return XMM_OK;
+  const int nvec = channels / 8;
+  const size_t total = npix * size_t(nvec);
+  const size_t want = (total + 255) / 256, cap = size_t(dev.sm_count) * 16;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  copy_channels_kernel<<<unsigned(want < cap ? want : cap), 256, 0, s>>>(
+      static_cast<const uint4*>(src), src_ctot / 8, src_coff / 8, static_cast<uint4*>(dst), dst_ctot / 8, dst_coff / 8,
+      nvec, total);
+  XMM_CUDA_OK(cudaGetLastError());
+  return XMM_OK;
 }
 
 extern "C" size_t xmm_det_slots(int site, int batch, int height, int width, int channels) {

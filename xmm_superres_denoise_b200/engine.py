@@ -305,14 +305,21 @@ class RRDBEngine(_LayerPlans):
         return bufs
 
     # ------------------------------------------------------------------ dense blocks
+    def _rdb_layers(self, name: str, buf: torch.Tensor, out: torch.Tensor, *, s0: float, s1: float,
+                    r2: Optional[torch.Tensor], s2: float):
+        """The launches of one ResidualDenseBlock_5C.forward: conv1..conv4 (x1..x4 into buf), conv5 (into out)."""
+        f = self.nf
+        first4 = []
+        for k in range(1, 5):
+            first4 += self._conv(f"{name}.{k}", buf, 0, k * f, buf, k * f, lrelu=0.2)
+        return first4, self._conv(f"{name}.5", buf, 0, 5 * f, out, 0, s0=s0, r1=buf, r1_coff=0, s1=s1, r2=r2, r2_coff=0,
+                                  s2=s2)
+
     def _rdb_forward(self, name: str, buf: torch.Tensor, out: torch.Tensor, *, s0: float, s1: float,
                      r2: Optional[torch.Tensor], s2: float) -> None:
         """One ResidualDenseBlock_5C (rrdb_blocks.py:37-54): x in buf[..., :F]; result -> out[..., :F]."""
-        f = self.nf
-        layers = []
-        for k in range(1, 5):
-            layers += self._conv(f"{name}.{k}", buf, 0, k * f, buf, k * f, lrelu=0.2)
-        layers += self._conv(f"{name}.5", buf, 0, 5 * f, out, 0, s0=s0, r1=buf, r1_coff=0, s1=s1, r2=r2, r2_coff=0, s2=s2)
+        first4, last = self._rdb_layers(name, buf, out, s0=s0, s1=s1, r2=r2, s2=s2)
+        layers = first4 + last
         if len(layers) == 5:
             # inference keeps nothing of a block but its output: x4 need not be written (training reads x1..x4 back)
             ops.conv3x3_chain(layers, self.chain_mode | (0 if self._keep_all else ops.CHAIN_SKIP_DEAD_STORES))
@@ -320,9 +327,10 @@ class RRDBEngine(_LayerPlans):
             self._run(layers)
 
     def _trunk_forward(self, x: torch.Tensor, rdb_bufs: List[torch.Tensor], fea: torch.Tensor,
-                       trunk_out: torch.Tensor) -> None:
+                       trunk_out: torch.Tensor, ckpt: Optional[torch.Tensor] = None) -> None:
         """_GeneratorRRDB.forward (generator_rrdb.py:66-69).  rdb_bufs: 3 buffers (ping-pong, inference)
-        or 3*nb + 1 buffers (training: every dense block keeps its activations)."""
+        or 3*nb + 1 buffers (training: every dense block keeps its activations).  ckpt (3 buffers, memory-efficient
+        training): [3*nb + 1, B, H, W, F]; dense block k's output is copied to ckpt[k + 1] (fea is ckpt[0])."""
         g, f = self.gen, self.nf
         ring = len(rdb_bufs)
         keep_all = ring > 3
@@ -346,6 +354,8 @@ class RRDBEngine(_LayerPlans):
                     # (x5 * 0.2 + x_rdb3) * 0.2 + x_rrdb   (rrdb_blocks.py:54,70)
                     self._rdb_forward(f"f.{i}.{r}", cur, nxt, s0=0.04, s1=0.2, r2=x_rrdb, s2=1.0)
                 idx += 1
+                if ckpt is not None:
+                    ops.copy_channels(nxt, 0, ckpt[idx], 0, f)
         last = rdb_bufs[idx % ring]
         self._run(self._conv("f.trunk", last, 0, f, trunk_out, 0, s0=1.0, r1=fea, r1_coff=0, s1=1.0))
 

@@ -15,6 +15,13 @@ explicit launch sequence over the same two tensor-core kernels:
 Buffers per dense block: activations A = [x0|x1|x2|x3|x4] (kept from the forward), gradients
 G = [dY1|dY2|dY3|dY4|g] where g = dL/d(block output) (conv5's 0.2 is folded into the packed
 weights).  Three G buffers rotate: RDB3 -> ring[2], RDB2 -> ring[1], RDB1 -> ring[0].
+
+Memory-efficient training (the generator's ``memory_efficient``, what the reference does with torch.utils.checkpoint
+in ResidualDenseBlock_5C): the forward runs as inference does, on the three rotating buffers, and keeps only every
+block's F-channel input (``ckpt``).  Before a block's backward, its input is copied into one 5F scratch buffer and
+conv1..conv4 run again (XMM_CHAIN_SKIP_LAST: the same kernels on the same inputs, so x1..x4 are bit-identical to the
+ones the other mode keeps); the scratch buffer is then that block's A.  The rotating forward buffers double as the
+gradient ring: the forward is over before the backward writes them.
 """
 from __future__ import annotations
 
@@ -69,8 +76,8 @@ class TrainEngine(RRDBEngine):
         self._det: Optional[determinism.DetPlan] = None  # the running backward's plan in deterministic mode
 
     # ------------------------------------------------------------------ buffers
-    def _train_buffers(self, b: int, h: int, w: int, device: torch.device) -> Dict[str, object]:
-        key = ("train", b, h, w, str(device))
+    def _train_buffers(self, b: int, h: int, w: int, device: torch.device, memeff: bool) -> Dict[str, object]:
+        key = ("train", memeff, b, h, w, str(device))
         bufs = self._bufs.get(key)
         if bufs is None:
             self._bufs.clear()
@@ -78,11 +85,16 @@ class TrainEngine(RRDBEngine):
             f = self.nf
             bf = dict(dtype=torch.bfloat16, device=device)
             nrdb = 3 * self.nb
-            act = [torch.empty(b, h, w, 5 * f, **bf) for _ in range(nrdb)]
-            act.append(torch.empty(b, h, w, f, **bf))  # output of the last RRDB
-            bufs = {"act": act, "trunk": torch.empty(b, h, w, f, **bf),
+            bufs = {"trunk": torch.empty(b, h, w, f, **bf),
                     "ring": [torch.empty(b, h, w, 5 * f, **bf) for _ in range(3)],
                     "d_trunk": torch.empty(b, h, w, f, **bf), "d_fea": torch.empty(b, h, w, f, **bf)}
+            if memeff:  # every block's input (and the last RRDB's output) + one block's recomputed activations
+                bufs["ckpt"] = torch.empty(nrdb + 1, b, h, w, f, **bf)
+                bufs["scratch"] = torch.empty(b, h, w, 5 * f, **bf)
+            else:
+                act = [torch.empty(b, h, w, 5 * f, **bf) for _ in range(nrdb)]
+                act.append(torch.empty(b, h, w, f, **bf))  # output of the last RRDB
+                bufs["act"] = act
             hh, ww = h, w
             if self.kind == "sr":
                 for s in range(self.num_upsample):
@@ -102,9 +114,12 @@ class TrainEngine(RRDBEngine):
         x = x.contiguous().float()
         b, _, h, w = x.shape
         self.arena.ensure(x.device)
-        bufs = self._train_buffers(b, h, w, x.device)
+        bufs = self._train_buffers(b, h, w, x.device, bool(g.memory_efficient))
         self.generation += 1
-        self._trunk_forward(x, bufs["act"], bufs["act"][0], bufs["trunk"])
+        if "ckpt" in bufs:
+            self._trunk_forward(x, bufs["ring"], bufs["ckpt"][0], bufs["trunk"], ckpt=bufs["ckpt"])
+        else:
+            self._trunk_forward(x, bufs["act"], bufs["act"][0], bufs["trunk"])
         if self.kind == "dn":
             if g.in_channels != g.out_channels:
                 raise RuntimeError("GeneratorRRDB_DN adds its input to its output: in_channels must equal out_channels")
@@ -188,10 +203,28 @@ class TrainEngine(RRDBEngine):
             else:
                 self._colsum(dy, [(0, n, db, 1.0, True)])  # db is a view of the zero-initialised flat buffer
 
+    def _block_act(self, bufs, i: int, r: int) -> torch.Tensor:
+        """A = [x0|x1|x2|x3|x4] of dense block (i, r): kept from the forward, or (memory-efficient) the scratch buffer
+        _recompute filled."""
+        return bufs["scratch"] if "ckpt" in bufs else bufs["act"][3 * i + r]
+
+    def _recompute(self, i: int, r: int, bufs) -> None:
+        """Memory-efficient training: x0 of dense block (i, r) from its checkpoint, then x1..x4 by the block's own forward
+        launches.  conv5's output argument is the next checkpoint slot; XMM_CHAIN_SKIP_LAST never writes it."""
+        f, ckpt, A = self.nf, bufs["ckpt"], bufs["scratch"]
+        k = 3 * i + r
+        ops.copy_channels(ckpt[k], 0, A, 0, f)
+        s0, s1, r2, s2 = (0.04, 0.2, ckpt[3 * i], 1.0) if r == 2 else (0.2, 1.0, None, 0.0)
+        first4, last = self._rdb_layers(f"f.{i}.{r}", A, ckpt[k + 1], s0=s0, s1=s1, r2=r2, s2=s2)
+        if len(first4) + len(last) == 5:  # the forward's decision (fused / layer by layer), conv5 left out
+            ops.conv3x3_chain(first4 + last, self.chain_mode | ops.CHAIN_SKIP_LAST)
+        else:  # split layers (F = 64): the forward's plain launches of conv1..conv4
+            self._run(first4)
+
     def _rdb_backward(self, i: int, r: int, bufs, grads, d_fea: torch.Tensor) -> None:
         f, kc, a = self.nf, self.kc, self.arena
-        act, ring = bufs["act"], bufs["ring"]
-        A, G = act[3 * i + r], ring[r]
+        ring = bufs["ring"]
+        A, G = self._block_act(bufs, i, r), ring[r]
         rdb = self._rdb(i, r)
         layers = []
         for j in range(4, 0, -1):  # dY_j = LeakyReLU'(x_j) * sum_k dgrad_k(dY_k); its column sums are conv_j's bias grad
@@ -232,7 +265,7 @@ class TrainEngine(RRDBEngine):
         f = self.nf
         rrdb = self.gen.rrdb[i]
         rdb = (rrdb.RDB1, rrdb.RDB2, rrdb.RDB3)[r]
-        A, G = bufs["act"][3 * i + r], bufs["ring"][r]
+        A, G = self._block_act(bufs, i, r), bufs["ring"][r]
         s5 = 0.04 if r == 2 else 0.2
         convs = [getattr(rdb, f"conv{k}") for k in range(1, 6)]
         dws = [self._gv(grads, c.weight) for c in convs]
@@ -342,7 +375,7 @@ class TrainEngine(RRDBEngine):
                 self._single_conv_wgrad(g.upsampling[3 * s], ups[s], dy, grads, perm=1)
             self._run(self._conv(blob, dy, 0, nin, bufs["d_trunk"], 0))
         d_trunk = bufs["d_trunk"]  # dL/d(fea + trunk_conv(...)): feeds trunk_conv and the `fea` skip
-        last_act = bufs["act"][3 * self.nb]
+        last_act = bufs["ckpt"][3 * self.nb] if "ckpt" in bufs else bufs["act"][3 * self.nb]
         self._single_conv_wgrad(g.trunk_conv, last_act, d_trunk, grads)
         ring = bufs["ring"]
         d_fea = bufs["d_fea"]
@@ -351,6 +384,8 @@ class TrainEngine(RRDBEngine):
                                  **self._bias_sum(grads, self._rdb(self.nb - 1, 2).conv5, 0.04)))
             for i in range(self.nb - 1, -1, -1):
                 for r in (2, 1, 0):
+                    if "ckpt" in bufs:
+                        self._recompute(i, r, bufs)
                     self._rdb_backward(i, r, bufs, grads, d_fea)
                     self._rdb_wgrad(i, r, bufs, grads)
                 if det is not None:  # this RRDB's (and, first time round, the tail layers') reductions, in order

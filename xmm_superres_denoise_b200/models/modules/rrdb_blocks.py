@@ -23,8 +23,10 @@ def make_layer(block, n_layers):
 class ResidualDenseBlock_5C(nn.Module):
     def __init__(self, nf=64, gc=32, bias=True, memory_efficient: bool = False):
         super().__init__()
-        # memory_efficient (activation checkpointing of the concats, rrdb_blocks.py:17-19,39-47)
-        # is accepted for API compatibility: there are no concat tensors to checkpoint here.
+        # memory_efficient (activation checkpointing of the concats, rrdb_blocks.py:17-19,39-47): training reads the
+        # GENERATOR's flag (engine_train.TrainEngine), keeps each dense block's input only and recomputes x1..x4 in the
+        # backward pass.  A per-block mix is not supported: this block's own flag is kept for API compatibility only.
+        # Inference ignores the flag, as checkpointing does.
         self.mem_efficient = memory_efficient
         self.nf, self.gc = nf, gc
         self.conv1 = nn.Conv2d(nf, gc, 3, 1, 1, bias=bias)

@@ -114,6 +114,7 @@ _TORCH_FWD_KEYS = {"lrelu", "s0", "r1", "r1_coff", "s1", "r2", "r2_coff", "s2", 
 CHAIN_AUTO, CHAIN_PIPELINED, CHAIN_LAYER_BY_LAYER, CHAIN_FUSED = 0, 1, 2, 3
 CHAIN_SKIP_DEAD_STORES = 0x100  # flag: outputs of layers 1..n-1 are not read after the call (inference)
 CHAIN_RDB_PAIR, CHAIN_RDB_SINGLE = 0x200, 0x400  # flags: both kernels of the fused block as CTA pairs / single CTAs
+CHAIN_SKIP_LAST = 0x800  # flag: layers 1..n-1 only, the last layer's output is not written (recompute for a backward)
 _chain_ws: dict = {}
 _chain_ws_retired: list = []  # outgrown workspaces stay allocated: a captured CUDA graph may still hold their address
 
@@ -124,7 +125,7 @@ def conv3x3_chain(layers, mode: int = CHAIN_AUTO) -> None:
     calling conv3x3 on them in order (up to fp32 summation order).  mode: CHAIN_AUTO (the fused dense-block kernels
     where the layers qualify, else layer by layer) / CHAIN_PIPELINED (one launch, layers pipelined over SM groups) /
     CHAIN_LAYER_BY_LAYER / CHAIN_FUSED (error if the layers are not a dense block), optionally
-    ``| CHAIN_SKIP_DEAD_STORES`` and ``| CHAIN_RDB_PAIR`` or ``| CHAIN_RDB_SINGLE``."""
+    ``| CHAIN_SKIP_DEAD_STORES`` or ``| CHAIN_SKIP_LAST``, and ``| CHAIN_RDB_PAIR`` or ``| CHAIN_RDB_SINGLE``."""
     n = len(layers)
     arr = (Conv3x3Params * n)()
     for p, (a, kw) in zip(arr, layers):
@@ -142,6 +143,19 @@ def conv3x3_chain(layers, mode: int = CHAIN_AUTO) -> None:
     global LAST_CHAIN_LAUNCHES
     LAST_CHAIN_LAUNCHES = int(lib.xmm_last_chain_launches())  # 2 fused, 1 pipelined, n layer by layer
     _count(LAST_CHAIN_LAUNCHES)
+
+
+def copy_channels(src: torch.Tensor, src_coff: int, dst: torch.Tensor, dst_coff: int, channels: int) -> None:
+    """dst[..., dst_coff:dst_coff+channels] = src[..., src_coff:src_coff+channels] for two NHWC bf16 buffers of the same
+    spatial shape (a dense block's input into and out of its 5F-channel buffer); 16-byte accesses."""
+    _nhwc(src, "copy_channels source")
+    _nhwc(dst, "copy_channels destination")
+    if tuple(src.shape[:3]) != tuple(dst.shape[:3]):
+        raise RuntimeError(f"copy_channels: spatial shapes {tuple(src.shape[:3])} and {tuple(dst.shape[:3])} differ")
+    b, h, w, _ = src.shape
+    _lib.check(_lib.load().xmm_copy_channels_bf16(src.data_ptr(), src.shape[3], src_coff, dst.data_ptr(), dst.shape[3],
+                                                  dst_coff, channels, b * h * w, _lib.stream_ptr()))
+    _count()
 
 
 def conv_first(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor], out: torch.Tensor,

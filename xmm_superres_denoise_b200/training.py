@@ -202,8 +202,9 @@ class TrainStep:
         return st, flat_grad
 
     def __call__(self, lr_img: torch.Tensor, hr_img: torch.Tensor) -> torch.Tensor:
-        # (the deterministic mode changes the backward's launches: a graph is captured per mode)
-        key = (tuple(lr_img.shape), tuple(hr_img.shape), lr_img.dtype, hr_img.dtype, determinism.enabled())
+        # (the deterministic and memory-efficient modes change the launches and buffers: a graph is captured per mode)
+        key = (tuple(lr_img.shape), tuple(hr_img.shape), lr_img.dtype, hr_img.dtype, determinism.enabled(),
+               bool(self.model.memory_efficient))
         if self.use_graph and self._graph is not None and self._graph[0] == key:
             _, graph, s_lr, s_hr, st, flat_grad = self._graph
             s_lr.copy_(lr_img)
