@@ -16,11 +16,17 @@ routine and no Lightning branch.  What it keeps of the reference's configuration
 * [trainer] deterministic (Lightning's ``Trainer(deterministic=...)``; ``--deterministic`` sets it too):
   ``torch.use_deterministic_algorithms(True)`` and a seeded torch generator, so two runs of the same configuration on
   the same GPU give the same weights bit for bit (the gradient all-reduce of multi-GPU runs is outside that promise);
+* [trainer] accumulate_grad_batches (Lightning's ``Trainer`` argument; ``--accumulate-grad-batches`` overrides it;
+  default 1): k micro-batches of ``batch_size`` per optimizer step, their gradients added in place, one all-reduce and
+  one Adam step per window (``TrainStep``).  ``--steps`` counts optimizer steps, each consuming k seeded micro-batches;
+  the printed img/s counts every image and the printed loss is the mean over the window.  As under Lightning, the loss
+  terms are defined per micro-batch (the Poisson term's division by the batch size, MS-SSIM's data range), so this is
+  not one batch of k * batch_size;
 * ``res/configs/loss_functions.toml`` (train.py:45-53) when present: the [loss] percentages and, with
   ``use_scaling = true``, the [scaling.<dataset scaling>] table as ``sc_dict`` of ``create_loss``.  Without the file the
   [loss] table of the run file is used, unscaled (the scaling constants live in that file only).
 
-    python train.py fit run.toml [--synthetic] [--steps N] [--deterministic]
+    python train.py fit run.toml [--synthetic] [--steps N] [--deterministic] [--accumulate-grad-batches K]
     python -m torch.distributed.run --nproc-per-node 8 train.py fit run.toml --synthetic
 """
 from __future__ import annotations
@@ -43,7 +49,7 @@ DEFAULTS = {
     "loss": {"l1": 0.5, "poisson": 0.5, "psnr": 0.0, "ssim": 0.0, "ms_ssim": 0.0, "use_scaling": True},
     "dataset": {"scaling": "sqrt", "lr": {"max": 0.0022336, "res": 416, "exps": [20]},
                 "hr": {"max": 0.0022336, "res": 416, "exp": 50}},
-    "trainer": {"epochs": 1, "deterministic": False},
+    "trainer": {"epochs": 1, "deterministic": False, "accumulate_grad_batches": 1},
 }
 
 DETERMINISTIC_SEED = 0
@@ -100,6 +106,14 @@ def configure_determinism(cfg: dict, flag: bool) -> bool:
     return det
 
 
+def accumulate_grad_batches(cfg: dict, flag) -> int:
+    """--accumulate-grad-batches (when given) or [trainer] accumulate_grad_batches: micro-batches per optimizer step."""
+    k = flag if flag is not None else cfg["trainer"].get("accumulate_grad_batches", 1)
+    if isinstance(k, bool) or not isinstance(k, int) or k < 1:
+        raise ValueError(f"accumulate_grad_batches = {k!r}: expected an integer >= 1")
+    return k
+
+
 def synthetic_batch(kind: str, batch: int, seed: int, cfg: dict, device):
     """Seeded Poisson count images of the reference shape (SURVEY.md 8d), normalised on the GPU."""
     from xmm_superres_denoise_b200 import ops
@@ -117,7 +131,7 @@ def synthetic_batch(kind: str, batch: int, seed: int, cfg: dict, device):
     return x, y
 
 
-def main() -> None:
+def parser() -> argparse.ArgumentParser:
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("routine", choices=["fit"])
     ap.add_argument("config", nargs="?", default=None, help="run TOML (reference layout); defaults are the DeNoise setup")
@@ -125,8 +139,15 @@ def main() -> None:
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--deterministic", action="store_true",
                     help="bit-reproducible training on one GPU ([trainer] deterministic = true does the same)")
-    a = ap.parse_args()
+    ap.add_argument("--accumulate-grad-batches", type=int, default=None, metavar="K",
+                    help="micro-batches per optimizer step (default: [trainer] accumulate_grad_batches, else 1)")
+    return ap
+
+
+def main() -> None:
+    a = parser().parse_args()
     cfg = load_run_config(a.config)
+    k = accumulate_grad_batches(cfg, a.accumulate_grad_batches)
     configure_determinism(cfg, a.deterministic)
 
     import torch.distributed as dist
@@ -153,13 +174,18 @@ def main() -> None:
     model = Model(mcfg, (d["lr"]["res"],) * 2, (d["hr"]["res"],) * 2, loss)
     model.configure_model()
     model = model.to(dev).train()
-    step = TrainStep(model.model, loss, lr=mcfg.optimizer.learning_rate, betas=tuple(mcfg.optimizer.betas))
+    step = TrainStep(model.model, loss, lr=mcfg.optimizer.learning_rate, betas=tuple(mcfg.optimizer.betas),
+                     accumulate_grad_batches=k)
     t0 = time.time()
-    for it in range(a.steps):
-        x, y = synthetic_batch(kind, mcfg.batch_size, 1234 + rank + world * it, cfg, dev)
-        val = step(x, y)
+    for it in range(a.steps):  # optimizer steps; micro-batch m = it * k + j has seed 1234 + rank + world * m
+        vals = []
+        for j in range(k):
+            x, y = synthetic_batch(kind, mcfg.batch_size, 1234 + rank + world * (it * k + j), cfg, dev)
+            vals.append(step(x, y))
         if rank == 0 and (it % 5 == 0 or it == a.steps - 1):
-            print(f"step {it:4d}  train/loss {float(val):.5f}  ({(it + 1) * mcfg.batch_size * world / (time.time() - t0):.1f} img/s)")
+            val = vals[0] if k == 1 else torch.stack(vals).mean()
+            rate = (it + 1) * k * mcfg.batch_size * world / (time.time() - t0)
+            print(f"step {it:4d}  train/loss {float(val):.5f}  ({rate:.1f} img/s)")
     if world > 1:
         dist.destroy_process_group()
 

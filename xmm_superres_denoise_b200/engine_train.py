@@ -74,6 +74,7 @@ class TrainEngine(RRDBEngine):
         self._params = list(gen.parameters())
         self._pindex = {id(p): n for n, p in enumerate(self._params)}
         self._det: Optional[determinism.DetPlan] = None  # the running backward's plan in deterministic mode
+        self._acc = 0  # 1 while a backward adds into its gradient buffer (backward(accumulate=True))
 
     # ------------------------------------------------------------------ buffers
     def _train_buffers(self, b: int, h: int, w: int, device: torch.device, memeff: bool) -> Dict[str, object]:
@@ -137,11 +138,31 @@ class TrainEngine(RRDBEngine):
         return out, bufs
 
     # ------------------------------------------------------------------ backward
-    def _grad_views(self, device: torch.device, extra: int = 0) -> List[torch.Tensor]:
-        """Fresh flat fp32 gradient buffer (autograd may adopt the returned tensors as .grad).  extra: zeroed scratch
-        floats after the gradients (deterministic mode: destinations that are copied into a gradient afterwards)."""
+    def grad_buffer(self, device: torch.device) -> torch.Tensor:
+        """A caller-owned flat gradient buffer for ``backward(grad=...)``: the gradients in parameter order, then the
+        deterministic mode's scratch floats (so one buffer serves both modes)."""
+        return torch.zeros(sum(p.numel() for p in self._params) + self._det_scratch_floats(), dtype=torch.float32,
+                           device=device)
+
+    def _grad_views(self, device: torch.device, extra: int = 0, out: Optional[torch.Tensor] = None,
+                    accumulate: bool = False) -> List[torch.Tensor]:
+        """Flat fp32 gradient buffer and its per-parameter views (autograd may adopt them as .grad): a fresh zeroed one,
+        or ``out`` (from grad_buffer), zeroed unless ``accumulate``.  extra: scratch floats after the gradients
+        (deterministic mode: destinations that are copied into a gradient afterwards), zero in every case."""
         total = sum(p.numel() for p in self._params)
-        flat = torch.zeros(total + extra, dtype=torch.float32, device=device)
+        if out is None:
+            if accumulate:
+                raise RuntimeError("backward(accumulate=True) adds into a caller-owned gradient buffer: pass grad=")
+            flat = torch.zeros(total + extra, dtype=torch.float32, device=device)
+        else:
+            if (out.dtype != torch.float32 or out.device != device or not out.is_contiguous()
+                    or out.numel() != total + self._det_scratch_floats()):
+                raise RuntimeError("backward: grad must be a buffer from grad_buffer() on the input's device")
+            flat = out[:total + extra]
+            if not accumulate:
+                flat.zero_()
+            elif extra:
+                flat[total:].zero_()
         views, off = [], 0
         for p in self._params:
             views.append(flat[off:off + p.numel()].view(p.shape))
@@ -176,6 +197,13 @@ class TrainEngine(RRDBEngine):
     def _gv(self, grads, p: torch.Tensor) -> torch.Tensor:
         return grads[self._pindex[id(p)]]
 
+    def _put(self, dst: torch.Tensor, src: torch.Tensor) -> None:
+        """A gradient computed outside the buffer (a permuted copy): stored, or added on an accumulating backward."""
+        if self._acc:
+            dst.add_(src)
+        else:
+            dst.copy_(src)
+
     def _single_conv_wgrad(self, conv, x: torch.Tensor, dy: torch.Tensor, grads, perm: int = 0) -> None:
         f = self.nf
         n = conv.weight.shape[0]
@@ -187,7 +215,7 @@ class TrainEngine(RRDBEngine):
             for y0 in range(0, n, 128):
                 m = min(128, n - y0)
                 roles.append((0, 3, x0, 1 if m <= 64 else 2, y0, 96, 1))
-                dsts.append((dw, m, f, x0, x0 + 32, len(roles) - 1, 0, 0, 1.0, 0, perm, y0, n))
+                dsts.append((dw, m, f, x0, x0 + 32, len(roles) - 1, 0, 0, 1.0, self._acc, perm, y0, n))
         ops.conv3x3_wgrad(x, dy, roles, dsts)
         if conv.bias is not None:
             db = self._gv(grads, conv.bias)
@@ -195,13 +223,13 @@ class TrainEngine(RRDBEngine):
                 if self._det is None:
                     tmp = torch.empty(n, dtype=torch.float32, device=dy.device)
                     ops.colsum(dy, 0, n, tmp)
-                    db.copy_(tmp.view(4, n // 4).t().reshape(n))  # packed g*F+c -> channel 4c+g
+                    self._put(db, tmp.view(4, n // 4).t().reshape(n))  # packed g*F+c -> channel 4c+g
                 else:
                     tmp = self._scratch(n)
                     self._det.colsum([dy], [(0, n, tmp, 1.0, False)])
-                    self._det.after(lambda: db.copy_(tmp.view(4, n // 4).t().reshape(n)))
+                    self._det.after(lambda: self._put(db, tmp.view(4, n // 4).t().reshape(n)))
             else:
-                self._colsum(dy, [(0, n, db, 1.0, True)])  # db is a view of the zero-initialised flat buffer
+                self._colsum(dy, [(0, n, db, 1.0, True)])  # db is a view of the zeroed (or accumulating) flat buffer
 
     def _block_act(self, bufs, i: int, r: int) -> torch.Tensor:
         """A = [x0|x1|x2|x3|x4] of dense block (i, r): kept from the forward, or (memory-efficient) the scratch buffer
@@ -253,8 +281,8 @@ class TrainEngine(RRDBEngine):
         return (rrdb.RDB1, rrdb.RDB2, rrdb.RDB3)[r]
 
     def _bias_sum(self, grads, conv, scale: float) -> dict:
-        """conv3x3 keywords that make the producing layer accumulate `conv`'s bias gradient (views of the
-        zero-initialised flat gradient buffer)."""
+        """conv3x3 keywords that make the producing layer accumulate `conv`'s bias gradient (views of the flat
+        gradient buffer, which is zero on entry or holds the gradient being accumulated)."""
         if conv.bias is None or not self.fuse_bias:
             return {}
         if self._det is not None:
@@ -274,8 +302,9 @@ class TrainEngine(RRDBEngine):
                     for k, c in enumerate(convs, 1) if c.bias is not None]
             if segs:
                 self._colsum(G, segs)
+        acc = self._acc
         if f == 64:
-            self._rdb_wgrad_64(A, G, dws, s5)
+            self._rdb_wgrad_64(A, G, dws, s5, acc)
             return
         # x0..x3 against all five dY slots, one role per filter row; x4 x dY5 as a stacked role (three dx taps per
         # MMA, operands swapped: lanes = channels of the [dY4|dY5] box)
@@ -284,18 +313,19 @@ class TrainEngine(RRDBEngine):
         for k in range(1, 6):
             sc = s5 if k == 5 else 1.0
             for d in range(3):
-                dsts.append((dws[k - 1], f, k * f, 0, min(k * f, 4 * f), d, 0, (k - 1) * f, sc, 0, 0))
+                dsts.append((dws[k - 1], f, k * f, 0, min(k * f, 4 * f), d, 0, (k - 1) * f, sc, acc, 0))
             if k == 5:
-                dsts.append((dws[k - 1], f, 5 * f, 4 * f, 5 * f, 3, f, 0, sc, 0, 0))
+                dsts.append((dws[k - 1], f, 5 * f, 4 * f, 5 * f, 3, f, 0, sc, acc, 0))
         # (bias gradients: accumulated by the conv launches that produced G's slots -- _rdb_backward / backward)
         ops.conv3x3_wgrad(A, G, roles, dsts)
 
     @staticmethod
-    def _rdb_wgrad_64(A: torch.Tensor, G: torch.Tensor, dws, s5: float) -> None:
+    def _rdb_wgrad_64(A: torch.Tensor, G: torch.Tensor, dws, s5: float, acc: int = 0) -> None:
         """64 filters: X and dY are 320 channels, the needed (x_i, dY_k) blocks (i < k) are 64 x 64.  An M tile is two
         X slots (128 channels), a role keeps taps * N <= 512 accumulator columns -> five launches:
         [x0|x1] x [dY1|dY2], [x0|x1] x [dY3|dY4], [x2|x3] x [dY3|dY4] (one role per filter row, N = 128),
-        [x0|x1] and [x2|x3] x dY5 (N = 64, 5 + 4 taps per role), x4 x dY5 (stacked roles, 32 X channels each)."""
+        [x0|x1] and [x2|x3] x dY5 (N = 64, 5 + 4 taps per role), x4 x dY5 (stacked roles, 32 X channels each).
+        acc: the destinations' accumulate flag (every (x_i, dY_k) block has one destination)."""
         f = 64
         dw1, dw2, dw3, dw4, dw5 = dws
 
@@ -303,49 +333,58 @@ class TrainEngine(RRDBEngine):
             return [(3 * d, 3, x_c0, 2, y_c0, 2 * f) for d in range(3)]
 
         ops.conv3x3_wgrad(A, G, rows(0, 0),
-                          [(dw1, f, f, 0, f, d, 0, 0, 1.0, 0, 0) for d in range(3)] +
-                          [(dw2, f, 2 * f, 0, 2 * f, d, 0, f, 1.0, 0, 0) for d in range(3)])
+                          [(dw1, f, f, 0, f, d, 0, 0, 1.0, acc, 0) for d in range(3)] +
+                          [(dw2, f, 2 * f, 0, 2 * f, d, 0, f, 1.0, acc, 0) for d in range(3)])
         ops.conv3x3_wgrad(A, G, rows(0, 2 * f),
-                          [(dw3, f, 3 * f, 0, 2 * f, d, 0, 0, 1.0, 0, 0) for d in range(3)] +
-                          [(dw4, f, 4 * f, 0, 2 * f, d, 0, f, 1.0, 0, 0) for d in range(3)])
+                          [(dw3, f, 3 * f, 0, 2 * f, d, 0, 0, 1.0, acc, 0) for d in range(3)] +
+                          [(dw4, f, 4 * f, 0, 2 * f, d, 0, f, 1.0, acc, 0) for d in range(3)])
         ops.conv3x3_wgrad(A, G, rows(2 * f, 2 * f),
-                          [(dw3, f, 3 * f, 2 * f, 3 * f, d, 0, 0, 1.0, 0, 0) for d in range(3)] +
-                          [(dw4, f, 4 * f, 2 * f, 4 * f, d, 0, f, 1.0, 0, 0) for d in range(3)])
+                          [(dw3, f, 3 * f, 2 * f, 3 * f, d, 0, 0, 1.0, acc, 0) for d in range(3)] +
+                          [(dw4, f, 4 * f, 2 * f, 4 * f, d, 0, f, 1.0, acc, 0) for d in range(3)])
         roles = [(0, 5, 0, 2, 4 * f, f), (5, 4, 0, 2, 4 * f, f), (0, 5, 2 * f, 2, 4 * f, f), (5, 4, 2 * f, 2, 4 * f, f)]
         ops.conv3x3_wgrad(A, G, roles,
-                          [(dw5, f, 5 * f, 0, 2 * f, q, 0, 0, s5, 0, 0) for q in (0, 1)] +
-                          [(dw5, f, 5 * f, 2 * f, 4 * f, q, 0, 0, s5, 0, 0) for q in (2, 3)])
+                          [(dw5, f, 5 * f, 0, 2 * f, q, 0, 0, s5, acc, 0) for q in (0, 1)] +
+                          [(dw5, f, 5 * f, 2 * f, 4 * f, q, 0, 0, s5, acc, 0) for q in (2, 3)])
         ops.conv3x3_wgrad(A, G, [(0, 3, 4 * f, 1, 4 * f, 96, 1), (0, 3, 4 * f + 32, 1, 4 * f, 96, 1)],
-                          [(dw5, f, 5 * f, 4 * f, 4 * f + 32, 0, 0, 0, s5, 0, 0),
-                           (dw5, f, 5 * f, 4 * f + 32, 5 * f, 1, 0, 0, s5, 0, 0)])
+                          [(dw5, f, 5 * f, 4 * f, 4 * f + 32, 0, 0, 0, s5, acc, 0),
+                           (dw5, f, 5 * f, 4 * f + 32, 5 * f, 1, 0, 0, s5, acc, 0)])
 
     def backward(self, bufs, generation: int, x: torch.Tensor, gout: torch.Tensor, need_x_grad: bool,
-                 rrdb_done_hook=None):
+                 rrdb_done_hook=None, grad: Optional[torch.Tensor] = None, accumulate: bool = False):
+        """Parameter gradients (and dL/dx if need_x_grad) of the last forward_train; returns (dL/dx, gradient views).
+        The gradients go to a fresh zeroed buffer, or to ``grad`` (a buffer from grad_buffer()): overwritten, or with
+        ``accumulate`` added to what it holds -- every site adds in place, so k backward passes into one buffer
+        (gradient accumulation) cost no extra pass and no second buffer."""
         if generation != self.generation:
             raise RuntimeError("backward through a GeneratorRRDB forward whose saved activations were overwritten by a "
                                "later forward (run backward before the next training-mode forward)")
-        if not determinism.enabled():
-            self._det = None
-            return self._backward(bufs, x, gout, need_x_grad, rrdb_done_hook)
-        # deterministic mode: the plan (slot ranges, finalize job tables) lives with this shape's training buffers
-        plan = bufs.get("det")
-        if plan is None:
-            plan = bufs["det"] = determinism.DetPlan(x.device)
-        self._det = plan
+        self._acc = int(bool(accumulate))
         try:
-            return self._backward(bufs, x, gout, need_x_grad, rrdb_done_hook)
-        except BaseException:
-            bufs.pop("det", None)  # slots written without their finalize: start the next deterministic call afresh
-            raise
+            if not determinism.enabled():
+                self._det = None
+                return self._backward(bufs, x, gout, need_x_grad, rrdb_done_hook, grad)
+            # deterministic mode: the plan (slot ranges, finalize job tables) lives with this shape's training buffers
+            plan = bufs.get("det")
+            if plan is None:
+                plan = bufs["det"] = determinism.DetPlan(x.device)
+            self._det = plan
+            try:
+                return self._backward(bufs, x, gout, need_x_grad, rrdb_done_hook, grad)
+            except BaseException:
+                bufs.pop("det", None)  # slots written without their finalize: start the next deterministic call afresh
+                raise
+            finally:
+                self._det = None
         finally:
-            self._det = None
+            self._acc = 0
 
-    def _backward(self, bufs, x: torch.Tensor, gout: torch.Tensor, need_x_grad: bool, rrdb_done_hook):
+    def _backward(self, bufs, x: torch.Tensor, gout: torch.Tensor, need_x_grad: bool, rrdb_done_hook,
+                  grad: Optional[torch.Tensor] = None):
         g, f, kc, a = self.gen, self.nf, self.kc, self.arena
         det = self._det
         gout = gout.contiguous().float()
         x = x.contiguous().float()
-        grads = self._grad_views(x.device, self._det_scratch_floats() if det is not None else 0)
+        grads = self._grad_views(x.device, self._det_scratch_floats() if det is not None else 0, grad, bool(self._acc))
         if det is not None:
             det.begin(self._flat_ext)
             self._det_bhw = tuple(bufs["trunk"].shape[:3])
@@ -400,17 +439,19 @@ class TrainEngine(RRDBEngine):
         if det is None:
             r_first = torch.zeros(cin, f, 9, dtype=torch.float32, device=x.device)
             ops.edge_wgrad(x, d_fea, 0, f, r_first, v2=d_trunk, v2_coff=0)
-            dwf.copy_(r_first.flip(2).permute(1, 0, 2).reshape(f, cin, 3, 3))
+            self._put(dwf, r_first.flip(2).permute(1, 0, 2).reshape(f, cin, 3, 3))
             if g.conv_first.bias is not None:
                 dbf = self._gv(grads, g.conv_first.bias)
-                ops.colsum(d_fea, 0, f, dbf)
+                ops.colsum(d_fea, 0, f, dbf, accumulate=bool(self._acc))
                 ops.colsum(d_trunk, 0, f, dbf, accumulate=True)
         else:
             r_first = self._scratch(cin * f * 9).view(cin, f, 9)
             det.edge_wgrad(x, d_fea, 0, f, r_first, v2=d_trunk, v2_coff=0)
-            det.after(lambda: dwf.copy_(r_first.flip(2).permute(1, 0, 2).reshape(f, cin, 3, 3)))
+            det.after(lambda: self._put(dwf, r_first.flip(2).permute(1, 0, 2).reshape(f, cin, 3, 3)))
             if g.conv_first.bias is not None:  # both integrands in one job: d_fea's slots, then d_trunk's
-                det.colsum([d_fea, d_trunk], [(0, f, self._gv(grads, g.conv_first.bias), 1.0, False)])
+                # an adding job: the destination is zero unless the backward accumulates, and a window's micro-batches
+                # then share the finalize job tables
+                det.colsum([d_fea, d_trunk], [(0, f, self._gv(grads, g.conv_first.bias), 1.0, True)])
             det.flush()
         gx = None
         if need_x_grad:

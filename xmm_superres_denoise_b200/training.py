@@ -103,17 +103,34 @@ class FusedAdam:
 
 
 class TrainStep:
-    """forward + loss + backward + gradient all-reduce + Adam for one (lr, hr) batch."""
+    """forward + loss + backward + gradient all-reduce + Adam for one (lr, hr) batch -- or, with
+    ``accumulate_grad_batches = k``, for one micro-batch of a window of k.
+
+    Gradient accumulation follows Lightning's ``Trainer(accumulate_grad_batches=k)``: every call runs forward + loss +
+    backward of its micro-batch and returns that micro-batch's loss (unscaled, merged into the loss state as ever); the
+    loss gradient is seeded with 1/k (Lightning's ``loss / accumulate_grad_batches``) and the backward adds into one
+    flat gradient buffer.  Calls k, 2k, ... close the window: the gradient all-reduce (overlapped with that call's
+    backward) and one Adam step.  Other calls run no collective and no optimizer step; ``pending`` counts the
+    micro-batches since the last optimizer step, and an open window simply continues on the next call.  Per-micro-batch
+    definitions stay per micro-batch, as under Lightning: the Poisson term's division by the batch size and MS-SSIM's
+    data range are those of each micro-batch, so a window of k batches of B is not one batch of k * B."""
 
     def __init__(self, model: nn.Module, loss, lr: float = 1e-4, betas=(0.9, 0.999), group=None,
-                 overlap_allreduce: bool = True, use_graph: Optional[bool] = None) -> None:
+                 overlap_allreduce: bool = True, use_graph: Optional[bool] = None,
+                 accumulate_grad_batches: int = 1) -> None:
         """use_graph: replay forward + loss + backward (~800 launches, ~95 % GPU-busy when launched through Python) as
-        ONE CUDA graph per input shape; Adam and the running loss state stay outside.  Off by default
+        ONE CUDA graph per input shape (two with accumulate_grad_batches > 1: a window's first micro-batch and the later
+        ones differ in their launches); Adam and the running loss state stay outside.  Off by default
         (XMM_TRAIN_GRAPH=1 enables): measured on B200 the eager step is already GPU-bound (362 vs 363 img/s, DN
         training, profiles/r01_bench_train_graph_ab.log); it pays with a slow host.  Single-process runs only: with a
         process group the NCCL chunks are issued eagerly."""
         import torch.distributed as dist
 
+        k = accumulate_grad_batches
+        if isinstance(k, bool) or not isinstance(k, int) or k < 1:
+            raise ValueError(f"accumulate_grad_batches={k!r}: expected an integer >= 1")
+        self.accumulate_grad_batches = k
+        self.pending = 0  # micro-batches since the last optimizer step
         self.model, self.loss, self.group = model, loss, group
         self.world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
         self.flat = flatten_parameters(model)
@@ -141,14 +158,18 @@ class TrainStep:
         # 2622..2635 img/s (SR training) -- the 4 % the step loses at 8 GPUs is not SM contention -- so it stays off.
         self.sm_reserve = int(os.environ.get("XMM_COMM_SM_RESERVE", "0")) if self.overlap else 0
         self._works: List = []
-        self._ones = torch.ones(1, dtype=torch.float32, device=self.flat.device)
+        # seed of the loss gradient: 1/k, the scaling of an accumulated micro-batch at no extra pass
+        self._seed = torch.full((1,), 1.0 / k, dtype=torch.float32, device=self.flat.device)
+        # k > 1: the buffer a window's micro-batches add into (one for every input shape: the gradient's size does not
+        # depend on it); k = 1 keeps the engine's fresh buffer per step
+        self._grad = self.engine.grad_buffer(self.flat.device) if k > 1 else None
         # chunk boundaries of the flat buffer: one chunk per RRDB (parameters are registered in module order)
         self._chunks = self._rrdb_chunks()
         if use_graph is None:
             use_graph = os.environ.get("XMM_TRAIN_GRAPH", "0") == "1"
         self.use_graph = bool(use_graph) and self.world == 1
-        self._graph = None      # (key, CUDAGraph, static lr, static hr, loss state, flat gradient)
-        self._seen_key = None   # shapes of the last eager step (the capture follows one eager step of that shape)
+        self._graph = None  # {key: (CUDAGraph, static lr, static hr, loss state, flat gradient)}, one shape / mode
+        self._seen = set()  # keys of that shape / mode stepped eagerly (a capture follows one eager step of its key)
 
     def _rrdb_chunks(self):
         offs, off = {}, 0
@@ -176,13 +197,15 @@ class TrainStep:
         else:
             dist.all_reduce(flat_grad[lo:hi], op=dist.ReduceOp.SUM, group=self.group)
 
-    def _fwd_bwd(self, lr_img: torch.Tensor, hr_img: torch.Tensor):
-        """forward + loss + backward (+ the gradient all-reduce chunks); returns (loss state, flat gradient)."""
+    def _fwd_bwd(self, lr_img: torch.Tensor, hr_img: torch.Tensor, accumulate: bool = False,
+                 exchange: bool = True):
+        """forward + loss + backward (+ the gradient all-reduce chunks when ``exchange``: the call that closes a
+        window); ``accumulate``: add to the window's gradient instead of starting it.  Returns (loss state, gradient)."""
         eng = self.engine
         out, bufs = eng.forward_train(lr_img)
         # Model.forward's second clamp (models/model.py:49) is the identity on an output already in [0,1]
         st = self.loss._evaluate(out, hr_img.contiguous().float())
-        gout = self.loss._gradient(out, hr_img.contiguous().float(), st, self._ones)
+        gout = self.loss._gradient(out, hr_img.contiguous().float(), st, self._seed)
         done = [len(self.flat)]  # upper end of the not-yet-reduced tail of the flat buffer
 
         def hook(rrdb_index: int, flat_grad: torch.Tensor) -> None:
@@ -191,9 +214,11 @@ class TrainStep:
             done[0] = lo
 
         _, _ = eng.backward(bufs, eng.generation, lr_img, gout, need_x_grad=False,
-                            rrdb_done_hook=hook if self.overlap else None)
+                            rrdb_done_hook=hook if self.overlap and exchange else None, grad=self._grad,
+                            accumulate=accumulate)
         flat_grad = eng.last_flat_grad
-        self._allreduce_range(flat_grad, 0, done[0])
+        if exchange:
+            self._allreduce_range(flat_grad, 0, done[0])
         for w in self._works:
             w.wait()
         if self._works and self.sm_reserve > 0:
@@ -202,26 +227,35 @@ class TrainStep:
         return st, flat_grad
 
     def __call__(self, lr_img: torch.Tensor, hr_img: torch.Tensor) -> torch.Tensor:
-        # (the deterministic and memory-efficient modes change the launches and buffers: a graph is captured per mode)
+        accumulate = self.pending > 0
+        closing = self.pending + 1 == self.accumulate_grad_batches
+        # (the deterministic and memory-efficient modes change the launches and buffers: a graph is captured per mode;
+        # so does the window position: a window's first micro-batch writes the gradient, the later ones add to it)
         key = (tuple(lr_img.shape), tuple(hr_img.shape), lr_img.dtype, hr_img.dtype, determinism.enabled(),
-               bool(self.model.memory_efficient))
-        if self.use_graph and self._graph is not None and self._graph[0] == key:
-            _, graph, s_lr, s_hr, st, flat_grad = self._graph
+               bool(self.model.memory_efficient), accumulate)
+        if self._seen and next(iter(self._seen))[:-1] != key[:-1]:
+            # another shape or mode: the engine releases the buffers the graphs of the last one write
+            self._graph, self._seen = None, set()
+        if self.use_graph and self._graph is not None and key in self._graph:
+            graph, s_lr, s_hr, st, flat_grad = self._graph[key]
             s_lr.copy_(lr_img)
             s_hr.copy_(hr_img)
             graph.replay()
-        elif self.use_graph and self._seen_key == key and not torch.cuda.is_current_stream_capturing():
-            # second step of this shape: every lazily created buffer / tensor map / function attribute exists now
+        elif self.use_graph and key in self._seen and not torch.cuda.is_current_stream_capturing():
+            # second step of this key: every lazily created buffer / tensor map / function attribute exists now
             s_lr, s_hr = lr_img.clone(), hr_img.clone()
             gc.collect()  # nothing may release device memory in mid-capture
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                st, flat_grad = self._fwd_bwd(s_lr, s_hr)
-            self._graph = (key, graph, s_lr, s_hr, st, flat_grad)
+                st, flat_grad = self._fwd_bwd(s_lr, s_hr, accumulate, closing)
+            self._graph = {**(self._graph or {}), key: (graph, s_lr, s_hr, st, flat_grad)}
             graph.replay()
         else:
-            self._seen_key = key
-            st, flat_grad = self._fwd_bwd(lr_img, hr_img)
+            self._seen.add(key)
+            st, flat_grad = self._fwd_bwd(lr_img, hr_img, accumulate, closing)
         self.loss._merge(st)
-        self.opt.step(flat_grad, 1.0 / self.world)
+        self.pending += 1
+        if closing:
+            self.opt.step(flat_grad, 1.0 / self.world)
+            self.pending = 0
         return st["total"]
