@@ -455,6 +455,24 @@ int xmm_msssim_finalize(const xmm_msssim_finalize_params* p, void* stream);
 int xmm_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, size_t n, float lr,
                   float beta1, float beta2, float eps, int step, float grad_scale, void* stream);
 
+/* Gradient clipping (Lightning's Trainer(gradient_clip_val, gradient_clip_algorithm), applied once per optimizer step
+ * to the averaged gradient g = grads * grad_scale).
+ * xmm_grad_clip_coef: out[0] = ||g||_2 (squares added in fp64, rounded once to fp32), out[1] = the coefficient of
+ * torch.nn.utils.clip_grad_norm_(max_norm=max_norm), in fp32 as torch computes it: min(max_norm / (out[0] + 1e-6), 1)
+ * (an inf norm gives 0, a NaN norm NaN).  Two launches, no host synchronisation; the order of every addition depends
+ * on n only, so the result is the same bits on every run.  grads 16-byte aligned; grad_scale > 0; max_norm >= 0;
+ * workspace: xmm_grad_norm_workspace_bytes(n) bytes (per-CTA partial sums, overwritten).                          */
+size_t xmm_grad_norm_workspace_bytes(size_t n);
+int xmm_grad_clip_coef(const float* grads, size_t n, float grad_scale, float max_norm, float* out, void* workspace,
+                       size_t workspace_bytes, void* stream);
+/* xmm_adam_step on a clipped gradient: Adam sees grads * (grad_scale * clip_coef[0]) when clip_coef (a device float,
+ * e.g. out + 1 of xmm_grad_clip_coef) is given -- clip by norm -- or clamp(grads * grad_scale, -clip_value,
+ * clip_value) when clip_value > 0 -- clip by value, torch.nn.utils.clip_grad_value_.  Exactly one of the two.  With
+ * clip_coef[0] == 1 and grad_scale == 1 the step is xmm_adam_step's, bit for bit.                                 */
+int xmm_adam_step_clip(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, size_t n, float lr,
+                       float beta1, float beta2, float eps, int step, float grad_scale, const float* clip_coef,
+                       float clip_value, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -22,11 +22,16 @@ routine and no Lightning branch.  What it keeps of the reference's configuration
   the printed img/s counts every image and the printed loss is the mean over the window.  As under Lightning, the loss
   terms are defined per micro-batch (the Poisson term's division by the batch size, MS-SSIM's data range), so this is
   not one batch of k * batch_size;
+* [trainer] gradient_clip_val and gradient_clip_algorithm (Lightning's ``Trainer`` arguments;
+  ``--gradient-clip-val`` / ``--gradient-clip-algorithm`` override them; default: no clipping, algorithm "norm"): the
+  averaged gradient of every optimizer step is clipped by its global L2 norm (``clip_grad_norm_``) or by value
+  (``clip_grad_value_``) before Adam; 0 turns clipping off.  With "norm" the printed lines add the pre-clip norm;
 * ``res/configs/loss_functions.toml`` (train.py:45-53) when present: the [loss] percentages and, with
   ``use_scaling = true``, the [scaling.<dataset scaling>] table as ``sc_dict`` of ``create_loss``.  Without the file the
   [loss] table of the run file is used, unscaled (the scaling constants live in that file only).
 
     python train.py fit run.toml [--synthetic] [--steps N] [--deterministic] [--accumulate-grad-batches K]
+                                 [--gradient-clip-val V] [--gradient-clip-algorithm {norm,value}]
     python -m torch.distributed.run --nproc-per-node 8 train.py fit run.toml --synthetic
 """
 from __future__ import annotations
@@ -49,7 +54,8 @@ DEFAULTS = {
     "loss": {"l1": 0.5, "poisson": 0.5, "psnr": 0.0, "ssim": 0.0, "ms_ssim": 0.0, "use_scaling": True},
     "dataset": {"scaling": "sqrt", "lr": {"max": 0.0022336, "res": 416, "exps": [20]},
                 "hr": {"max": 0.0022336, "res": 416, "exp": 50}},
-    "trainer": {"epochs": 1, "deterministic": False, "accumulate_grad_batches": 1},
+    "trainer": {"epochs": 1, "deterministic": False, "accumulate_grad_batches": 1, "gradient_clip_val": None,
+                "gradient_clip_algorithm": "norm"},
 }
 
 DETERMINISTIC_SEED = 0
@@ -114,6 +120,17 @@ def accumulate_grad_batches(cfg: dict, flag) -> int:
     return k
 
 
+def gradient_clip(cfg: dict, val_flag, algorithm_flag):
+    """--gradient-clip-val / --gradient-clip-algorithm (when given) or [trainer] gradient_clip_val /
+    gradient_clip_algorithm, checked as TrainStep checks them: (max value or None when off, algorithm)."""
+    from xmm_superres_denoise_b200.training import gradient_clip_settings
+
+    t = cfg["trainer"]
+    val = val_flag if val_flag is not None else t.get("gradient_clip_val")
+    algorithm = algorithm_flag if algorithm_flag is not None else t.get("gradient_clip_algorithm", "norm")
+    return gradient_clip_settings(val, algorithm)
+
+
 def synthetic_batch(kind: str, batch: int, seed: int, cfg: dict, device):
     """Seeded Poisson count images of the reference shape (SURVEY.md 8d), normalised on the GPU."""
     from xmm_superres_denoise_b200 import ops
@@ -141,6 +158,11 @@ def parser() -> argparse.ArgumentParser:
                     help="bit-reproducible training on one GPU ([trainer] deterministic = true does the same)")
     ap.add_argument("--accumulate-grad-batches", type=int, default=None, metavar="K",
                     help="micro-batches per optimizer step (default: [trainer] accumulate_grad_batches, else 1)")
+    ap.add_argument("--gradient-clip-val", type=float, default=None, metavar="V",
+                    help="clip each optimizer step's averaged gradient at V (0: off; default: [trainer] "
+                         "gradient_clip_val, else off)")
+    ap.add_argument("--gradient-clip-algorithm", default=None, metavar="{norm,value}",
+                    help="clip by global L2 norm (default) or by value (default: [trainer] gradient_clip_algorithm)")
     return ap
 
 
@@ -148,6 +170,7 @@ def main() -> None:
     a = parser().parse_args()
     cfg = load_run_config(a.config)
     k = accumulate_grad_batches(cfg, a.accumulate_grad_batches)
+    clip_val, clip_algorithm = gradient_clip(cfg, a.gradient_clip_val, a.gradient_clip_algorithm)
     configure_determinism(cfg, a.deterministic)
 
     import torch.distributed as dist
@@ -175,7 +198,7 @@ def main() -> None:
     model.configure_model()
     model = model.to(dev).train()
     step = TrainStep(model.model, loss, lr=mcfg.optimizer.learning_rate, betas=tuple(mcfg.optimizer.betas),
-                     accumulate_grad_batches=k)
+                     accumulate_grad_batches=k, gradient_clip_val=clip_val, gradient_clip_algorithm=clip_algorithm)
     t0 = time.time()
     for it in range(a.steps):  # optimizer steps; micro-batch m = it * k + j has seed 1234 + rank + world * m
         vals = []
@@ -185,7 +208,8 @@ def main() -> None:
         if rank == 0 and (it % 5 == 0 or it == a.steps - 1):
             val = vals[0] if k == 1 else torch.stack(vals).mean()
             rate = (it + 1) * k * mcfg.batch_size * world / (time.time() - t0)
-            print(f"step {it:4d}  train/loss {float(val):.5f}  ({rate:.1f} img/s)")
+            norm = "" if step.grad_norm is None else f"  grad_norm {float(step.grad_norm):.5g}"
+            print(f"step {it:4d}  train/loss {float(val):.5f}{norm}  ({rate:.1f} img/s)")
     if world > 1:
         dist.destroy_process_group()
 

@@ -178,6 +178,10 @@ SIGNATURES = {
     "xmm_msssim_finalize": (c_int, [POINTER(MsssimFinalizeParams), c_void_p]),
     "xmm_adam_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_float, c_float, c_float, c_float,
                               c_int, c_float, c_void_p]),
+    "xmm_grad_norm_workspace_bytes": (c_size_t, [c_size_t]),
+    "xmm_grad_clip_coef": (c_int, [c_void_p, c_size_t, c_float, c_float, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "xmm_adam_step_clip": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_float, c_float, c_float,
+                                   c_float, c_int, c_float, c_void_p, c_float, c_void_p]),
 }
 
 _lib = None

@@ -224,6 +224,50 @@ void adam_step(Tensor params, const Tensor& grads, Tensor exp_avg, Tensor exp_av
            "adam_step");
 }
 
+// torch.nn.utils.clip_grad_norm_(max_norm) without the multiply: out = {||grads * grad_scale||_2, min(max_norm /
+// (norm + 1e-6), 1)} (fp32, on the device); workspace: any contiguous CUDA tensor of
+// xmm_grad_norm_workspace_bytes(grads.numel()) bytes or more.
+void grad_clip_coef(const Tensor& grads, double grad_scale, double max_norm, Tensor out, Tensor workspace) {
+  need(grads, at::kFloat, "grad_clip_coef grads");
+  need(out, at::kFloat, "grad_clip_coef out");
+  TORCH_CHECK(workspace.is_cuda() && workspace.is_contiguous(), "grad_clip_coef workspace: expected a contiguous CUDA tensor");
+  TORCH_CHECK(out.numel() >= 2, "grad_clip_coef: out holds {norm, coef}");
+  TORCH_CHECK(out.device() == grads.device() && workspace.device() == grads.device(),
+              "grad_clip_coef: tensors live on different devices");
+  c10::cuda::CUDAGuard guard(grads.device());
+  check_rc(xmm_grad_clip_coef(grads.data_ptr<float>(), size_t(grads.numel()), float(grad_scale), float(max_norm),
+                              out.data_ptr<float>(), workspace.data_ptr(), size_t(workspace.nbytes()), stream_of(grads)),
+           "grad_clip_coef");
+}
+
+// adam_step on a clipped gradient: grads * (grad_scale * clip_coef[0]) (clip_coef: one float on the device, e.g.
+// out[1:] of grad_clip_coef) or clamp(grads * grad_scale, -clip_value, clip_value) (clip_value > 0); exactly one.
+void adam_step_clip(Tensor params, const Tensor& grads, Tensor exp_avg, Tensor exp_avg_sq, double lr, double beta1,
+                    double beta2, double eps, int64_t step, double grad_scale, const OptTensor& clip_coef,
+                    double clip_value) {
+  need(params, at::kFloat, "adam_step_clip params");
+  need(grads, at::kFloat, "adam_step_clip grads");
+  need(exp_avg, at::kFloat, "adam_step_clip exp_avg");
+  need(exp_avg_sq, at::kFloat, "adam_step_clip exp_avg_sq");
+  const int64_t n = params.numel();
+  TORCH_CHECK(grads.numel() == n && exp_avg.numel() == n && exp_avg_sq.numel() == n,
+              "adam_step_clip: buffer sizes differ");
+  TORCH_CHECK(grads.device() == params.device() && exp_avg.device() == params.device() &&
+                  exp_avg_sq.device() == params.device(), "adam_step_clip: tensors live on different devices");
+  same_device(params, clip_coef, "adam_step_clip clip_coef");
+  const float* coef = nullptr;
+  if (clip_coef.has_value()) {
+    need(*clip_coef, at::kFloat, "adam_step_clip clip_coef");
+    TORCH_CHECK(clip_coef->numel() >= 1, "adam_step_clip: clip_coef is empty");
+    coef = clip_coef->data_ptr<float>();
+  }
+  c10::cuda::CUDAGuard guard(params.device());
+  check_rc(xmm_adam_step_clip(params.data_ptr<float>(), grads.data_ptr<float>(), exp_avg.data_ptr<float>(),
+                              exp_avg_sq.data_ptr<float>(), size_t(n), float(lr), float(beta1), float(beta2),
+                              float(eps), int(step), float(grad_scale), coef, float(clip_value), stream_of(params)),
+           "adam_step_clip");
+}
+
 int64_t abi_version() { return xmm_version(); }
 
 }  // namespace
@@ -239,6 +283,10 @@ TORCH_LIBRARY(xmm_b200, m) {
   m.def("image_upsample(Tensor inp, Tensor(a!) out, int scale) -> ()");
   m.def("adam_step(Tensor(a!) params, Tensor grads, Tensor(b!) exp_avg, Tensor(c!) exp_avg_sq, float lr, float beta1, "
         "float beta2, float eps, int step, float grad_scale=1.0) -> ()");
+  m.def("grad_clip_coef(Tensor grads, float grad_scale, float max_norm, Tensor(a!) out, Tensor(b!) workspace) -> ()");
+  m.def("adam_step_clip(Tensor(a!) params, Tensor grads, Tensor(b!) exp_avg, Tensor(c!) exp_avg_sq, float lr, "
+        "float beta1, float beta2, float eps, int step, float grad_scale=1.0, Tensor? clip_coef=None, "
+        "float clip_value=0.0) -> ()");
   m.def("abi_version() -> int", &abi_version);
 }
 
@@ -249,4 +297,6 @@ TORCH_LIBRARY_IMPL(xmm_b200, CUDA, m) {
   m.impl("denormalize", &denormalize);
   m.impl("image_upsample", &image_upsample);
   m.impl("adam_step", &adam_step);
+  m.impl("grad_clip_coef", &grad_clip_coef);
+  m.impl("adam_step_clip", &adam_step_clip);
 }

@@ -10,6 +10,7 @@
 #include "conv3x3_rdb.cuh"
 #include "conv3x3_tc.cuh"
 #include "edge_kernels.cuh"
+#include "grad_clip.cuh"
 #include "host_common.cuh"
 #include "loss_kernels.cuh"
 #include "pack_weights.cuh"
@@ -22,7 +23,7 @@
 using namespace xmm;
 
 extern "C" const char* xmm_last_error(void) { return last_error_ref().c_str(); }
-extern "C" int xmm_version(void) { return 101; }
+extern "C" int xmm_version(void) { return 102; }
 extern "C" int xmm_check_device(void) {
   DeviceInfo d;
   return require_sm100(&d);
@@ -1625,6 +1626,51 @@ extern "C" int xmm_adam_step(float* params, const float* grads, float* exp_avg, 
   const double bc2 = 1.0 - pow(double(beta2), double(step));
   adam_kernel<<<unsigned((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       params, grads, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, float(bc1), float(sqrt(bc2)), grad_scale);
+  XMM_CUDA_OK(cudaGetLastError());
+  return XMM_OK;
+}
+
+// ----------------------------------------------------------------------------- gradient clipping
+extern "C" size_t xmm_grad_norm_workspace_bytes(size_t n) { return grad_norm_blocks(n) * sizeof(double); }
+
+extern "C" int xmm_grad_clip_coef(const float* grads, size_t n, float grad_scale, float max_norm, float* out,
+                                  void* workspace, size_t workspace_bytes, void* stream) {
+  DeviceInfo dev;
+  int rc = require_sm100(&dev);
+  if (rc != XMM_OK) return rc;
+  XMM_REQUIRE(out && (grads || n == 0), "grad_clip_coef: null pointer");
+  XMM_REQUIRE((reinterpret_cast<uintptr_t>(grads) & 15) == 0, "grad_clip_coef: gradients must be 16-byte aligned");
+  XMM_REQUIRE(grad_scale > 0.0f && max_norm >= 0.0f, "grad_clip_coef: grad_scale %g must be > 0, max_norm %g >= 0",
+              double(grad_scale), double(max_norm));
+  const size_t blocks = grad_norm_blocks(n);
+  XMM_REQUIRE(blocks <= 0x7fffffffu, "grad_clip_coef: n = %zu too large", n);
+  XMM_REQUIRE(blocks == 0 || (workspace && workspace_bytes >= blocks * sizeof(double)),
+              "grad_clip_coef: workspace of %zu bytes, %zu needed (xmm_grad_norm_workspace_bytes)", workspace_bytes,
+              blocks * sizeof(double));
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  double* partials = static_cast<double*>(workspace);
+  if (blocks > 0) grad_norm_partial_kernel<<<unsigned(blocks), kNormThreads, 0, st>>>(grads, n, partials);
+  grad_norm_finalize_kernel<<<1, kNormThreads, 0, st>>>(partials, blocks, grad_scale, max_norm, out);
+  XMM_CUDA_OK(cudaGetLastError());
+  return XMM_OK;
+}
+
+extern "C" int xmm_adam_step_clip(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, size_t n,
+                                  float lr, float beta1, float beta2, float eps, int step, float grad_scale,
+                                  const float* clip_coef, float clip_value, void* stream) {
+  DeviceInfo dev;
+  int rc = require_sm100(&dev);
+  if (rc != XMM_OK) return rc;
+  XMM_REQUIRE(params && grads && exp_avg && exp_avg_sq, "adam_clip: null pointer");
+  XMM_REQUIRE(step >= 1, "adam_clip: step count starts at 1 (got %d)", step);
+  XMM_REQUIRE((clip_coef != nullptr) != (clip_value > 0.0f),
+              "adam_clip: give exactly one of clip_coef and clip_value > 0 (clip_value %g)", double(clip_value));
+  if (n == 0) return XMM_OK;
+  const double bc1 = 1.0 - pow(double(beta1), double(step));
+  const double bc2 = 1.0 - pow(double(beta2), double(step));
+  adam_clip_kernel<<<unsigned((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      params, grads, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, float(bc1), float(sqrt(bc2)), grad_scale, clip_coef,
+      clip_value);
   XMM_CUDA_OK(cudaGetLastError());
   return XMM_OK;
 }

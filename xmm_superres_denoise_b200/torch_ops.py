@@ -6,6 +6,7 @@
 
     torch.ops.xmm_b200.conv3x3_fwd(inp, in_coff, cin, wblob, kc, cout, out, out_coff, lrelu=0.2, wblob_row=...)
     torch.ops.xmm_b200.conv3x3_dgrad / normalize / denormalize / image_upsample / adam_step / abi_version
+    torch.ops.xmm_b200.grad_clip_coef / adam_step_clip  (gradient clipping, training.FusedAdam)
 
 are ordinary dispatcher ops (mutating their ``out`` argument, returning nothing).  The engine itself keeps calling
 the launchers through ctypes (``_lib.py``): both faces end in the same C entry point, and the engine's calls are

@@ -15,6 +15,7 @@ gradients.
 from __future__ import annotations
 
 import gc
+import math
 import os
 from typing import List, Optional, Tuple
 
@@ -62,6 +63,40 @@ def allreduce_mean_(flat: torch.Tensor, group=None) -> torch.Tensor:
     return flat
 
 
+def gradient_clip_settings(gradient_clip_val=None, gradient_clip_algorithm: Optional[str] = "norm"):
+    """Lightning's ``Trainer(gradient_clip_val, gradient_clip_algorithm)``, checked: returns ``(max value, algorithm)``,
+    the value None when clipping is off (None or 0).  The algorithm is "norm" (``clip_grad_norm_``, also for None) or
+    "value" (``clip_grad_value_``); a negative or NaN value, or another algorithm, raises ValueError."""
+    algorithm = "norm" if gradient_clip_algorithm is None else gradient_clip_algorithm
+    if algorithm not in ("norm", "value"):
+        raise ValueError(f"gradient_clip_algorithm={gradient_clip_algorithm!r}: expected 'norm' or 'value'")
+    val = gradient_clip_val
+    if val is None:
+        return None, algorithm
+    if isinstance(val, bool) or not isinstance(val, (int, float)) or math.isnan(val) or val < 0:
+        raise ValueError(f"gradient_clip_val={val!r}: expected a number >= 0 (0 or None: no clipping)")
+    return (float(val) if val > 0 else None), algorithm
+
+
+def grad_clip_coef(flat_grads: torch.Tensor, grad_scale: float, max_norm: float, out: torch.Tensor,
+                   workspace: torch.Tensor) -> None:
+    """out[0] = ||flat_grads * grad_scale||_2, out[1] = ``clip_grad_norm_``'s coefficient min(max_norm / (out[0] + 1e-6),
+    1), both fp32 on the device (no host synchronisation); workspace: ``grad_norm_workspace(n)`` bytes or more."""
+    _lib.require_cuda_tensor(flat_grads, torch.float32, "grad_clip_coef gradients")
+    _lib.require_cuda_tensor(out, torch.float32, "grad_clip_coef out")
+    if out.numel() < 2:
+        raise RuntimeError("grad_clip_coef: out holds {norm, coef}")
+    _lib.check(_lib.load().xmm_grad_clip_coef(flat_grads.data_ptr(), flat_grads.numel(), grad_scale, max_norm,
+                                              out.data_ptr(), workspace.data_ptr(), workspace.nbytes,
+                                              _lib.stream_ptr()))
+    ops._count(2)
+
+
+def grad_norm_workspace(n: int, device) -> torch.Tensor:
+    """The partial-sum workspace of ``grad_clip_coef`` for n gradients."""
+    return torch.empty(max(int(_lib.load().xmm_grad_norm_workspace_bytes(n)), 1), dtype=torch.uint8, device=device)
+
+
 class FusedAdam:
     """torch.optim.Adam semantics on a flat parameter buffer (one kernel per step)."""
 
@@ -77,14 +112,32 @@ class FusedAdam:
         # copies of these parameters (engine.WeightArena) must be told explicitly
         self.on_update = on_update
 
-    def step(self, flat_grads: torch.Tensor, grad_scale: float = 1.0) -> None:
+    def step(self, flat_grads: torch.Tensor, grad_scale: float = 1.0, clip_coef: Optional[torch.Tensor] = None,
+             clip_value: Optional[float] = None) -> None:
+        """One Adam step on ``flat_grads * grad_scale``.  Clipped (at most one of the two): ``clip_coef``, a one-element
+        fp32 device tensor (``grad_clip_coef``'s out[1:]), multiplies the gradient -- clip by norm; ``clip_value`` > 0
+        clamps it to [-clip_value, clip_value] -- clip by value."""
         _lib.require_cuda_tensor(flat_grads, torch.float32, "FusedAdam gradients")
         if flat_grads.numel() != self.params.numel():
             raise RuntimeError("gradient buffer size does not match the parameter buffer")
+        if clip_coef is not None:
+            _lib.require_cuda_tensor(clip_coef, torch.float32, "FusedAdam clip_coef")
+        if clip_coef is not None and clip_value is not None:
+            raise ValueError("FusedAdam.step: clip by norm (clip_coef) or by value (clip_value), not both")
+        if clip_value is not None and not clip_value > 0:
+            raise ValueError(f"FusedAdam.step: clip_value={clip_value!r} must be > 0")
         self.step_count += 1
-        _lib.check(_lib.load().xmm_adam_step(self.params.data_ptr(), flat_grads.data_ptr(), self.exp_avg.data_ptr(),
-                                             self.exp_avg_sq.data_ptr(), self.params.numel(), self.lr, self.betas[0],
-                                             self.betas[1], self.eps, self.step_count, grad_scale, _lib.stream_ptr()))
+        lib = _lib.load()
+        if clip_coef is None and clip_value is None:
+            _lib.check(lib.xmm_adam_step(self.params.data_ptr(), flat_grads.data_ptr(), self.exp_avg.data_ptr(),
+                                         self.exp_avg_sq.data_ptr(), self.params.numel(), self.lr, self.betas[0],
+                                         self.betas[1], self.eps, self.step_count, grad_scale, _lib.stream_ptr()))
+        else:
+            _lib.check(lib.xmm_adam_step_clip(self.params.data_ptr(), flat_grads.data_ptr(), self.exp_avg.data_ptr(),
+                                              self.exp_avg_sq.data_ptr(), self.params.numel(), self.lr, self.betas[0],
+                                              self.betas[1], self.eps, self.step_count, grad_scale,
+                                              None if clip_coef is None else clip_coef.data_ptr(),
+                                              0.0 if clip_value is None else float(clip_value), _lib.stream_ptr()))
         ops._count()
         if self.on_update is not None:
             self.on_update()
@@ -113,11 +166,19 @@ class TrainStep:
     backward) and one Adam step.  Other calls run no collective and no optimizer step; ``pending`` counts the
     micro-batches since the last optimizer step, and an open window simply continues on the next call.  Per-micro-batch
     definitions stay per micro-batch, as under Lightning: the Poisson term's division by the batch size and MS-SSIM's
-    data range are those of each micro-batch, so a window of k batches of B is not one batch of k * B."""
+    data range are those of each micro-batch, so a window of k batches of B is not one batch of k * B.
+
+    Gradient clipping follows Lightning's ``Trainer(gradient_clip_val=v, gradient_clip_algorithm=...)``: once per
+    optimizer step, in the call that closes a window, on the averaged window gradient (after the all-reduce), before
+    Adam.  "norm" is ``clip_grad_norm_(max_norm=v)`` (norm type 2, no error on a non-finite norm): the norm and the
+    coefficient are computed on the device and Adam's kernel reads the coefficient from there, so the step never waits
+    for the host; ``grad_norm`` is then the pre-clip norm, a 0-dim device tensor that the next clipped step overwrites.
+    "value" is ``clip_grad_value_(v)``, a clamp inside Adam's kernel.  v None or 0: no clipping, the plain step."""
 
     def __init__(self, model: nn.Module, loss, lr: float = 1e-4, betas=(0.9, 0.999), group=None,
                  overlap_allreduce: bool = True, use_graph: Optional[bool] = None,
-                 accumulate_grad_batches: int = 1) -> None:
+                 accumulate_grad_batches: int = 1, gradient_clip_val: Optional[float] = None,
+                 gradient_clip_algorithm: Optional[str] = "norm") -> None:
         """use_graph: replay forward + loss + backward (~800 launches, ~95 % GPU-busy when launched through Python) as
         ONE CUDA graph per input shape (two with accumulate_grad_batches > 1: a window's first micro-batch and the later
         ones differ in their launches); Adam and the running loss state stay outside.  Off by default
@@ -130,6 +191,8 @@ class TrainStep:
         if isinstance(k, bool) or not isinstance(k, int) or k < 1:
             raise ValueError(f"accumulate_grad_batches={k!r}: expected an integer >= 1")
         self.accumulate_grad_batches = k
+        self.gradient_clip_val, self.gradient_clip_algorithm = gradient_clip_settings(gradient_clip_val,
+                                                                                      gradient_clip_algorithm)
         self.pending = 0  # micro-batches since the last optimizer step
         self.model, self.loss, self.group = model, loss, group
         self.world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
@@ -142,6 +205,10 @@ class TrainStep:
         self.engine = model._get_engine(train=True)
         self.engine.arena.invalidate()  # packed bf16 weight images follow the (possibly replaced) parameters
         self.opt = FusedAdam(self.flat, lr, betas, on_update=self.engine.arena.invalidate)
+        self.grad_norm: Optional[torch.Tensor] = None
+        if self.gradient_clip_val is not None and self.gradient_clip_algorithm == "norm":
+            self._clip_out = torch.zeros(2, dtype=torch.float32, device=self.flat.device)  # {norm, coefficient}
+            self._clip_ws = grad_norm_workspace(self.flat.numel(), self.flat.device)
         # XMM_COMM_MODE (experiments): "overlap" (default: chunks released per RRDB on a side stream), "serial" (one
         # all-reduce after the backward pass), "none" (NO gradient exchange -- replicas diverge; only to measure what the
         # collective costs next to the spread between the GPUs of a box)
@@ -256,6 +323,18 @@ class TrainStep:
         self.loss._merge(st)
         self.pending += 1
         if closing:
-            self.opt.step(flat_grad, 1.0 / self.world)
+            self._optimizer_step(flat_grad, 1.0 / self.world)
             self.pending = 0
         return st["total"]
+
+    def _optimizer_step(self, flat_grad: torch.Tensor, grad_scale: float) -> None:
+        """Adam on flat_grad * grad_scale (the averaged window gradient), clipped as configured.  Every rank clips the
+        same all-reduced buffer, so the replicas stay identical."""
+        if self.gradient_clip_val is None:
+            self.opt.step(flat_grad, grad_scale)
+        elif self.gradient_clip_algorithm == "value":
+            self.opt.step(flat_grad, grad_scale, clip_value=self.gradient_clip_val)
+        else:
+            grad_clip_coef(flat_grad, grad_scale, self.gradient_clip_val, self._clip_out, self._clip_ws)
+            self.grad_norm = self._clip_out[0]
+            self.opt.step(flat_grad, grad_scale, clip_coef=self._clip_out[1:])
